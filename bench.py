@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- atom-steps/sec of SGPR E+F+stress prediction (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--dump-outputs DIR]
 
 A step = one full evaluation (neighbour list -> descriptors -> kernel GEMMs -> energy,
 forces, virial) of one synthetic structure.  Workload (default c3, the configuration the
@@ -47,7 +47,24 @@ def parse():
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "p2p-nccl", "halo"],
                     help="multi-GPU force exchange: peer-memory adds over NVLink with the fused mailbox/flag exchange step "
                          "(default), the same with an NCCL all-reduce of E + virial as the barrier, or halo recompute")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's energy, forces and virial to DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl b200)")
+    return args
+
+
+def dump_outputs(dirname, E, F, W):
+    """What a caller of the timed path receives from its last step: energy [1], forces [N,3], virial [3,3], float64.
+    The inputs are seeded, so two builds run with the same arguments can be compared output for output: energy and
+    virial repeat bit for bit, forces to rounding (atomic adds in the force scatter; 2e-15 eV/A apart at c3 on a B200).
+    The largest workload (c5, 1,000,188 atoms) writes 24 MB."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in (("energy", [E]), ("forces", F), ("virial", W)):
+        np.save(os.path.join(dirname, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def workload_inputs(name, variants):
@@ -449,6 +466,7 @@ def main():
         return E
 
     def timed(fn, steps, warmup):
+        """-> (device ms, wall ms, what the last timed step returned)"""
         for it in range(warmup):
             fn(it)
         barrier()
@@ -456,7 +474,7 @@ def main():
         e0.record()
         t0 = time.perf_counter()
         for it in range(steps):
-            fn(it)
+            last = fn(it)
         e1.record()
         barrier()
         wall = time.perf_counter() - t0
@@ -464,16 +482,33 @@ def main():
         t = torch.tensor([ms, wall * 1e3], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t[0].item()), float(t[1].item())
+        return float(t[0].item()), float(t[1].item()), last
+
+    def full_results(res):
+        """(E, F [N,3] device tensor, W [3,3]) of one step_device() result, summed over the ranks where the step leaves
+        partial results.  A collective when sharded: every rank calls it; read it before the next step overwrites it."""
+        if px is not None:
+            Fd = res[1] * res[3].to(torch.float64)[:, None]
+            dist.all_reduce(Fd)
+            return float(res[0].item()), Fd, res[2].cpu().numpy().reshape(3, 3)
+        Fd = res[1].clone()
+        if world > 1:
+            dist.all_reduce(Fd)   # halo mode: forces only on owned atoms, zeros elsewhere
+            return float(ew[0].item()), Fd, ew[1:].cpu().numpy().reshape(3, 3)
+        return float(res[0].item()), Fd, res[2].cpu().numpy().reshape(3, 3)
 
     # ---- device-resident leg (value): no in-library events, no stats calls inside the timed region; after the first
     # (sizing) step the library enqueues every step without host synchronisation -- validated after the timed region
     eng.set_async(True)
     sampler = make_sampler(local_rank)
     sampler.start()
-    ms_dev, wall_dev = timed(step_device, args.steps, args.warmup)
+    ms_dev, wall_dev, last = timed(step_device, args.steps, args.warmup)
     clocks = sampler.stop()
     eng.check()          # raises if any asynchronous step was invalid (pair list outgrew its capacity ...)
+    if args.dump_outputs:
+        E_last, F_last, W_last = full_results(last)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, E_last, F_last.cpu().numpy(), W_last)
     launches_per_step = eng.stats()["kernel_launches"] + (1 if px is not None else 0)
     # ---- stage split: a separate, untimed pass with CUDA events between the stages inside the library
     eng.enable_timing(True)
@@ -493,7 +528,7 @@ def main():
         print(f"rank {rank}: " + " ".join(f"{k[3:]}={stage[k]:.4f}" for k in ("ms_nl", "ms_desc", "ms_gemm", "ms_force", "ms_beta", "ms_total")),
               file=sys.stderr, flush=True)
     # ---- end-to-end leg: host buffers through the public host API (H2D + D2H inside)
-    ms_e2e, wall_e2e = timed(step_host, args.steps, args.warmup)
+    ms_e2e, wall_e2e, _ = timed(step_host, args.steps, args.warmup)
     eng.check()
 
     # ---- parity, outside the timed regions, every N
@@ -502,16 +537,8 @@ def main():
         # (1) full-size structure: sampled atoms against the oracle port
         res = step_device(0)
         torch.cuda.synchronize()
-        if px is not None:
-            Fd = res[1] * res[3].to(torch.float64)[:, None]
-            dist.all_reduce(Fd)
-        else:
-            Fd = res[1].clone()
-            if world > 1:
-                dist.all_reduce(Fd)   # halo mode: forces only on owned atoms, zeros elsewhere
+        E_sh, Fd, W_sh = full_results(res)
         F_gpu = Fd.cpu().numpy()
-        E_sh, W_sh = (float(res[0].item()), res[2].cpu().numpy().reshape(3, 3)) if px is not None else \
-            ((float(ew[0].item()), ew[1:].cpu().numpy().reshape(3, 3)) if world > 1 else (float(res[0].item()), res[2].cpu().numpy().reshape(3, 3)))
         if rank == 0:
             parity["full_size_vs_oracle_port"] = parity_full_size(eng, model, pos_variants[0], cell, numbers, F_gpu,
                                                                    n_probe=3 if N <= 200000 else 2)

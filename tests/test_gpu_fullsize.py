@@ -248,3 +248,35 @@ def test_c3_large_weights_int8_slices_vs_fp64_dmma(c3, monkeypatch):
     assert np.abs(Fi - Fd).max() < 1e-6
     vol = abs(np.linalg.det(cell))
     assert np.abs(Wi - Wd).max() / vol < 1e-7
+
+
+def test_bench_dumps_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs DIR: energy, forces and virial of the last timed step as float64 .npy files, equal to a
+    prediction of the same seeded inputs through the host API.  Run from another directory: bench.py needs none."""
+    import subprocess
+    import sys
+
+    import autoforce_b200 as ab
+    from autoforce_b200 import synth
+
+    sys.path.insert(0, ROOT)
+    from bench import workload_inputs
+
+    steps, variants = 3, 2
+    out = tmp_path / "dump"
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c2", "--steps", str(steps), "--warmup", "1",
+           "--variants", str(variants), "--no-cpu-baseline", "--dump-outputs", str(out)]
+    r = subprocess.run(cmd, cwd=str(tmp_path), capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = {name: np.load(out / f"{name}.npy") for name in ("energy", "forces", "virial")}
+    w, pos_variants, cell, numbers = workload_inputs("c2", variants)
+    N = len(numbers)
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["energy"].shape == (1,) and got["forces"].shape == (N, 3) and got["virial"].shape == (3, 3)
+    model = synth.synth_model(w["Zs"], w["M"], 1, lmax=w["lmax"], nmax=w["nmax"], rc=w["rc"])
+    eng = ab.SgprEngine(model, species=w["Zs"])
+    E, F, W, _ = eng.predict(pos_variants[(steps - 1) % variants], numbers, cell, True)
+    eng.close()
+    assert abs(got["energy"][0] - E) / N < 1e-12
+    assert np.abs(got["forces"] - F).max() < 1e-10
+    assert np.abs(got["virial"] - W).max() < 1e-9
