@@ -205,6 +205,52 @@ class B200Calculator(_AseCalculator):
         self.step += 1
         return self.results
 
+    def calculate_batch(self, images):
+        """Many structures in one GPU call (``SgprEngine.predict_batch``): testing a model on a trajectory, the images of
+        an NEB, scoring a data set.  Returns one results dict per image, with the keys, dtypes and stress convention of
+        ``calculate``.  With ``covloss=True`` each image also gets ``beta`` and ``covlog``, and ``on_uncertain(image,
+        beta)`` is called for each image whose max(beta) exceeds ``ediff``.  Under torch.distributed the images given
+        are evaluated on the local device: splitting a data set over ranks is the caller's job.  Does not change
+        ``self.atoms`` / ``self.results`` of the step-by-step interface."""
+        images = list(images)
+        if not images:
+            return []
+        numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images])
+        eng = self._get_engine(numbers)
+        if self.covloss:
+            E, F, W, beta = eng.predict_batch(images, want_beta=True)
+        else:
+            E, F, W = eng.predict_batch(images)
+            for e in self._more_engines:   # kernels with different hyper-parameters: the contributions add up
+                E2, F2, W2 = e.predict_batch(images)
+                E, F, W = E + E2, F + F2, W + W2
+            beta = None
+        _, rank, _ = self._dist()
+        out = []
+        a0 = 0
+        for b, a in enumerate(images):
+            n = len(a.numbers)
+            cell = np.asarray(a.cell, dtype=np.float64).reshape(3, 3)
+            vol = abs(np.linalg.det(cell))
+            if vol == 0.0:
+                vol = -2.0  # calculator/active.py:606-609
+            r = {
+                "energy": np.array(E[b], dtype=np.float64),
+                "forces": F[a0:a0 + n].copy(),
+                "stress": (W[b] / vol).reshape(-1)[[0, 4, 8, 5, 2, 1]],
+                "free_energy": np.array(E[b], dtype=np.float64),
+            }
+            if beta is not None:
+                bb = beta[a0:a0 + n].copy()
+                covloss_max = float(np.max(bb)) if n else 0.0   # like torch.max: NaN / inf propagate
+                r["beta"] = bb
+                r["covlog"] = f"{covloss_max}"
+                if covloss_max > self.ediff and self.on_uncertain is not None and rank == 0:
+                    self.on_uncertain(a, bb)
+            out.append(r)
+            a0 += n
+        return out
+
     # ------------------------------------------------------------------ getters (callers without ASE)
     def _same_state(self, atoms):
         a = self.atoms

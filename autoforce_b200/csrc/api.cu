@@ -3,6 +3,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 
 #include <nvtx3/nvToolsExt.h>
@@ -20,6 +21,9 @@ struct NvtxRange {
 
 static thread_local char g_err[1024] = "";
 
+static std::atomic<unsigned long long> g_buf_generation{0};
+unsigned long long buf_generation() { return g_buf_generation.load(); }
+
 void set_error(const char* fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
@@ -31,6 +35,7 @@ int DevBuf::ensure(size_t need) {
     if (need <= bytes) return SGPR_OK;
     if (p) cudaFree(p);
     p = nullptr;
+    g_buf_generation.fetch_add(1);
     size_t want = need + need / 4 + 256;
     cudaError_t e = cudaMalloc(&p, want);
     if (e != cudaSuccess) {
@@ -434,6 +439,40 @@ __global__ void nl_export_kernel(int64_t N, const AtomRec* __restrict__ atoms, c
     }
 }
 
+// Per-structure sums of a batch, one warp per structure: E = local energies + mean + lone-atom terms
+// (atom_terms_kernel's work), W = the environments' virials.  A structure is the cell-order range first[b] ..
+// first[b+1]-1 (structure-major keys), whose order depends on that structure alone; lane-strided partial sums and a
+// fixed shuffle tree make E and W reproducible and independent of the rest of the batch.
+__global__ void batch_reduce_kernel(int B, const long long* __restrict__ first, const AtomRec* __restrict__ atoms,
+                                    const int* __restrict__ rowof, const long long* __restrict__ nl_first,
+                                    const double* __restrict__ erow, const double* __restrict__ mean_w,
+                                    const double* __restrict__ lone_mu, const double* __restrict__ wenv,
+                                    double* __restrict__ E, double* __restrict__ W) {
+    const int lane = threadIdx.x & 31;
+    const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (b >= B) return;
+    double e = 0.0, w[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+    for (long long c = first[b] + lane; c < first[b + 1]; c += 32) {
+        const int sp = meta_species(atoms[c].meta);
+        e += erow[rowof[c]];
+        e += mean_w[sp];
+        if (nl_first[c + 1] == nl_first[c]) e += lone_mu[sp];
+#pragma unroll
+        for (int q = 0; q < 9; ++q) w[q] += wenv[9 * c + q];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        e += __shfl_xor_sync(0xffffffffu, e, o);
+#pragma unroll
+        for (int q = 0; q < 9; ++q) w[q] += __shfl_xor_sync(0xffffffffu, w[q], o);
+    }
+    if (lane == 0) {
+        E[b] = e;
+#pragma unroll
+        for (int q = 0; q < 9; ++q) W[9 * (size_t)b + q] = w[q];
+    }
+}
+
 }  // namespace sgpr
 
 using namespace sgpr;
@@ -803,7 +842,8 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->nl_first, &h->nl_pairs, &h->scan_tmp, &h->phat, &h->cbuf, &h->pnorm, &h->sflag, &h->gmat,
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
-                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2};
+                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
+                      &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv};
     for (DevBuf* b : bufs) b->release();
     if (h->pinned) cudaFreeHost(h->pinned);
     if (h->i8_probs_pinned) cudaFreeHost(h->i8_probs_pinned);
@@ -938,6 +978,74 @@ static bool warm_possible(sgpr_handle h, int64_t N, const int32_t* pbc_h, int32_
            rank == h->warm_rank && world == h->warm_world && beta == h->warm_beta;
 }
 
+constexpr int kRowEnergyGrid = 128;   // blocks (= energy partials) of row_energy_kernel
+
+// energy partials per row of each central species (0 where the species has no usable inducing points)
+static RowSpecies row_species(sgpr_context* h, int* max_part) {
+    RowSpecies rs{};
+    rs.S = h->S;
+    for (int s = 0; s < h->S; ++s) {
+        const int Ms = h->m_first[s + 1] - h->m_first[s];
+        rs.n_part[s] = (Ms > 0 && h->dp.central_enabled[s]) ? (h->use_i8_now ? i8_energy_parts(Ms) : gemm_energy_parts(Ms)) : 0;
+        if (rs.n_part[s] > *max_part) *max_part = rs.n_part[s];
+    }
+    return rs;
+}
+
+// kernel matrix of the step's rows -> local energies erow (+ block partials epart) -> back projection gvec = dE/dq_hat
+static int gemm_stage(sgpr_context* h, cudaStream_t st, const RowSpecies& rs, bool with_beta) {
+    const size_t nrows = (size_t)h->n_active + 1;
+    nvtxRangePushA("sgpr:gemm");
+    struct PopGemm {
+        bool armed = true;
+        ~PopGemm() {
+            if (armed) nvtxRangePop();
+        }
+    } gemm_range;
+    if (h->use_i8_now)
+        SGPR_TRY(i8_kernel_matrix(h, st, with_beta));
+    else
+        SGPR_TRY(gemm_kernel_matrix(h, nullptr, 0, nullptr, with_beta, st));
+    row_energy_kernel<<<kRowEnergyGrid, 256, 0, st>>>((int)h->n_active, rs, h->row_first_d.as<int>(), h->erow_part.as<double>(),
+                                                      (int)nrows, h->active_all ? nullptr : h->row_owned.as<unsigned char>(),
+                                                      h->erow.as<double>(), h->epart.as<double>());
+    h->stats.kernel_launches += 1;
+    if (h->use_i8_now)
+        SGPR_TRY(i8_back_projection(h, st));
+    else
+        SGPR_TRY(gemm_back_projection(h, st));
+    if (h->timing) cudaEventRecord(h->ev[3], st);
+    gemm_range.armed = false;
+    nvtxRangePop();
+    return SGPR_OK;
+}
+
+// covloss of the step's environments into beta_d [N] (caller's order)
+static int covloss_stage(sgpr_context* h, cudaStream_t st, int64_t N, const int* active, const unsigned char* owned,
+                         double* beta_d) {
+    const size_t nrows = (size_t)h->n_active + 1;
+    NvtxRange covloss_range("sgpr:covloss");
+    const int n_part = h->use_i8_now ? i8_covloss_parts(h) : gemm_covloss_parts(h);
+    SGPR_TRY(h->cpart.ensure(sizeof(double) * (size_t)n_part * nrows));
+    SGPR_CUDA(cudaMemsetAsync(beta_d, 0, sizeof(double) * (size_t)N, st));
+    if (h->use_i8_now)
+        SGPR_TRY(i8_covloss(h, (int64_t)nrows, st));
+    else
+        SGPR_TRY(gemm_covloss(h, (int64_t)nrows, st));
+    if (h->n_active > 0) {
+        SGPR_TRY(h->misc.ensure(sizeof(int) * SGPR_MAX_SPECIES));
+        SGPR_CUDA(cudaMemcpyAsync(h->misc.p, h->dp.central_enabled, sizeof(int) * SGPR_MAX_SPECIES,
+                                  cudaMemcpyHostToDevice, st));
+        beta_finish_kernel<<<h->sm_count * 2, 256, 0, st>>>(
+            (int)h->n_active, active, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1), h->nl_first.as<long long>(),
+            owned, h->sp_on.as<unsigned char>(), h->misc.as<int>(), h->cpart.as<double>(), n_part, (int)nrows,
+            h->clone_d.as<double>(), h->vscale_d.as<double>(), h->prow.as<double>(), h->dp.normalize, h->xi, beta_d);
+        h->stats.kernel_launches += 1;
+    }
+    SGPR_CUDA(cudaGetLastError());
+    return SGPR_OK;
+}
+
 static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,
                         const int32_t* pbc_h, int32_t rank, int32_t world, void* stream, double* E_d, double* F_d,
                         double* W_d, double* beta_d, uint8_t* owned_d, const uint64_t* peer_f_h, bool allow_warm,
@@ -1000,18 +1108,12 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
     }
     const unsigned char* owned = h->active_all ? nullptr : h->owned.as<unsigned char>();
     const int* active = h->active_all ? nullptr : h->active_list.as<int>();
-    const int grid_g = 128;   // blocks (= energy partials) of row_energy_kernel
+    const int grid_g = kRowEnergyGrid;
     const int nblk_b = backward_grid(h);
     const int nblk_x = 64;
     const size_t nrows = (size_t)h->n_active + 1;
-    RowSpecies rs{};
-    rs.S = h->S;
     int max_part = 1;
-    for (int s = 0; s < h->S; ++s) {
-        const int Ms = h->m_first[s + 1] - h->m_first[s];
-        rs.n_part[s] = (Ms > 0 && h->dp.central_enabled[s]) ? (h->use_i8_now ? i8_energy_parts(Ms) : gemm_energy_parts(Ms)) : 0;
-        if (rs.n_part[s] > max_part) max_part = rs.n_part[s];
-    }
+    const RowSpecies rs = row_species(h, &max_part);
     SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * nrows));
     SGPR_TRY(h->erow.ensure(sizeof(double) * nrows));
     if (!h->use_i8_now) SGPR_TRY(h->gmat.ensure(sizeof(double) * nrows * h->ldg));
@@ -1027,28 +1129,7 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
     }
     if (!peer_f_h) SGPR_CUDA(cudaMemsetAsync(h->fcell.p, 0, sizeof(double) * 3 * ((size_t)N + 1), st));
     if (beta_d && !h->use_i8_now) SGPR_TRY(h->kcmat.ensure(sizeof(double) * nrows * h->ldg));
-    nvtxRangePushA("sgpr:gemm");
-    struct PopGemm {
-        bool armed = true;
-        ~PopGemm() {
-            if (armed) nvtxRangePop();
-        }
-    } gemm_range;
-    if (h->use_i8_now)
-        SGPR_TRY(i8_kernel_matrix(h, st, beta_d != nullptr));
-    else
-        SGPR_TRY(gemm_kernel_matrix(h, nullptr, 0, nullptr, beta_d != nullptr, st));
-    row_energy_kernel<<<grid_g, 256, 0, st>>>((int)h->n_active, rs, h->row_first_d.as<int>(), h->erow_part.as<double>(),
-                                              (int)nrows, h->active_all ? nullptr : h->row_owned.as<unsigned char>(),
-                                              h->erow.as<double>(), h->epart.as<double>());
-    h->stats.kernel_launches += 1;
-    if (h->use_i8_now)
-        SGPR_TRY(i8_back_projection(h, st));
-    else
-        SGPR_TRY(gemm_back_projection(h, st));
-    if (h->timing) cudaEventRecord(h->ev[3], st);
-    gemm_range.armed = false;
-    nvtxRangePop();
+    SGPR_TRY(gemm_stage(h, st, rs, beta_d != nullptr));
     NvtxRange force_range("sgpr:force");
     SGPR_TRY(descriptor_backward_atoms(h, g, owned, st, peer_f_h ? &peers : nullptr));
     if (peer_f_h && N > 0) {
@@ -1071,27 +1152,7 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
     SGPR_CUDA(cudaGetLastError());
     if (h->timing) cudaEventRecord(h->ev[4], st);
     if (!warm) h->stats.covloss_flops = 0.0;
-    if (beta_d) {
-        NvtxRange covloss_range("sgpr:covloss");
-        const int n_part = h->use_i8_now ? i8_covloss_parts(h) : gemm_covloss_parts(h);
-        SGPR_TRY(h->cpart.ensure(sizeof(double) * (size_t)n_part * nrows));
-        SGPR_CUDA(cudaMemsetAsync(beta_d, 0, sizeof(double) * (size_t)N, st));
-        if (h->use_i8_now)
-            SGPR_TRY(i8_covloss(h, (int64_t)nrows, st));
-        else
-            SGPR_TRY(gemm_covloss(h, (int64_t)nrows, st));
-        if (h->n_active > 0) {
-            SGPR_TRY(h->misc.ensure(sizeof(int) * SGPR_MAX_SPECIES));
-            SGPR_CUDA(cudaMemcpyAsync(h->misc.p, h->dp.central_enabled, sizeof(int) * SGPR_MAX_SPECIES,
-                                      cudaMemcpyHostToDevice, st));
-            beta_finish_kernel<<<h->sm_count * 2, 256, 0, st>>>(
-                (int)h->n_active, active, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1), h->nl_first.as<long long>(),
-                owned, h->sp_on.as<unsigned char>(), h->misc.as<int>(), h->cpart.as<double>(), n_part, (int)nrows,
-                h->clone_d.as<double>(), h->vscale_d.as<double>(), h->prow.as<double>(), h->dp.normalize, h->xi, beta_d);
-            h->stats.kernel_launches += 1;
-        }
-        SGPR_CUDA(cudaGetLastError());
-    }
+    if (beta_d) SGPR_TRY(covloss_stage(h, st, N, active, owned, beta_d));
     if (px) {
         long long* counter = reinterpret_cast<long long*>(h->p2p_local.as<double>() + 16);
         p2p_publish_wait_kernel<<<1, 32, 0, st>>>(rank, world, px->peers, h->p2p_local.as<double>(), counter, E_out, W_out,
@@ -1155,6 +1216,13 @@ static int predict_impl(sgpr_handle h, int64_t N, const double* pos_d, const int
         key.px_ptr[1] = px->owned_d;
         key.px_ptr[2] = px->own_base;
         for (int r = 0; r < SGPR_MAX_RANKS; ++r) key.px_mail[r] = (uint64_t)(uintptr_t)px->peers.mail[r];
+    }
+    // a workspace was reallocated since the graphs were captured (e.g. a larger structure or a batch in between):
+    // their nodes point at freed memory
+    const unsigned long long gen = buf_generation();
+    if (gen != h->graph_gen) {
+        drop_graphs(h);
+        h->graph_gen = gen;
     }
     for (auto& e : h->graphs) {
         if (memcmp(&e.key, &key, sizeof(key)) == 0) {
@@ -1386,6 +1454,144 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_host(sgpr_han
     if (!f_pinned) memcpy(F_h, pin_out + 16, nb_pos);
     if (owned_h) memcpy(owned_h, pin_own, (size_t)N);
     if (beta_h) memcpy(beta_h, pin_out + 16 + 3 * (size_t)N, sizeof(double) * (size_t)N);
+    return SGPR_OK;
+}
+
+// B independent structures in one call (include/sgpr_b200.h).  Same stages as a sizing step of sgpr_predict over the
+// concatenated atoms; what differs is per-structure geometry (batched cell sort, neighbour search and image shifts) and
+// the per-structure reductions.  The rows are ordinary descriptor rows: GEMMs, covloss and force scatter are shared.
+extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_handle h, int32_t B, const int64_t* first_h,
+                                                                         const double* pos_d, const int32_t* Z_d,
+                                                                         const double* cell_h, const int32_t* pbc_h,
+                                                                         void* stream, double* E_d, double* F_d,
+                                                                         double* W_d, double* beta_d) {
+    if (!h || B < 0 || !first_h || (B > 0 && (!cell_h || !pbc_h || !E_d || !W_d))) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    if (first_h[0] != 0) {
+        set_error("first_h[0] = %lld, must be 0", (long long)first_h[0]);
+        return SGPR_ERR_INVALID;
+    }
+    for (int b = 0; b < B; ++b)
+        if (first_h[b + 1] < first_h[b]) {
+            set_error("first_h is not monotone at structure %d (%lld > %lld)", b, (long long)first_h[b], (long long)first_h[b + 1]);
+            return SGPR_ERR_INVALID;
+        }
+    const int64_t N = first_h[B];
+    if (N > 0x7fffff00ll) {
+        set_error("bad atom count");
+        return SGPR_ERR_INVALID;
+    }
+    if (N > 0 && (!pos_d || !Z_d || !F_d)) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    if (beta_d && !h->has_choli) {
+        set_error("covloss requested but the model has no choli");
+        return SGPR_ERR_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    SGPR_CUDA(cudaSetDevice(h->device));
+    h->fwd_valid = false;   // no state for sgpr_kernel_backward
+    h->warm_ok = false;     // the next single-structure step sizes its buffers again
+    h->step_was_warm = false;
+    if (B == 0) return SGPR_OK;
+    h->use_i8_now = h->use_i8;
+    h->stats.i8_ops = 0.0;
+    h->stats.gemm_flops = 0.0;
+    h->stats.covloss_flops = 0.0;
+    h->stats.kernel_launches = 0;
+    h->stats.n_atoms = N;
+    h->last_N = N;
+    // geometry of every structure, as build_geometry gives it alone; bins of the batch one after the other
+    std::vector<Geom> gs;
+    SGPR_TRY(build_geometry_batch(h, B, first_h, pos_d, cell_h, pbc_h, st, &gs));
+    std::vector<int> bin_base(B + 1, 0);
+    std::vector<double> cells(9 * (size_t)B);
+    long long ncell = 0;
+    for (int b = 0; b < B; ++b) {
+        bin_base[b] = (int)ncell;
+        ncell += gs[b].ncell;
+        for (int q = 0; q < 9; ++q) cells[9 * (size_t)b + q] = gs[b].cell[q];
+    }
+    if ((ncell + 1) * h->S > 0x7fffffffll) {
+        set_error("batch too large: %lld bins", ncell);
+        return SGPR_ERR_INVALID;
+    }
+    bin_base[B] = (int)ncell;
+    SGPR_TRY(h->b_geom.ensure(sizeof(Geom) * (size_t)B));
+    SGPR_TRY(h->b_first.ensure(sizeof(long long) * ((size_t)B + 1)));
+    SGPR_TRY(h->b_bins.ensure(sizeof(int) * ((size_t)B + 1)));
+    SGPR_TRY(h->b_cell.ensure(sizeof(double) * 9 * (size_t)B));
+    SGPR_TRY(h->b_err.ensure(sizeof(unsigned long long) * 2));
+    SGPR_TRY(h->astr.ensure(sizeof(int) * ((size_t)N + 1)));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_geom.p, gs.data(), sizeof(Geom) * (size_t)B, cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_first.p, first_h, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_bins.p, bin_base.data(), sizeof(int) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, cells.data(), sizeof(double) * 9 * (size_t)B, cudaMemcpyHostToDevice, st));
+    BatchGeom bg{};
+    bg.B = B;
+    bg.ncell = (int)ncell;
+    bg.geoms = h->b_geom.as<Geom>();
+    bg.first = h->b_first.as<long long>();
+    bg.bin_base = h->b_bins.as<int>();
+    bg.cells = h->b_cell.as<double>();
+    bg.astr = h->astr.as<int>();
+    bg.err = h->b_err.as<unsigned long long>();
+    const Geom unused{};
+    // cell sort -> neighbour list (the call's one sizing synchronisation) -> descriptors
+    if (h->timing) cudaEventRecord(h->ev[0], st);
+    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, bg, st));
+    int64_t n_pairs = 0;
+    SGPR_TRY(batch_neighbor_build(h, N, bg, st, &n_pairs));
+    h->stats.n_active = h->n_active;
+    h->stats.n_pairs = n_pairs;
+    if (h->timing) cudaEventRecord(h->ev[1], st);
+    const size_t nrows = (size_t)N + 1;
+    SGPR_TRY(h->phat.ensure(sizeof(double) * nrows * h->dp.ldp));
+    if (h->use_i8_now) SGPR_TRY(i8_ensure_step_buffers(h, (size_t)N, beta_d != nullptr));
+    SGPR_TRY(descriptor_forward_atoms(h, unused, st, &bg));
+    if (h->timing) cudaEventRecord(h->ev[2], st);
+    if (h->use_i8_now) SGPR_TRY(i8_setup_step(h, st));
+    int max_part = 1;
+    const RowSpecies rs = row_species(h, &max_part);
+    SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * nrows));
+    SGPR_TRY(h->erow.ensure(sizeof(double) * nrows));
+    if (!h->use_i8_now) SGPR_TRY(h->gmat.ensure(sizeof(double) * nrows * h->ldg));
+    SGPR_TRY(h->gvec.ensure(sizeof(double) * nrows * h->dp.ldp));
+    SGPR_TRY(h->epart.ensure(sizeof(double) * kRowEnergyGrid));
+    SGPR_TRY(h->fcell.ensure(sizeof(double) * 3 * nrows));
+    SGPR_TRY(h->wenv.ensure(sizeof(double) * 9 * nrows));
+    SGPR_CUDA(cudaMemsetAsync(h->fcell.p, 0, sizeof(double) * 3 * nrows, st));
+    SGPR_CUDA(cudaMemsetAsync(h->wenv.p, 0, sizeof(double) * 9 * nrows, st));
+    if (beta_d && !h->use_i8_now) SGPR_TRY(h->kcmat.ensure(sizeof(double) * nrows * h->ldg));
+    SGPR_TRY(gemm_stage(h, st, rs, beta_d != nullptr));
+    {
+        NvtxRange force_range("sgpr:force");
+        SGPR_TRY(descriptor_backward_atoms(h, unused, nullptr, st, nullptr, &bg));
+        if (N > 0)
+            scatter_forces_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->fcell.as<double>(),
+                                                                          nullptr, F_d, nullptr);
+        batch_reduce_kernel<<<(B + 7) / 8, 256, 0, st>>>(B, bg.first, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1),
+                                                        h->nl_first.as<long long>(), h->erow.as<double>(),
+                                                        h->mean_w_d.as<double>(), h->lone_mu.as<double>(),
+                                                        h->wenv.as<double>(), E_d, W_d);
+        h->stats.kernel_launches += 2;
+        SGPR_CUDA(cudaGetLastError());
+    }
+    if (h->timing) cudaEventRecord(h->ev[4], st);
+    if (beta_d) SGPR_TRY(covloss_stage(h, st, N, nullptr, nullptr, beta_d));
+    if (h->timing) {
+        cudaEventRecord(h->ev[5], st);
+        SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
+        cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
+        cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
+        cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
+        cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
+        cudaEventElapsedTime(&h->stats.ms_beta, h->ev[4], h->ev[5]);
+        cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
+    }
     return SGPR_OK;
 }
 

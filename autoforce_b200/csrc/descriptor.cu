@@ -56,10 +56,16 @@ struct EnvSrc {
     const unsigned char* env_sp;
 };
 
+// image-shift cell of a batched step: the lattice vectors of the centre's structure (G = Geom otherwise)
+struct CellRef {
+    const double* cell;
+};
+
 template <bool ENV>
 struct Nbr {
     // displacement r_ij (as the reference computes it) and species of neighbour k
-    __device__ static __forceinline__ void load(const EnvSrc& src, const Geom& g, const AtomRec& ai, long long k,
+    template <class G>
+    __device__ static __forceinline__ void load(const EnvSrc& src, const G& g, const AtomRec& ai, long long k,
                                                 double& rx, double& ry, double& rz, int& sp, int& j) {
         if (ENV) {
             rx = src.env_r[3 * k];
@@ -72,7 +78,8 @@ struct Nbr {
         }
     }
     // atoms mode with the pair record already in registers (software-pipelined loops)
-    __device__ static __forceinline__ void load_pair(const EnvSrc& src, const Geom& g, const AtomRec& ai, const PairRec pr,
+    template <class G>
+    __device__ static __forceinline__ void load_pair(const EnvSrc& src, const G& g, const AtomRec& ai, const PairRec pr,
                                                      double& rx, double& ry, double& rz, int& sp, int& j) {
         {
             const AtomRec aj = src.atoms[pr.j];
@@ -133,7 +140,8 @@ __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double
 // FP64 tensor cores -- M = lm (8-row tiles), N = n (8-column tiles), K = neighbours of the species (4 per step),
 // fragments read from the chunk buffer.  (TN, TL only shape the chunk-buffer rows.)
 // EXNB > 0: dp.nb == EXNB and dp.lmax == LMAX (bounds, strides and tile predicates fold at compile time)
-template <int LMAX, int TN, int TL, bool ENV, int EXNB>
+// BATCH: batched step, image shifts from bcell [B,9] of the centre's structure astr[c]
+template <int LMAX, int TN, int TL, bool ENV, int EXNB, bool BATCH = false>
 __global__ void __launch_bounds__(128, (LMAX <= 3 ? 7 : 4)) desc_forward_kernel(DescParams dp, Geom g, int n_env, EnvSrc src,
                                                            const int* __restrict__ row_of,
                                                            const unsigned* __restrict__ ptab,
@@ -141,7 +149,9 @@ __global__ void __launch_bounds__(128, (LMAX <= 3 ? 7 : 4)) desc_forward_kernel(
                                                            double* __restrict__ cbuf, double* __restrict__ prow,
                                                            unsigned char* __restrict__ sflag, int per_warp_doubles,
                                                            int stride_, int nbp_, signed char* __restrict__ p8,
-                                                           long long p8_slice, int kp1) {
+                                                           long long p8_slice, int kp1,
+                                                           const double* __restrict__ bcell = nullptr,
+                                                           const int* __restrict__ astr = nullptr) {
     extern __shared__ __align__(16) double smem[];
     constexpr bool EXACT = EXNB > 0;
     constexpr int kNbp = ((EXNB + TN - 1) / TN) * TN, kL2 = (LMAX + 1) * (LMAX + 1);
@@ -182,13 +192,18 @@ __global__ void __launch_bounds__(128, (LMAX <= 3 ? 7 : 4)) desc_forward_kernel(
             beg = src.nl_first[env];
             end = src.nl_first[env + 1];
         }
+        [[maybe_unused]] CellRef cref{nullptr};
+        if constexpr (BATCH) cref.cell = bcell + 9 * (size_t)astr[c];
         for (int t = lane; t < dp.csize; t += 32) c_s[t] = 0.0;
         // pass 0: does any neighbour sit (almost) on the z axis?   ylm.py:10-23
         bool hit = false;
         for (long long k = beg + lane; k < end; k += 32) {
             double rx, ry, rz;
             int sp, j;
-            Nbr<ENV>::load(src, g, ai, k, rx, ry, rz, sp, j);
+            if constexpr (BATCH)
+                Nbr<ENV>::load(src, cref, ai, k, rx, ry, rz, sp, j);
+            else
+                Nbr<ENV>::load(src, g, ai, k, rx, ry, rz, sp, j);
             hit |= near_z_axis(rx, ry, rz);   // |x| < a |z| and |y| < a |z| does not depend on the length unit
         }
         const bool flag = __any_sync(0xffffffffu, hit);
@@ -218,7 +233,10 @@ __global__ void __launch_bounds__(128, (LMAX <= 3 ? 7 : 4)) desc_forward_kernel(
             if (k < end) {
                 double rx, ry, rz;
                 int sp, j;
-                Nbr<ENV>::load(src, g, ai, k, rx, ry, rz, sp, j);
+                if constexpr (BATCH)
+                    Nbr<ENV>::load(src, cref, ai, k, rx, ry, rz, sp, j);
+                else
+                    Nbr<ENV>::load(src, g, ai, k, rx, ry, rz, sp, j);
                 const double u = dp.radii[sp], ru = dp.rinv[sp];
                 const double x = rx * ru, y = ry * ru, z = rz * ru;
                 const double d2 = x * x + y * y + z * z;
@@ -448,7 +466,9 @@ struct BackOut {
 };
 
 // EXACT: dp.lmax == LMAX and dp.nb == NB (the loop bounds, strides and radial-index predicates fold at compile time)
-template <int LMAX, int NB, bool EXACT>
+// BATCH: batched step -- image shifts from bcell [B,9] of the centre's structure astr[c]; each environment writes its
+// virial (lane partials, fixed shuffle tree) to wenv [c, 9] instead of the per-block partials
+template <int LMAX, int NB, bool EXACT, bool BATCH = false>
 __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(DescParams dp, Geom g, int n_env, EnvSrc src,
                                                             const int* __restrict__ row_of,
                                                             const double* __restrict__ tvec,
@@ -458,7 +478,9 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
                                                             const double* __restrict__ prow, double xi,
                                                             const double* __restrict__ cbuf,
                                                             const unsigned char* __restrict__ sflag, BackOut out,
-                                                            int per_warp_doubles) {
+                                                            int per_warp_doubles, const double* __restrict__ bcell = nullptr,
+                                                            const int* __restrict__ astr = nullptr,
+                                                            double* __restrict__ wenv = nullptr) {
     extern __shared__ __align__(16) double smem[];
     __shared__ double wred[8][9];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
@@ -536,6 +558,12 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
         const int c = src.active ? src.active[env] : env;
         const AtomRec ai = src.atoms[c];
         const int si = meta_species(ai.meta);
+        [[maybe_unused]] CellRef cref{nullptr};
+        if constexpr (BATCH) {
+            cref.cell = bcell + 9 * (size_t)astr[c];
+#pragma unroll
+            for (int q = 0; q < 9; ++q) Wacc[q] = 0.0;
+        }
         const long long beg = src.nl_first[env], end = src.nl_first[env + 1];
         const bool skip = end == beg || !out.sp_on[si];   // warp-uniform
         const bool flag = sflag[env] != 0;
@@ -630,7 +658,10 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
             const PairRec pr = pr_n;
             const bool more = k + 32 < end;
             if (more) pr_n = src.pairs[k + 32];
-            Nbr<false>::load_pair(src, g, ai, pr, rx, ry, rz, sp, j);
+            if constexpr (BATCH)
+                Nbr<false>::load_pair(src, cref, ai, pr, rx, ry, rz, sp, j);
+            else
+                Nbr<false>::load_pair(src, g, ai, pr, rx, ry, rz, sp, j);
             const double u = dp.radii[sp], ru = dp.rinv[sp];
             const double x = rx * ru, y = ry * ru, z = rz * ru;
             const double d2 = x * x + y * y + z * z;
@@ -720,18 +751,27 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
             atomicAdd(fown + 3 * (size_t)c + 1, Fy);
             atomicAdd(fown + 3 * (size_t)c + 2, Fz);
         }
+        if constexpr (BATCH) {
+#pragma unroll
+            for (int q = 0; q < 9; ++q) Wacc[q] = warp_sum(Wacc[q]);
+            if (lane == 0)
+#pragma unroll
+                for (int q = 0; q < 9; ++q) wenv[9 * (size_t)c + q] = Wacc[q];
+        }
         __syncwarp();
     }
+    if constexpr (!BATCH) {
 #pragma unroll
-    for (int q = 0; q < 9; ++q) Wacc[q] = warp_sum(Wacc[q]);
-    if (lane == 0)
+        for (int q = 0; q < 9; ++q) Wacc[q] = warp_sum(Wacc[q]);
+        if (lane == 0)
 #pragma unroll
-        for (int q = 0; q < 9; ++q) wred[warp][q] = Wacc[q];
-    __syncthreads();
-    if (threadIdx.x < 9) {
-        double s = 0.0;
-        for (int w = 0; w < nwarps; ++w) s += wred[w][threadIdx.x];
-        out.wpart[blockIdx.x * 9 + threadIdx.x] = s;
+            for (int q = 0; q < 9; ++q) wred[warp][q] = Wacc[q];
+        __syncthreads();
+        if (threadIdx.x < 9) {
+            double s = 0.0;
+            for (int w = 0; w < nwarps; ++w) s += wred[w][threadIdx.x];
+            out.wpart[blockIdx.x * 9 + threadIdx.x] = s;
+        }
     }
 }
 
@@ -777,9 +817,9 @@ Launch plan_backward(const DescParams& dp) {
     return {warps, (size_t)warps * per_warp * 8, per_warp};
 }
 
-template <int LMAX, int TN, int TL, bool ENV, int EXNB>
+template <int LMAX, int TN, int TL, bool ENV, int EXNB, bool BATCH>
 int launch_forward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src, const int* row_of, double* phat,
-                   double* cbuf, double* pnorm, unsigned char* sflag, cudaStream_t st) {
+                   double* cbuf, double* pnorm, unsigned char* sflag, cudaStream_t st, const BatchGeom* bg) {
     const DescParams& dp = h->dp;
     // row of a neighbour in the chunk buffer: f padded to whole n tiles, Y padded to whole lm tiles
     const int nbp = ((dp.nb + TN - 1) / TN) * TN;
@@ -794,7 +834,7 @@ int launch_forward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src,
         set_error("descriptor too large for shared memory (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
         return SGPR_ERR_INVALID;
     }
-    auto kern = desc_forward_kernel<LMAX, TN, TL, ENV, EXNB>;
+    auto kern = desc_forward_kernel<LMAX, TN, TL, ENV, EXNB, BATCH>;
     SGPR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem));
     int grid = (n_env + L.warps - 1) / L.warps;
     // one resident wave: environments are dealt round-robin to warps, so a grid that is not a whole number of waves
@@ -813,23 +853,24 @@ int launch_forward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src,
     kern<<<grid, L.warps * 32, L.smem, st>>>(dp, g, n_env, src, row_of, h->ptab.as<unsigned>(), h->nnlk.as<double>(), phat,
                                              cbuf, pnorm, sflag, L.per_warp, stride, nbp,
                                              (!ENV && h->use_i8_now) ? h->p8.as<signed char>() : nullptr,
-                                             (long long)h->i8_cap_rows * h->i8_kp1, h->i8_kp1);
+                                             (long long)h->i8_cap_rows * h->i8_kp1, h->i8_kp1, bg ? bg->cells : nullptr,
+                                             bg ? bg->astr : nullptr);
     SGPR_CUDA(cudaGetLastError());
     h->stats.kernel_launches += 1;
     return SGPR_OK;
 }
 
-template <bool ENV>
+template <bool ENV, bool BATCH = false>
 int dispatch_forward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src, const int* row_of, double* phat,
-                     double* cbuf, double* pnorm, unsigned char* sflag, cudaStream_t st) {
+                     double* cbuf, double* pnorm, unsigned char* sflag, cudaStream_t st, const BatchGeom* bg = nullptr) {
     const int lmax = h->dp.lmax, nb = h->dp.nb;
     // (LMAX bucket, n-tile, lm-tile): ceil(L2/TL) * ceil(nb/TN) <= 32 lanes
-#define FWD(LM, TN, TL) return launch_forward<LM, TN, TL, ENV, 0>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st)
+#define FWD(LM, TN, TL) return launch_forward<LM, TN, TL, ENV, 0, BATCH>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st, bg)
     if (lmax == 3 && nb == 4)   // the reference's default descriptor
-        return launch_forward<3, 2, 1, ENV, 4>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st);
+        return launch_forward<3, 2, 1, ENV, 4, BATCH>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st, bg);
     if (lmax <= 3 && nb <= 4) FWD(3, 2, 1);
     if (lmax == 6 && nb == 9)   // the high-resolution configuration (lmax 6, nmax 8)
-        return launch_forward<6, 3, 5, ENV, 9>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st);
+        return launch_forward<6, 3, 5, ENV, 9, BATCH>(h, g, n_env, src, row_of, phat, cbuf, pnorm, sflag, st, bg);
     if (lmax <= 3 && nb <= 8) FWD(3, 4, 1);
     if (lmax <= 3) FWD(3, 6, 1);
     if (lmax <= 6 && nb <= 6) FWD(6, 2, 5);
@@ -841,21 +882,22 @@ int dispatch_forward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& sr
     return SGPR_ERR_INVALID;
 }
 
-template <int LMAX, int NB, bool EXACT>
+template <int LMAX, int NB, bool EXACT, bool BATCH>
 int launch_backward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src, const BackOut& out, int grid,
-                    cudaStream_t st) {
+                    cudaStream_t st, const BatchGeom* bg) {
     const DescParams& dp = h->dp;
     Launch L = plan_backward(dp);
     if ((size_t)L.per_warp * 8 > 200 * 1024) {
         set_error("descriptor too large for shared memory (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
         return SGPR_ERR_INVALID;
     }
-    auto kern = desc_backward_kernel<LMAX, NB, EXACT>;
+    auto kern = desc_backward_kernel<LMAX, NB, EXACT, BATCH>;
     SGPR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem));
     kern<<<grid, L.warps * 32, L.smem, st>>>(dp, g, n_env, src, h->rowof.as<int>() + (h->last_N + 1),
                                              h->gvec.as<double>(), h->phat.as<double>(), h->ttab.as<double>(),
                                              h->erow.as<double>(), h->prow.as<double>(), h->xi, h->cbuf.as<double>(),
-                                             h->sflag.as<unsigned char>(), out, L.per_warp);
+                                             h->sflag.as<unsigned char>(), out, L.per_warp, bg ? bg->cells : nullptr,
+                                             bg ? bg->astr : nullptr, bg ? h->wenv.as<double>() : nullptr);
     SGPR_CUDA(cudaGetLastError());
     h->stats.kernel_launches += 1;
     return SGPR_OK;
@@ -873,7 +915,7 @@ int descriptor_forward_env(sgpr_context* h, int M, const long long* env_first_d,
     return dispatch_forward<true>(h, g, M, src, row_of_d, phat_d, nullptr, nullptr, nullptr, st);
 }
 
-int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st) {
+int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st, const BatchGeom* bg) {
     const int na = (int)h->n_active;
     const DescParams& dp = h->dp;
     SGPR_TRY(h->cbuf.ensure(sizeof(double) * ((size_t)na * dp.csize + 1)));
@@ -885,14 +927,36 @@ int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st) {
     src.pairs = h->nl_pairs.as<PairRec>();
     src.nl_first = h->nl_first.as<long long>();
     src.active = h->active_all ? nullptr : h->active_list.as<int>();
+    if (bg)
+        return dispatch_forward<false, true>(h, g, na, src, h->rowof.as<int>() + (h->last_N + 1), h->phat.as<double>(),
+                                             h->cbuf.as<double>(), h->prow.as<double>(), h->sflag.as<unsigned char>(), st, bg);
     return dispatch_forward<false>(h, g, na, src, h->rowof.as<int>() + (h->last_N + 1), h->phat.as<double>(),
                                    h->cbuf.as<double>(), h->prow.as<double>(), h->sflag.as<unsigned char>(), st);
 }
 
 int backward_grid(sgpr_context* h) { return h->sm_count * 16; }
 
+template <bool BATCH>
+static int dispatch_backward(sgpr_context* h, const Geom& g, int na, const EnvSrc& src, const BackOut& out, cudaStream_t st,
+                             const BatchGeom* bg) {
+    const int grid = backward_grid(h);
+    const int lmax = h->dp.lmax, nb = h->dp.nb;
+#define BWD(LM, NBB) return launch_backward<LM, NBB, false, BATCH>(h, g, na, src, out, grid, st, bg)
+    if (lmax == 3 && nb == 4) return launch_backward<3, 4, true, BATCH>(h, g, na, src, out, grid, st, bg);   // the reference's default
+    if (lmax <= 3 && nb <= 4) BWD(3, 4);
+    if (lmax == 6 && nb == 9) return launch_backward<6, 9, true, BATCH>(h, g, na, src, out, grid, st, bg);
+    if (lmax <= 3 && nb <= 8) BWD(3, 8);
+    if (lmax <= 6 && nb <= 6) BWD(6, 6);
+    if (lmax <= 6 && nb <= 9) BWD(6, 9);
+    if (lmax <= 6 && nb <= 12) BWD(6, 12);
+    if (lmax <= 8 && nb <= 12) BWD(8, 12);
+#undef BWD
+    set_error("unsupported descriptor size lmax=%d nmax=%d", lmax, nb - 1);
+    return SGPR_ERR_INVALID;
+}
+
 int descriptor_backward_atoms(sgpr_context* h, const Geom& g, const unsigned char* owned_d, cudaStream_t st,
-                              const PeerForces* peers) {
+                              const PeerForces* peers, const BatchGeom* bg) {
     const int na = (int)h->n_active;
     if (na == 0) return SGPR_OK;
     EnvSrc src{};
@@ -906,20 +970,7 @@ int descriptor_backward_atoms(sgpr_context* h, const Geom& g, const unsigned cha
     out.wpart = h->wpart.as<double>();
     out.owned = owned_d;
     out.sp_on = h->sp_on.as<unsigned char>();
-    const int grid = backward_grid(h);
-    const int lmax = h->dp.lmax, nb = h->dp.nb;
-#define BWD(LM, NBB) return launch_backward<LM, NBB, false>(h, g, na, src, out, grid, st)
-    if (lmax == 3 && nb == 4) return launch_backward<3, 4, true>(h, g, na, src, out, grid, st);   // the reference's default
-    if (lmax <= 3 && nb <= 4) BWD(3, 4);
-    if (lmax == 6 && nb == 9) return launch_backward<6, 9, true>(h, g, na, src, out, grid, st);
-    if (lmax <= 3 && nb <= 8) BWD(3, 8);
-    if (lmax <= 6 && nb <= 6) BWD(6, 6);
-    if (lmax <= 6 && nb <= 9) BWD(6, 9);
-    if (lmax <= 6 && nb <= 12) BWD(6, 12);
-    if (lmax <= 8 && nb <= 12) BWD(8, 12);
-#undef BWD
-    set_error("unsupported descriptor size lmax=%d nmax=%d", lmax, nb - 1);
-    return SGPR_ERR_INVALID;
+    return bg ? dispatch_backward<true>(h, g, na, src, out, st, bg) : dispatch_backward<false>(h, g, na, src, out, st, nullptr);
 }
 
 int unpack_descriptors(sgpr_context* h, long long rows, const double* packed_d, const int* src_row_d, double* full_d,

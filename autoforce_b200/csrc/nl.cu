@@ -105,8 +105,8 @@ __global__ void frac_minmax_kernel(int64_t N, const double* __restrict__ pos, Ge
         }
 }
 
-int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double* cell_h, const int32_t* pbc_h,
-                   cudaStream_t st, Geom* g) {
+// completed cell, its inverse and the distances between opposite faces (host)
+static int geom_cell(const double* cell_h, const int32_t* pbc_h, double rc, Geom* g, double* hface) {
     for (int i = 0; i < 9; ++i) g->cell[i] = cell_h[i];
     for (int c = 0; c < 3; ++c) g->pbc[c] = pbc_h[c] ? 1 : 0;
     complete_cell(g->cell);
@@ -124,27 +124,13 @@ int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double
     const double* rec[3] = {bc, ca, ab};
     for (int c = 0; c < 3; ++c)
         for (int k = 0; k < 3; ++k) g->inv[k * 3 + c] = rec[c][k] / vol;
-    g->rc = h->dp.rc;
-    double hface[3];
+    g->rc = rc;
     for (int c = 0; c < 3; ++c) hface[c] = fabs(vol) / norm3(rec[c]);
-    bool open = !(g->pbc[0] && g->pbc[1] && g->pbc[2]);
-    double lo[3] = {0, 0, 0}, hi[3] = {1, 1, 1};
-    if (open && N > 0) {
-        int nblk = 64;
-        SGPR_TRY(h->misc.ensure(sizeof(double) * 6 * nblk));
-        frac_minmax_kernel<<<nblk, 256, 0, st>>>(N, pos_d, *g, h->misc.as<double>());
-        std::vector<double> part(6 * nblk);
-        SGPR_CUDA(cudaMemcpyAsync(part.data(), h->misc.p, sizeof(double) * 6 * nblk, cudaMemcpyDeviceToHost, st));
-        SGPR_CUDA(cudaStreamSynchronize(st));
-        for (int c = 0; c < 3; ++c) {
-            lo[c] = 1e300;
-            hi[c] = -1e300;
-            for (int b = 0; b < nblk; ++b) {
-                lo[c] = fmin(lo[c], part[b * 6 + c]);
-                hi[c] = fmax(hi[c], part[b * 6 + 3 + c]);
-            }
-        }
-    }
+    return SGPR_OK;
+}
+
+// bins and stencil reach from the fractional bounds lo / hi of the non-periodic axes (host)
+static void geom_bins(Geom* g, const double* hface, const double* lo, const double* hi, int64_t N) {
     const double rcs = g->rc * (1.0 + 1e-7);
     for (int c = 0; c < 3; ++c) {
         if (g->pbc[c]) {
@@ -182,6 +168,108 @@ int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double
         g->nb[c] = nb;
     }
     g->ncell = g->nb[0] * g->nb[1] * g->nb[2];
+}
+
+int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double* cell_h, const int32_t* pbc_h,
+                   cudaStream_t st, Geom* g) {
+    double hface[3];
+    SGPR_TRY(geom_cell(cell_h, pbc_h, h->dp.rc, g, hface));
+    bool open = !(g->pbc[0] && g->pbc[1] && g->pbc[2]);
+    double lo[3] = {0, 0, 0}, hi[3] = {1, 1, 1};
+    if (open && N > 0) {
+        int nblk = 64;
+        SGPR_TRY(h->misc.ensure(sizeof(double) * 6 * nblk));
+        frac_minmax_kernel<<<nblk, 256, 0, st>>>(N, pos_d, *g, h->misc.as<double>());
+        std::vector<double> part(6 * nblk);
+        SGPR_CUDA(cudaMemcpyAsync(part.data(), h->misc.p, sizeof(double) * 6 * nblk, cudaMemcpyDeviceToHost, st));
+        SGPR_CUDA(cudaStreamSynchronize(st));
+        for (int c = 0; c < 3; ++c) {
+            lo[c] = 1e300;
+            hi[c] = -1e300;
+            for (int b = 0; b < nblk; ++b) {
+                lo[c] = fmin(lo[c], part[b * 6 + c]);
+                hi[c] = fmax(hi[c], part[b * 6 + 3 + c]);
+            }
+        }
+    }
+    geom_bins(g, hface, lo, hi, N);
+    return SGPR_OK;
+}
+
+// Bounds of the fractional coordinates of the batch's non-periodic structures: one block per structure (list `which`).
+__global__ void batch_minmax_kernel(const int* __restrict__ which, const long long* __restrict__ first,
+                                    const double* __restrict__ pos, const Geom* __restrict__ geoms, double* __restrict__ out) {
+    __shared__ double smin[3][256], smax[3][256];
+    const int b = which[blockIdx.x];
+    const Geom& g = geoms[b];
+    double mn[3] = {1e300, 1e300, 1e300}, mx[3] = {-1e300, -1e300, -1e300};
+    for (long long i = first[b] + threadIdx.x; i < first[b + 1]; i += blockDim.x) {
+        double x = pos[3 * i], y = pos[3 * i + 1], z = pos[3 * i + 2];
+        for (int c = 0; c < 3; ++c) {
+            double f = x * g.inv[c] + y * g.inv[3 + c] + z * g.inv[6 + c];
+            mn[c] = fmin(mn[c], f);
+            mx[c] = fmax(mx[c], f);
+        }
+    }
+    for (int c = 0; c < 3; ++c) {
+        smin[c][threadIdx.x] = mn[c];
+        smax[c][threadIdx.x] = mx[c];
+    }
+    __syncthreads();
+    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s)
+            for (int c = 0; c < 3; ++c) {
+                smin[c][threadIdx.x] = fmin(smin[c][threadIdx.x], smin[c][threadIdx.x + s]);
+                smax[c][threadIdx.x] = fmax(smax[c][threadIdx.x], smax[c][threadIdx.x + s]);
+            }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0)
+        for (int c = 0; c < 3; ++c) {
+            out[blockIdx.x * 6 + c] = smin[c][0];
+            out[blockIdx.x * 6 + 3 + c] = smax[c][0];
+        }
+}
+
+int build_geometry_batch(sgpr_context* h, int B, const int64_t* first_h, const double* pos_d, const double* cell_h,
+                         const int32_t* pbc_h, cudaStream_t st, std::vector<Geom>* gs) {
+    gs->assign(B, Geom{});
+    std::vector<double> hface(3 * (size_t)B), lohi(6 * (size_t)B);
+    std::vector<int> which;
+    for (int b = 0; b < B; ++b) {
+        const int rc = geom_cell(cell_h + 9 * (size_t)b, pbc_h + 3 * (size_t)b, h->dp.rc, &(*gs)[b], &hface[3 * (size_t)b]);
+        if (rc != SGPR_OK) {
+            const std::string msg = sgpr_last_error();
+            set_error("structure %d: %s", b, msg.c_str());
+            return rc;
+        }
+        for (int c = 0; c < 3; ++c) {
+            lohi[6 * (size_t)b + c] = 0.0;
+            lohi[6 * (size_t)b + 3 + c] = 1.0;
+        }
+        const Geom& g = (*gs)[b];
+        if (!(g.pbc[0] && g.pbc[1] && g.pbc[2]) && first_h[b + 1] > first_h[b]) which.push_back(b);
+    }
+    if (!which.empty()) {
+        const int n = (int)which.size();
+        SGPR_TRY(h->b_geom.ensure(sizeof(Geom) * (size_t)B));
+        SGPR_TRY(h->b_first.ensure(sizeof(long long) * ((size_t)B + 1)));
+        SGPR_TRY(h->b_bins.ensure(sizeof(int) * ((size_t)B + 1)));
+        SGPR_TRY(h->misc.ensure(sizeof(double) * 6 * (size_t)n));
+        SGPR_CUDA(cudaMemcpyAsync(h->b_geom.p, gs->data(), sizeof(Geom) * (size_t)B, cudaMemcpyHostToDevice, st));
+        SGPR_CUDA(cudaMemcpyAsync(h->b_first.p, first_h, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
+        SGPR_CUDA(cudaMemcpyAsync(h->b_bins.p, which.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, st));
+        batch_minmax_kernel<<<n, 256, 0, st>>>(h->b_bins.as<int>(), h->b_first.as<long long>(), pos_d, h->b_geom.as<Geom>(),
+                                               h->misc.as<double>());
+        SGPR_CUDA(cudaGetLastError());
+        std::vector<double> part(6 * (size_t)n);
+        SGPR_CUDA(cudaMemcpyAsync(part.data(), h->misc.p, sizeof(double) * 6 * (size_t)n, cudaMemcpyDeviceToHost, st));
+        SGPR_CUDA(cudaStreamSynchronize(st));
+        for (int k = 0; k < n; ++k)
+            for (int q = 0; q < 6; ++q) lohi[6 * (size_t)which[k] + q] = part[6 * (size_t)k + q];
+    }
+    for (int b = 0; b < B; ++b)
+        geom_bins(&(*gs)[b], &hface[3 * (size_t)b], &lohi[6 * (size_t)b], &lohi[6 * (size_t)b + 3], first_h[b + 1] - first_h[b]);
     return SGPR_OK;
 }
 
@@ -485,6 +573,114 @@ int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_
 }
 
 // ---------------------------------------------------------------------------------
+// cell sort of a batch: keys (bin_base[b] + bin) * S + species -- structure-major, so every structure is one contiguous
+// range of the cell order and of each species' rows, and the second (species-major) scan still gives one row block per
+// central species for the whole batch
+// ---------------------------------------------------------------------------------
+// structure of atom i: the last b with first[b] <= i (empty structures are skipped)
+__device__ __forceinline__ int batch_of(const long long* __restrict__ first, int B, long long i) {
+    int lo = 0, hi = B;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (first[mid] <= i) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void batch_bin_count_kernel(int64_t N, const double* __restrict__ pos, const int32_t* __restrict__ Z,
+                                       const int* __restrict__ ztab, BatchGeom bg, int S, int* __restrict__ cnt,
+                                       int* __restrict__ key_out, int* __restrict__ rank_out) {
+    int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int b = batch_of(bg.first, bg.B, i);
+    int z = Z[i];
+    int s = (z >= 0 && z < 128) ? ztab[z] : -1;
+    if (s < 0) {
+        atomicMin(&bg.err[0], ((unsigned long long)b << 32) | (unsigned)z);
+        s = 0;
+    }
+    int bn[3], w[3];
+    frac_bin(bg.geoms[b], pos[3 * i], pos[3 * i + 1], pos[3 * i + 2], bn, w);
+    if (abs(w[0]) > 120 || abs(w[1]) > 120 || abs(w[2]) > 120) atomicMin(&bg.err[1], (unsigned long long)b);
+    const Geom& g = bg.geoms[b];
+    int bin = bg.bin_base[b] + (bn[0] * g.nb[1] + bn[1]) * g.nb[2] + bn[2];
+    int key = bin * S + s;
+    key_out[i] = key;
+    rank_out[i] = atomicAdd(&cnt[key], 1);
+}
+
+// cell-ordered atom records (runs already sorted by original index), global bin, row, structure
+__global__ void batch_gather_kernel(int64_t N, const double* __restrict__ pos, const int* __restrict__ key,
+                                    const int* __restrict__ order, const int* __restrict__ cstart,
+                                    const int* __restrict__ rstartT, BatchGeom bg, int S, AtomRec* __restrict__ atoms,
+                                    int* __restrict__ abin, int* __restrict__ rowof) {
+    int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (c >= N) return;
+    int i = order[c];
+    int k = key[i];
+    int bin = k / S, s = k - bin * S;
+    const int b = batch_of(bg.first, bg.B, i);
+    double x = pos[3 * (int64_t)i], y = pos[3 * (int64_t)i + 1], z = pos[3 * (int64_t)i + 2];
+    int b3[3], w[3];
+    frac_bin(bg.geoms[b], x, y, z, b3, w);
+    AtomRec r;
+    r.x = x;
+    r.y = y;
+    r.z = z;
+    r.meta = (unsigned long long)(unsigned int)i | ((unsigned long long)s << 32) |
+             ((unsigned long long)(w[0] + 128) << 40) | ((unsigned long long)(w[1] + 128) << 48) |
+             ((unsigned long long)(w[2] + 128) << 56);
+    atoms[c] = r;
+    abin[c] = bin;
+    rowof[c] = rstartT[s * bg.ncell + bin] + (int)(c - cstart[k]);
+    bg.astr[c] = b;
+}
+
+// Same workspace layout as cell_sort, plus h->astr.  Errors are reported by batch_neighbor_build's sizing step.
+int batch_cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const BatchGeom& bg, cudaStream_t st) {
+    const int S = h->S;
+    const int nkeys = bg.ncell * S;
+    SGPR_TRY(h->cnt.ensure(sizeof(int) * (nkeys + 1)));
+    SGPR_TRY(h->cstart.ensure(sizeof(int) * (nkeys + 1)));
+    SGPR_TRY(h->rstart.ensure(sizeof(int) * 2 * (nkeys + 1)));
+    SGPR_TRY(h->keyrank.ensure(sizeof(int) * 2 * (N + 1)));
+    SGPR_TRY(h->order.ensure(sizeof(int) * (N + 1)));
+    SGPR_TRY(h->atoms.ensure(sizeof(AtomRec) * (N + 1)));
+    SGPR_TRY(h->rowof.ensure(sizeof(int) * 2 * (N + 1)));
+    int* cnt = h->cnt.as<int>();
+    int* cstart = h->cstart.as<int>();
+    int* cntT = h->rstart.as<int>();
+    int* rstartT = cntT + (nkeys + 1);
+    int* key = h->keyrank.as<int>();
+    int* rank = key + (N + 1);
+    SGPR_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (nkeys + 1), st));
+    SGPR_CUDA(cudaMemsetAsync(h->errflag.p, 0, sizeof(int) * 4, st));
+    SGPR_CUDA(cudaMemsetAsync(bg.err, 0x7f, sizeof(unsigned long long) * 2, st));
+    const int T = 256;
+    const int nblkN = (int)((N + T - 1) / T);
+    const int nblkK = (nkeys + T - 1) / T;
+    if (N > 0) batch_bin_count_kernel<<<nblkN, T, 0, st>>>(N, pos_d, Z_d, h->ztab.as<int>(), bg, S, cnt, key, rank);
+    if (nkeys + 1 <= kScanMaxKeys) {
+        key_scan_kernel<<<2, kScanThreads, 0, st>>>(nkeys, bg.ncell, S, cnt, cstart, rstartT);
+    } else {
+        SGPR_CUDA(cudaMemsetAsync(cntT, 0, sizeof(int) * (nkeys + 1), st));
+        transpose_cnt_kernel<<<nblkK, T, 0, st>>>(bg.ncell, S, cnt, cntT);
+        SGPR_TRY(scan_exclusive_int(h, cnt, cstart, nkeys + 1, st));
+        SGPR_TRY(scan_exclusive_int(h, cntT, rstartT, nkeys + 1, st));
+    }
+    if (N > 0) {
+        scatter_order_kernel<<<nblkN, T, 0, st>>>(N, key, rank, cstart, h->order.as<int>());
+        sort_runs_kernel<<<nblkK, T, 0, st>>>(nkeys, cstart, h->order.as<int>());
+        batch_gather_kernel<<<nblkN, T, 0, st>>>(N, pos_d, key, h->order.as<int>(), cstart, rstartT, bg, S,
+                                                 h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->rowof.as<int>() + (N + 1));
+    }
+    h->stats.kernel_launches += 5;
+    SGPR_CUDA(cudaGetLastError());
+    return SGPR_OK;
+}
+
+// ---------------------------------------------------------------------------------
 // neighbour search: one warp per atom, lanes over the candidates of a bin run
 // ---------------------------------------------------------------------------------
 // exact image shift  ((S0*c0 + S1*c1) + S2*c2)  in the reference's rounding sequence (no FMA)
@@ -544,20 +740,37 @@ constexpr int kMaskSlots = 64;
 // per-lane counters, one warp reduction at the end), accept masks per candidate batch and halo
 // marks.  FILL pass: replays the traversal, takes the accept bits from the masks and writes the
 // pairs species-sorted (per-species ballots give each accepted candidate its rank).
-template <bool FILL, int NS>
+// the geometry an environment's search uses: the call's, or (batch) that of the centre's structure
+template <bool BATCH>
+__device__ __forceinline__ const Geom& env_geom(const Geom& g, const BatchGeom& bg, int b) {
+    if constexpr (BATCH)
+        return bg.geoms[b];
+    else
+        return g;
+}
+
+// BATCH: a batch of structures (sgpr_predict_batch) -- each environment reads its structure's Geom, and its stencil
+// stays inside that structure's bins (bg.bin_base); same traversal, pair_test and pair order as a call on the structure
+template <bool FILL, int NS, bool BATCH = false>
 __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, const int* __restrict__ active,
                                                        const AtomRec* __restrict__ atoms, const int* __restrict__ abin,
-                                                       const int* __restrict__ cstart, Geom g, int S,
+                                                       const int* __restrict__ cstart, Geom g_call, int S,
                                                        int* __restrict__ nl_cnt, const long long* __restrict__ nl_first,
                                                        PairRec* __restrict__ pairs, unsigned char* __restrict__ mark,
-                                                       unsigned* __restrict__ masks) {
+                                                       unsigned* __restrict__ masks, BatchGeom bg = BatchGeom{}) {
     const int lane = threadIdx.x & 31;
     int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (wid >= n_env) return;
     wid += env0;  // index into the active list / the neighbour-list rows
     const int c = active ? active[wid] : wid;
+    int sb = 0, bbase = 0;
+    if constexpr (BATCH) {
+        sb = bg.astr[c];
+        bbase = bg.bin_base[sb];
+    }
+    const Geom& g = env_geom<BATCH>(g_call, bg, sb);
     const AtomRec ai = atoms[c];
-    int bin = abin[c];
+    int bin = abin[c] - bbase;
     const int bz = bin % g.nb[2];
     bin /= g.nb[2];
     const int by = bin % g.nb[1];
@@ -598,8 +811,8 @@ __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, cons
                     if (!wrap_bin(bz + dz, g.nb[2], g.pbc[2], nz, sz)) continue;
                     nz_last = nz;
                 }
-                const int b2 = (nx * g.nb[1] + ny) * g.nb[2] + nz;
-                const int b3 = (nx * g.nb[1] + ny) * g.nb[2] + nz_last;
+                const int b2 = bbase + (nx * g.nb[1] + ny) * g.nb[2] + nz;
+                const int b3 = bbase + (nx * g.nb[1] + ny) * g.nb[2] + nz_last;
                 const int beg = cstart[b2 * S], end = cstart[b3 * S + S];
                 double sh0 = 0.0, sh1 = 0.0, sh2 = 0.0;
                 if (!FILL) shift_vec(g, sx, sy, sz, sh0, sh1, sh2);
@@ -964,7 +1177,19 @@ static bool use_bin_kernels(const sgpr_context* h, const Geom& g) { return h->nl
 template <bool FILL>
 static void launch_neighbor(int nblk, int T, cudaStream_t st, int S, int env0, int n_env, const int* active,
                             const AtomRec* atoms, const int* abin, const int* cstart, const Geom& g, int* nl_cnt,
-                            const long long* nl_first, PairRec* pairs, unsigned char* mark, unsigned* masks) {
+                            const long long* nl_first, PairRec* pairs, unsigned char* mark, unsigned* masks,
+                            const BatchGeom* bg = nullptr) {
+    if (bg) {
+        if (S <= 1)
+            neighbor_kernel<FILL, 1, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
+        else if (S <= 2)
+            neighbor_kernel<FILL, 2, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
+        else if (S <= 4)
+            neighbor_kernel<FILL, 4, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
+        else
+            neighbor_kernel<FILL, 8, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
+        return;
+    }
     if (S <= 1)
         neighbor_kernel<FILL, 1><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks);
     else if (S <= 2)
@@ -986,9 +1211,9 @@ __global__ void row_total_kernel(int n, int S, const int* __restrict__ nl_cnt, l
 
 // contig_c0 >= 0: environments env0 .. env0+n_env-1 are the atoms contig_c0 .. of the cell order
 static int launch_count(sgpr_context* h, int env0, int n_env, const Geom& g, unsigned char* mark, cudaStream_t st,
-                        int contig_c0) {
+                        int contig_c0, const BatchGeom* bg = nullptr) {
     if (n_env <= 0) return SGPR_OK;
-    if (contig_c0 >= 0 && use_bin_kernels(h, g)) {
+    if (contig_c0 >= 0 && !bg && use_bin_kernels(h, g)) {
         launch_neighbor_bins<false>(st, h->S, contig_c0, contig_c0 + n_env, env0, h->atoms.as<AtomRec>(), h->cstart.as<int>(), g,
                                     h->nl_cnt.as<int>(), nullptr, nullptr, mark, h->nl_masks.as<unsigned>(), nullptr);
         h->stats.kernel_launches += 1;
@@ -998,7 +1223,7 @@ static int launch_count(sgpr_context* h, int env0, int n_env, const Geom& g, uns
     const int nblk = (int)(((int64_t)n_env * 32 + T - 1) / T);
     launch_neighbor<false>(nblk, T, st, h->S, env0, n_env, h->active_all ? nullptr : h->active_list.as<int>(),
                            h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->cstart.as<int>(), g, h->nl_cnt.as<int>(), nullptr,
-                           nullptr, mark, h->nl_masks.as<unsigned>());
+                           nullptr, mark, h->nl_masks.as<unsigned>(), bg);
     h->stats.kernel_launches += 1;
     return SGPR_OK;
 }
@@ -1010,6 +1235,21 @@ static int check_err_flags(const int* err) {
     }
     if (err[0] == 2) {
         set_error("an atom lies more than 120 cells outside the unit cell; wrap positions first");
+        return SGPR_ERR_GEOMETRY;
+    }
+    return SGPR_OK;
+}
+
+// batch errors name the first structure that failed (batch_bin_count_kernel)
+static int check_batch_err(const unsigned long long* berr) {
+    const unsigned long long none = 0x7f7f7f7f7f7f7f7full;
+    if (berr[0] != none) {
+        set_error("structure %d: atomic number %d is not in the handle's species table", (int)(berr[0] >> 32),
+                  (int)(unsigned)(berr[0] & 0xffffffffull));
+        return SGPR_ERR_SPECIES;
+    }
+    if (berr[1] != none) {
+        set_error("structure %d: an atom lies more than 120 cells outside the unit cell; wrap positions first", (int)berr[1]);
         return SGPR_ERR_GEOMETRY;
     }
     return SGPR_OK;
@@ -1084,7 +1324,7 @@ __global__ void __launch_bounds__(1024) rows_scan_kernel(int na, int S, const in
 
 // row totals -> exclusive scan -> (sizing step: sync for pair count, error flags, species row ranges) -> fill
 static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int* row_first_src, int row_first_pitch,
-                     int64_t* n_pairs, int contig_c0, int n_contig, bool warm) {
+                     int64_t* n_pairs, int contig_c0, int n_contig, bool warm, const BatchGeom* bg = nullptr) {
     const int S = h->S;
     const int na = (int)h->n_active;
     SGPR_TRY(h->nl_first.ensure(sizeof(long long) * 2 * ((size_t)na + 1)));
@@ -1116,13 +1356,15 @@ static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int*
         }
     } else {
         int err[4] = {0, 0, 0, 0};
+        unsigned long long berr[2] = {0, 0};
         int rf[SGPR_MAX_SPECIES + 1];
         SGPR_CUDA(cudaMemcpyAsync(&total, first + na, sizeof(long long), cudaMemcpyDeviceToHost, st));
         SGPR_CUDA(cudaMemcpyAsync(err, h->errflag.p, sizeof(int) * 4, cudaMemcpyDeviceToHost, st));
+        if (bg) SGPR_CUDA(cudaMemcpyAsync(berr, bg->err, sizeof(berr), cudaMemcpyDeviceToHost, st));
         SGPR_CUDA(cudaMemcpy2DAsync(rf, sizeof(int), row_first_src, (size_t)row_first_pitch, sizeof(int), S + 1,
                                     cudaMemcpyDeviceToHost, st));
         SGPR_CUDA(cudaStreamSynchronize(st));
-        SGPR_TRY(check_err_flags(err));
+        SGPR_TRY(bg ? check_batch_err(berr) : check_err_flags(err));
         for (int s = 0; s <= S; ++s) h->row_first[s] = rf[s];
         h->row_first_host_valid = true;
         // capacity with head room: the following steps of a trajectory reuse it without asking the device
@@ -1133,7 +1375,7 @@ static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int*
         }
     }
     int done = 0;   // environments 0 .. n_contig-1 are a contiguous range of the cell order: block-per-bin fill
-    if (n_contig > 0 && use_bin_kernels(h, g)) {
+    if (n_contig > 0 && !bg && use_bin_kernels(h, g)) {
         SGPR_TRY(h->nl_run.ensure(sizeof(int) * ((size_t)n_contig * S + 1)));
         launch_neighbor_bins<true>(st, S, contig_c0, contig_c0 + n_contig, 0, h->atoms.as<AtomRec>(), h->cstart.as<int>(), g,
                                    h->nl_cnt.as<int>(), first, h->nl_pairs.as<PairRec>(), nullptr,
@@ -1144,7 +1386,7 @@ static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int*
         const int nblk = (int)(((int64_t)(na - done) * 32 + T - 1) / T);
         launch_neighbor<true>(nblk, T, st, S, done, na - done, h->active_all ? nullptr : h->active_list.as<int>(),
                               h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->cstart.as<int>(), g, h->nl_cnt.as<int>(), first,
-                              h->nl_pairs.as<PairRec>(), nullptr, h->nl_masks.as<unsigned>());
+                              h->nl_pairs.as<PairRec>(), nullptr, h->nl_masks.as<unsigned>(), bg);
     }
     h->stats.kernel_launches += lean ? 1 : 4;  // fill (+ row totals, cub scan (2) when not the one-kernel scan)
     SGPR_CUDA(cudaGetLastError());
@@ -1164,6 +1406,20 @@ int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, i
     const int nkeys = g.ncell * h->S;
     const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
     return nl_finish(h, g, st, rstartT, (int)sizeof(int) * g.ncell, n_pairs, 0, (int)N, warm);
+}
+
+// Neighbour list of all atoms of a batch: one warp per environment (batched neighbor_kernel), rows in the batch's cell
+// order, species row ranges from batch_cell_sort's species-major scan.  Always a sizing step.
+int batch_neighbor_build(sgpr_context* h, int64_t N, const BatchGeom& bg, cudaStream_t st, int64_t* n_pairs) {
+    h->active_all = true;
+    h->n_active = N;
+    SGPR_TRY(h->nl_cnt.ensure(sizeof(int) * ((size_t)N * h->S + 1)));
+    SGPR_TRY(h->nl_masks.ensure(sizeof(unsigned) * kMaskSlots * ((size_t)N + 1)));
+    const Geom unused{};
+    SGPR_TRY(launch_count(h, 0, (int)N, unused, nullptr, st, -1, &bg));
+    const int nkeys = bg.ncell * h->S;
+    const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
+    return nl_finish(h, unused, st, rstartT, (int)sizeof(int) * bg.ncell, n_pairs, 0, 0, false, &bg);
 }
 
 // ---------------------------------------------------------------------------------

@@ -94,6 +94,24 @@ struct I8Setup {
     int ncol[3][kMaxSpecies];
 };
 
+// Batched prediction (sgpr_predict_batch): per-structure geometry and indices, device pointers.  Structure b holds the
+// atoms first[b] .. first[b+1]-1 of the caller's order and, because the cell-sort keys are structure-major, the same
+// index range of the cell order; its bins are bin_base[b] .. bin_base[b+1]-1 of the batch's bin table.
+struct BatchGeom {
+    int B;
+    int ncell;                 // bins of the whole batch
+    const Geom* geoms;         // [B]   what build_geometry gives each structure alone
+    const long long* first;    // [B+1] atom offsets
+    const int* bin_base;       // [B+1]
+    const double* cells;       // [B,9] completed cells (image shifts of the descriptor kernels)
+    int* astr;                 // [N]   structure of cell-order atom c
+    unsigned long long* err;   // [2]   min (b << 32 | Z) over unknown species, min b over atoms too far outside their cell
+};
+
+// Number of DevBuf reallocations so far: CUDA graphs of warm steps bake the workspaces' addresses into their nodes and
+// must not outlive them (api.cu: predict_impl).
+unsigned long long buf_generation();
+
 // host-side mirror of a grow-only device buffer
 struct DevBuf {
     void* p = nullptr;
@@ -206,6 +224,7 @@ struct sgpr_context {
     };
     std::vector<GraphEntry> graphs;
     unsigned long long graph_clock = 0;
+    unsigned long long graph_gen = 0;   // sgpr::buf_generation() the graphs were captured under
     bool use_graph = true;          // SGPR_GRAPH=0 switches the replay off
     sgpr::DevBuf ptab, nnlk;  // packed-entry tables [D]
     sgpr::DevBuf ztab;        // [128] atomic number -> species
@@ -220,6 +239,8 @@ struct sgpr_context {
     sgpr::DevBuf phat, cbuf, pnorm, sflag, gmat, gvec, epart, wpart, fcell, misc;
     sgpr::DevBuf stage_pos, stage_z, stage_out;  // device staging for the host API
     sgpr::DevBuf p2p_local;                      // fused exchange step: [16] partial E/W + step counter
+    sgpr::DevBuf b_geom, b_first, b_bins, b_cell, b_err;   // batched prediction: BatchGeom arrays
+    sgpr::DevBuf astr, wenv;                     // batched prediction: structure per cell-order atom, [N,9] per-environment virials
     bool p2p_counter_init = false;
     void* pinned = nullptr;
     size_t pinned_bytes = 0;
@@ -243,6 +264,13 @@ namespace sgpr {
 // ---- nl.cu ------------------------------------------------------------------------
 int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double* cell_h, const int32_t* pbc_h,
                    cudaStream_t st, Geom* g);
+// every structure's Geom as build_geometry gives it alone (one segmented bounds kernel, one synchronisation when a
+// structure is not periodic on all axes)
+int build_geometry_batch(sgpr_context* h, int B, const int64_t* first_h, const double* pos_d, const double* cell_h,
+                         const int32_t* pbc_h, cudaStream_t st, std::vector<Geom>* gs);
+// structure-major cell sort + neighbour list of all atoms of a batch (sizing: synchronises the stream)
+int batch_cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const BatchGeom& bg, cudaStream_t st);
+int batch_neighbor_build(sgpr_context* h, int64_t N, const BatchGeom& bg, cudaStream_t st, int64_t* n_pairs);
 int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const Geom& g, cudaStream_t st);
 // warm = true: no device-to-host copy, no synchronisation -- pair count, error flags and species row ranges stay on
 // the device (status_d, row_first_d); needs h->pairs_cap from an earlier sizing step; *n_pairs is then not set
@@ -255,7 +283,7 @@ int scan_exclusive_ll(sgpr_context* h, const long long* in, long long* out, int 
 int upload_harm_coef();
 int descriptor_forward_env(sgpr_context* h, int M, const long long* env_first_d, const double* env_r_d,
                            const unsigned char* env_sp_d, const int* row_of_d, double* phat_d, cudaStream_t st);
-int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st);
+int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st, const BatchGeom* bg = nullptr);
 // peer-memory force exchange: neighbour forces go to the owner rank's buffer (peer_f[r] valid on this device)
 struct PeerForces {
     double* peer_f[SGPR_MAX_RANKS];
@@ -266,8 +294,9 @@ struct PeerForces {
     const long long* parity_src;      // nullptr: peer_f as given
     long long parity_stride;          // doubles between the two buffers
 };
+// bg: batched step -- image shifts from the centre's structure, per-environment virials into h->wenv [N,9]
 int descriptor_backward_atoms(sgpr_context* h, const Geom& g, const unsigned char* owned_d, cudaStream_t st,
-                              const PeerForces* peers = nullptr);
+                              const PeerForces* peers = nullptr, const BatchGeom* bg = nullptr);
 // fused exchange step (api.cu: sgpr_p2p_step)
 struct P2PPeers {
     double* mail[SGPR_MAX_RANKS];     // mailbox block of every rank, mapped on this device

@@ -50,6 +50,8 @@ EXPORTS = {
                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_predict_host": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "sgpr_predict_batch": (c_int32, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_predict_p2p": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
                                    c_void_p, c_void_p, c_void_p]),
     "sgpr_p2p_collect": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -312,6 +314,52 @@ class SgprEngine:
         _check(self.lib, self.lib.sgpr_predict(self._h, N, c_void_p(pos_t.data_ptr()), c_void_p(z_t.data_ptr()), _ptr(cell_h),
                                                _ptr(pbc_h), rank, world, self._stream(), c_void_p(E.data_ptr()),
                                                c_void_p(F.data_ptr()), c_void_p(W.data_ptr()), None, None))
+        return E, F, W
+
+    def predict_batch(self, pos, numbers=None, first=None, cells=None, pbcs=None, want_beta=False):
+        """B structures in one call (``sgpr_predict_batch``): the same E, F, W (and beta) as ``predict`` on each structure
+        alone, at a fraction of the cost when the structures are small.
+
+        ``pos`` [Ntot,3] and ``numbers`` [Ntot] hold the structures one after the other (host arrays or CUDA tensors),
+        ``first`` [B+1] their atom offsets, ``cells`` [B,3,3] and ``pbcs`` [B,3] (or one value for all) their cells.
+        Alternatively ``pos`` may be a list of structures (anything with positions / cell / pbc / numbers, like
+        ase.Atoms) and the other arguments are left out.  Returns host numpy E [B], F [Ntot,3], W [B,3,3] (+ beta [Ntot]
+        when ``want_beta``)."""
+        import torch
+
+        if first is None:
+            images = list(pos)
+            if numbers is not None or cells is not None or pbcs is not None:
+                raise ValueError("pass either a list of structures or pos, numbers, first, cells, pbcs")
+            counts = [len(a.numbers) for a in images]
+            pos = np.concatenate([np.asarray(a.positions, dtype=np.float64).reshape(-1, 3) for a in images]) if images else np.zeros((0, 3))
+            numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images]) if images else np.zeros(0, dtype=np.int32)
+            first = np.concatenate([[0], np.cumsum(counts)])
+            cells = [np.asarray(a.cell, dtype=np.float64).reshape(3, 3) for a in images]
+            pbcs = [np.broadcast_to(np.asarray(a.pbc), (3,)) for a in images]
+        first_h = np.ascontiguousarray(first, dtype=np.int64).reshape(-1)
+        B = len(first_h) - 1
+        if B < 0:
+            raise ValueError("first must have B+1 >= 1 entries")
+        cell_h = np.ascontiguousarray(np.broadcast_to(np.asarray(cells, dtype=np.float64).reshape(-1, 9), (B, 9)))
+        pb = np.asarray(pbcs).astype(np.int32)
+        pbc_h = np.ascontiguousarray(np.broadcast_to(pb.reshape(-1, 3) if pb.size and pb.size % 3 == 0 else pb.reshape(-1, 1), (B, 3)))
+        pos_t, z_t = self._dev(pos, numbers)
+        N = z_t.numel()
+        if pos_t.shape[0] != N or first_h[-1] != N:
+            raise ValueError(f"first[-1] = {first_h[-1]} does not match {N} atoms")
+        dev = pos_t.device
+        E = torch.zeros(max(B, 1), dtype=torch.float64, device=dev)
+        F = torch.zeros((N, 3), dtype=torch.float64, device=dev)
+        W = torch.zeros((max(B, 1), 9), dtype=torch.float64, device=dev)
+        beta = torch.zeros(max(N, 1), dtype=torch.float64, device=dev) if want_beta else None
+        _check(self.lib, self.lib.sgpr_predict_batch(self._h, B, _ptr(first_h), c_void_p(pos_t.data_ptr()),
+                                                     c_void_p(z_t.data_ptr()), _ptr(cell_h), _ptr(pbc_h), self._stream(),
+                                                     c_void_p(E.data_ptr()), c_void_p(F.data_ptr()), c_void_p(W.data_ptr()),
+                                                     c_void_p(beta.data_ptr()) if want_beta else None))
+        E, F, W = E[:B].cpu().numpy(), F.cpu().numpy(), W[:B].cpu().numpy().reshape(B, 3, 3)
+        if want_beta:
+            return E, F, W, beta[:N].cpu().numpy()
         return E, F, W
 
     def predict_p2p(self, pos_t, z_t, cell, pbc, rank, world, peer_ptrs, ew):

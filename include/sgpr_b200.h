@@ -143,6 +143,22 @@ int sgpr_predict_host(sgpr_handle h, int64_t N, const double* pos_h, const int32
                       const double* cell_h, const int32_t* pbc_h, int32_t rank, int32_t world,
                       double* E_h, double* F_h, double* W_h, double* beta_h, uint8_t* owned_h);
 
+/* B independent structures under the handle's model in ONE call (calculator/active.py:425-611 once per structure):
+ * testing a model on a trajectory, the images of an NEB, scoring a data set -- structures of tens to hundreds of atoms,
+ * for which a call per structure is mostly fixed cost.
+ *   first_h [B+1]   int64 host CSR offsets: structure b = atoms first_h[b] .. first_h[b+1]-1 (0-atom structures allowed)
+ *   pos_d [Ntot,3], Z_d [Ntot]   device, structures concatenated (Ntot = first_h[B])
+ *   cell_h [B,9], pbc_h [B,3]    host, per structure, same conventions as sgpr_predict
+ *   E_d [B], W_d [B,9], F_d [Ntot,3], beta_d [Ntot] or NULL   device, caller's order
+ * Per structure, E, W and beta mean exactly what they mean in sgpr_predict, and do not depend on the rest of the batch.
+ * Errors: SGPR_ERR_INVALID for malformed first_h (not starting at 0, not monotone); SGPR_ERR_GEOMETRY / _SPECIES name
+ * the first structure that failed in sgpr_last_error().  B = 0 does nothing.
+ * Synchronises the stream once (sizing); never sharded; never replayed as a graph; leaves no state for
+ * sgpr_kernel_backward.  sgpr_get_stats reports the batch's totals. */
+int sgpr_predict_batch(sgpr_handle h, int32_t B, const int64_t* first_h, const double* pos_d, const int32_t* Z_d,
+                       const double* cell_h, const int32_t* pbc_h, void* stream,
+                       double* E_d, double* F_d, double* W_d, double* beta_d);
+
 /* Atom-sharded prediction with a PEER-MEMORY force exchange over NVLink instead of the halo recompute
  * of sgpr_predict(rank, world): every rank evaluates only the environments it owns and accumulates all
  * pair forces in its own buffer; what it accumulated for atoms of other ranks (the halo) is then added
