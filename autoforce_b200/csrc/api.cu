@@ -236,36 +236,6 @@ __global__ void final_reduce_kernel(int n_e, const double* __restrict__ epart, i
     }
 }
 
-// One inducing LCE as the cotangent of the kernel matrix (training-time kernels, similarity/universal.py:124-183):
-// rows of its central species get  g = xi k^(xi-1) z_hat  and  e = k^xi  (so that q_hat . g = xi e), all others zero.
-__global__ void column_seed_kernel(int n_rows, int r0, int r1, int D, int ldp, const double* __restrict__ phat,
-                                   const double* __restrict__ z, double xi, int xi_int, double* __restrict__ gvec,
-                                   double* __restrict__ erow) {
-    const int lane = threadIdx.x & 31;
-    const int wpb = blockDim.x >> 5;
-    for (int r = blockIdx.x * wpb + (threadIdx.x >> 5); r < n_rows; r += gridDim.x * wpb) {
-        double* g = gvec + (size_t)r * ldp;
-        if (r < r0 || r >= r1) {
-            for (int e = lane; e < ldp; e += 32) g[e] = 0.0;
-            if (lane == 0) erow[r] = 0.0;
-            continue;
-        }
-        const double* q = phat + (size_t)r * ldp;
-        double k = 0.0;
-        for (int e = lane; e < D; e += 32) k = fma(q[e], z[e], k);
-        for (int o = 16; o; o >>= 1) k += __shfl_xor_sync(0xffffffffu, k, o);
-        double pw = 1.0;
-        if (xi_int >= 1) {
-            for (int t = 1; t < xi_int; ++t) pw *= k;
-        } else {
-            pw = pow(k, xi - 1.0);
-        }
-        const double c = xi * pw;
-        for (int e = lane; e < ldp; e += 32) g[e] = e < D ? c * z[e] : 0.0;
-        if (lane == 0) erow[r] = pw * k;
-    }
-}
-
 __global__ void row_to_orig_kernel(int64_t N, const AtomRec* __restrict__ atoms, const int* __restrict__ rowof,
                                    int* __restrict__ orig_of_row) {
     int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -470,6 +440,19 @@ __global__ void batch_reduce_kernel(int B, const long long* __restrict__ first, 
         E[b] = e;
 #pragma unroll
         for (int q = 0; q < 9; ++q) W[9 * (size_t)b + q] = w[q];
+    }
+}
+
+// Ke[b, col] = sum over the atoms of structure b of K[i, m0 + col] (caller's order, lone-lone term included), one thread
+// per (structure, column), atoms in order: a structure's sums do not depend on the rest of the batch.
+__global__ void ke_reduce_kernel(int B, const long long* __restrict__ first, int M, int m0, int ncol,
+                                 const double* __restrict__ K, double* __restrict__ Ke) {
+    const long long n = (long long)B * ncol;
+    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < n; t += (long long)gridDim.x * blockDim.x) {
+        const int b = (int)(t / ncol), col = (int)(t - (long long)b * ncol);
+        double s = 0.0;
+        for (long long i = first[b]; i < first[b + 1]; ++i) s += K[i * M + m0 + col];
+        Ke[t] = s;
     }
 }
 
@@ -843,7 +826,7 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
                       &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
-                      &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv};
+                      &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr};
     for (DevBuf* b : bufs) b->release();
     if (h->pinned) cudaFreeHost(h->pinned);
     if (h->i8_probs_pinned) cudaFreeHost(h->i8_probs_pinned);
@@ -1702,8 +1685,33 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_backward(sgpr_
     return SGPR_OK;
 }
 
+// Inducing LCEs m0 <= m < m1 (caller's order) of the Jacobian kernel: sorted positions grouped by central species, then
+// their output columns, into h->jsel.  Excluded central species get no entries: their columns stay zero.
+static int upload_selection(sgpr_context* h, int m0, int m1, cudaStream_t st, JacTarget* t) {
+    std::vector<int> sel, col;
+    t->sel_first[0] = 0;
+    for (int s = 0; s < SGPR_MAX_SPECIES; ++s) {
+        if (s < h->S && h->dp.central_enabled[s])
+            for (int p = h->m_first[s]; p < h->m_first[s + 1]; ++p) {
+                const int m = h->ind_perm[p];
+                if (m >= m0 && m < m1) {
+                    sel.push_back(p);
+                    col.push_back(m - m0);
+                }
+            }
+        t->sel_first[s + 1] = (int)sel.size();
+    }
+    t->n_sel = (int)sel.size();
+    t->ncol = m1 - m0;
+    sel.insert(sel.end(), col.begin(), col.end());
+    SGPR_TRY(h->jsel.ensure(sizeof(int) * (sel.size() + 1)));
+    if (!sel.empty()) SGPR_CUDA(cudaMemcpyAsync(h->jsel.p, sel.data(), sizeof(int) * sel.size(), cudaMemcpyHostToDevice, st));
+    t->sel = h->jsel.as<int>();
+    return SGPR_OK;
+}
+
 // Training-time kernels of the structure of the LAST sgpr_kernel_forward against inducing LCEs m0 <= m < m1
-// (caller's order): the Jacobian of Ke[m] = sum_i K[i,m], one backward pass per LCE with a rank-1 cotangent.
+// (caller's order): the Jacobian of Ke[m] = sum_i K[i,m] for all of them in one launch (descriptor.cu: jacobian_kernel).
 extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian(sgpr_handle h, int32_t m0, int32_t m1, void* stream, double* J_d, double* W_d) {
     if (!h || !J_d || !W_d) {
         set_error("null argument");
@@ -1720,40 +1728,179 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian(sgpr_
     cudaStream_t st = (cudaStream_t)stream;
     SGPR_CUDA(cudaSetDevice(h->device));
     const int64_t N = h->last_N;
-    const Geom g = h->last_geom;
-    const size_t nrows = (size_t)h->n_active + 1;
-    const int nblk_b = backward_grid(h), nblk_x = 64;
-    SGPR_TRY(h->gvec.ensure(sizeof(double) * nrows * h->dp.ldp));
-    SGPR_TRY(h->erow.ensure(sizeof(double) * nrows));
-    SGPR_TRY(h->epart.ensure(sizeof(double) * (16 + 9 * nblk_x)));
-    SGPR_TRY(h->wpart.ensure(sizeof(double) * 9 * nblk_b));
-    SGPR_TRY(h->fcell.ensure(sizeof(double) * 3 * ((size_t)N + 1)));
+    const int ncol = m1 - m0;
+    if (ncol == 0) return SGPR_OK;
     h->use_i8_now = false;
-    std::vector<int> pos_of(h->M);
-    for (int p = 0; p < h->M; ++p) pos_of[h->ind_perm[p]] = p;
-    double* scratch = h->epart.as<double>();
-    for (int m = m0; m < m1; ++m) {
-        const int p = pos_of[m], s = h->ind_sp[p];
-        const int r0 = h->row_first[s], r1 = h->row_first[s + 1];
-        double* Jm = J_d + (size_t)(m - m0) * 3 * (size_t)N;
-        double* Wm = W_d + (size_t)(m - m0) * 9;
-        if (N == 0 || r1 == r0 || !h->dp.central_enabled[s]) {
-            if (N > 0) SGPR_CUDA(cudaMemsetAsync(Jm, 0, sizeof(double) * 3 * (size_t)N, st));
-            SGPR_CUDA(cudaMemsetAsync(Wm, 0, sizeof(double) * 9, st));
-            continue;
-        }
-        SGPR_CUDA(cudaMemsetAsync(h->wpart.p, 0, sizeof(double) * 9 * nblk_b, st));
-        SGPR_CUDA(cudaMemsetAsync(h->fcell.p, 0, sizeof(double) * 3 * ((size_t)N + 1), st));
-        column_seed_kernel<<<std::min<int64_t>((h->n_active + 7) / 8, h->sm_count * 8), 256, 0, st>>>(
-            (int)h->n_active, r0, r1, h->dp.D, h->dp.ldp, h->phat.as<double>(), h->zhat.as<double>() + (size_t)p * h->dp.ldp,
-            h->xi, h->xi_int, h->gvec.as<double>(), h->erow.as<double>());
-        SGPR_TRY(descriptor_backward_atoms(h, g, nullptr, st));
-        vjp_finish_kernel<<<nblk_x, 128, 0, st>>>(N, h->atoms.as<AtomRec>(), h->fcell.as<double>(), Jm, scratch + 16);
-        final_reduce_kernel<<<1, 320, 0, st>>>(0, nullptr, 0, nullptr, nblk_b, h->wpart.as<double>(), scratch, Wm);
-        h->stats.kernel_launches += 3;
-    }
+    JacTarget t{};
+    SGPR_TRY(upload_selection(h, m0, m1, st, &t));
+    SGPR_TRY(h->b_cell.ensure(sizeof(double) * 9));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, h->last_geom.cell, sizeof(double) * 9, cudaMemcpyHostToDevice, st));
+    t.n_atoms = N;
+    t.J = J_d;
+    t.W = W_d;
+    t.cells = h->b_cell.as<double>();
+    t.astr = nullptr;
+    if (N > 0) SGPR_CUDA(cudaMemsetAsync(J_d, 0, sizeof(double) * 3 * (size_t)N * ncol, st));
+    SGPR_CUDA(cudaMemsetAsync(W_d, 0, sizeof(double) * 9 * (size_t)ncol, st));
+    if (N > 0) SGPR_TRY(descriptor_jacobian_atoms(h, t, st));
     SGPR_CUDA(cudaGetLastError());
     SGPR_CUDA(cudaStreamSynchronize(st));
+    return SGPR_OK;
+}
+
+// Training-time kernels of B independent structures in one call (include/sgpr_b200.h): the front end of
+// sgpr_predict_batch, the kernel matrix into a scratch buffer, per-structure column sums (Ke) and the Jacobian kernel.
+extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian_batch(sgpr_handle h, int32_t B, const int64_t* first_h,
+                                                                                 const double* pos_d, const int32_t* Z_d,
+                                                                                 const double* cell_h, const int32_t* pbc_h,
+                                                                                 int32_t m0, int32_t m1, void* stream,
+                                                                                 double* Ke_d, double* J_d, double* W_d) {
+    if (!h || B < 0 || !first_h || (B > 0 && (!cell_h || !pbc_h || !Ke_d))) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    if ((J_d == nullptr) != (W_d == nullptr)) {
+        set_error("J_d and W_d must both be given (Jacobian) or both be NULL (Ke only)");
+        return SGPR_ERR_INVALID;
+    }
+    if (m0 < 0 || m1 > h->M || m0 > m1) {
+        set_error("inducing range [%d, %d) outside [0, %d)", m0, m1, h->M);
+        return SGPR_ERR_INVALID;
+    }
+    if (first_h[0] != 0) {
+        set_error("first_h[0] = %lld, must be 0", (long long)first_h[0]);
+        return SGPR_ERR_INVALID;
+    }
+    for (int b = 0; b < B; ++b)
+        if (first_h[b + 1] < first_h[b]) {
+            set_error("first_h is not monotone at structure %d (%lld > %lld)", b, (long long)first_h[b], (long long)first_h[b + 1]);
+            return SGPR_ERR_INVALID;
+        }
+    const int64_t N = first_h[B];
+    if (N > 0x7fffff00ll) {
+        set_error("bad atom count");
+        return SGPR_ERR_INVALID;
+    }
+    if (N > 0 && (!pos_d || !Z_d)) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    SGPR_CUDA(cudaSetDevice(h->device));
+    h->fwd_valid = false;   // no state for sgpr_kernel_backward / sgpr_kernel_jacobian
+    h->warm_ok = false;     // the next single-structure step sizes its buffers again
+    h->step_was_warm = false;
+    if (B == 0) return SGPR_OK;
+    const int ncol = m1 - m0;
+    h->use_i8_now = false;
+    h->stats.i8_ops = 0.0;
+    h->stats.gemm_flops = 0.0;
+    h->stats.covloss_flops = 0.0;
+    h->stats.kernel_launches = 0;
+    h->stats.n_atoms = N;
+    h->last_N = N;
+    std::vector<Geom> gs;
+    SGPR_TRY(build_geometry_batch(h, B, first_h, pos_d, cell_h, pbc_h, st, &gs));
+    std::vector<int> bin_base(B + 1, 0);
+    std::vector<double> cells(9 * (size_t)B);
+    long long ncell = 0;
+    for (int b = 0; b < B; ++b) {
+        bin_base[b] = (int)ncell;
+        ncell += gs[b].ncell;
+        for (int q = 0; q < 9; ++q) cells[9 * (size_t)b + q] = gs[b].cell[q];
+    }
+    if ((ncell + 1) * h->S > 0x7fffffffll) {
+        set_error("batch too large: %lld bins", ncell);
+        return SGPR_ERR_INVALID;
+    }
+    bin_base[B] = (int)ncell;
+    SGPR_TRY(h->b_geom.ensure(sizeof(Geom) * (size_t)B));
+    SGPR_TRY(h->b_first.ensure(sizeof(long long) * ((size_t)B + 1)));
+    SGPR_TRY(h->b_bins.ensure(sizeof(int) * ((size_t)B + 1)));
+    SGPR_TRY(h->b_cell.ensure(sizeof(double) * 9 * (size_t)B));
+    SGPR_TRY(h->b_err.ensure(sizeof(unsigned long long) * 2));
+    SGPR_TRY(h->astr.ensure(sizeof(int) * ((size_t)N + 1)));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_geom.p, gs.data(), sizeof(Geom) * (size_t)B, cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_first.p, first_h, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_bins.p, bin_base.data(), sizeof(int) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
+    SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, cells.data(), sizeof(double) * 9 * (size_t)B, cudaMemcpyHostToDevice, st));
+    BatchGeom bg{};
+    bg.B = B;
+    bg.ncell = (int)ncell;
+    bg.geoms = h->b_geom.as<Geom>();
+    bg.first = h->b_first.as<long long>();
+    bg.bin_base = h->b_bins.as<int>();
+    bg.cells = h->b_cell.as<double>();
+    bg.astr = h->astr.as<int>();
+    bg.err = h->b_err.as<unsigned long long>();
+    const Geom unused{};
+    // cell sort -> neighbour list (the call's one sizing synchronisation) -> descriptors
+    if (h->timing) cudaEventRecord(h->ev[0], st);
+    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, bg, st));
+    int64_t n_pairs = 0;
+    SGPR_TRY(batch_neighbor_build(h, N, bg, st, &n_pairs));
+    h->stats.n_active = h->n_active;
+    h->stats.n_pairs = n_pairs;
+    if (h->timing) cudaEventRecord(h->ev[1], st);
+    const size_t nrows = (size_t)N + 1;
+    SGPR_TRY(h->phat.ensure(sizeof(double) * nrows * h->dp.ldp));
+    SGPR_TRY(descriptor_forward_atoms(h, unused, st, &bg));
+    if (h->timing) cudaEventRecord(h->ev[2], st);
+    // K [N, M] (caller's rows and columns, lone-lone term included) -> Ke
+    SGPR_TRY(h->gmat.ensure(sizeof(double) * nrows * h->ldg));
+    {
+        int max_part = 1;
+        for (int s = 0; s < h->S; ++s) max_part = std::max(max_part, gemm_energy_parts(h->m_first[s + 1] - h->m_first[s]));
+        SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * nrows));
+    }
+    SGPR_TRY(h->rowmap.ensure(sizeof(int) * nrows));
+    SGPR_TRY(h->kscr.ensure(sizeof(double) * ((size_t)N * h->M + 1)));
+    double* K = h->kscr.as<double>();
+    SGPR_CUDA(cudaMemsetAsync(K, 0, sizeof(double) * (size_t)N * h->M, st));
+    if (N > 0 && h->M > 0) {
+        row_to_orig_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1),
+                                                                   h->rowmap.as<int>());
+        SGPR_TRY(gemm_kernel_matrix(h, K, h->M, h->rowmap.as<int>(), false, st));
+        bool any = false;
+        for (int p = 0; p < h->M; ++p) any |= h->ind_lone[p] != 0;
+        if (any)
+            lone_k_kernel<<<h->sm_count, 128, 0, st>>>((int)h->n_active, nullptr, h->atoms.as<AtomRec>(),
+                                                       h->nl_first.as<long long>(), h->M, h->ind_sp_d.as<int>(),
+                                                       h->ind_lone_d.as<unsigned char>(), K, h->lone_w);
+        h->stats.kernel_launches += 2;
+    }
+    if (ncol > 0) {
+        const long long n = (long long)B * ncol;
+        ke_reduce_kernel<<<(int)std::min<long long>((n + 255) / 256, (long long)h->sm_count * 16), 256, 0, st>>>(
+            B, bg.first, h->M, m0, ncol, K, Ke_d);
+        h->stats.kernel_launches += 1;
+    }
+    if (h->timing) cudaEventRecord(h->ev[3], st);
+    if (J_d && ncol > 0) {
+        NvtxRange jac_range("sgpr:jacobian");
+        JacTarget t{};
+        SGPR_TRY(upload_selection(h, m0, m1, st, &t));
+        t.n_atoms = N;
+        t.J = J_d;
+        t.W = W_d;
+        t.cells = bg.cells;
+        t.astr = bg.astr;
+        if (N > 0) SGPR_CUDA(cudaMemsetAsync(J_d, 0, sizeof(double) * 3 * (size_t)N * ncol, st));
+        SGPR_CUDA(cudaMemsetAsync(W_d, 0, sizeof(double) * 9 * (size_t)B * ncol, st));
+        if (N > 0) SGPR_TRY(descriptor_jacobian_atoms(h, t, st));
+    }
+    SGPR_CUDA(cudaGetLastError());
+    if (h->timing) {
+        cudaEventRecord(h->ev[4], st);
+        cudaEventRecord(h->ev[5], st);
+        SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
+        cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
+        cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
+        cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
+        cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
+        h->stats.ms_beta = 0.0f;
+        cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
+    }
     return SGPR_OK;
 }
 

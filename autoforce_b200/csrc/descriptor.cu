@@ -22,6 +22,8 @@
 // (descriptor/sesoap.py:195-203), so only pairs a<=b of a=(s,n) are stored, off-diagonal
 // entries scaled by sqrt(2): dot products and norms of packed rows equal those of the
 // reference's full [S,S,n,n,L] layout.
+#include <algorithm>
+
 #include "sgpr_internal.cuh"
 
 namespace sgpr {
@@ -775,6 +777,284 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
     }
 }
 
+// ---------------------------------------------------------------------------------
+// training-time kernels: d Ke[m] / d x for a tile of inducing LCEs at once
+// ---------------------------------------------------------------------------------
+// Per environment i (centre species s) and inducing LCE m of species s, with the cotangent of the backward pass above
+// seeded by column m (g = xi k^(xi-1) z_hat_m, e = k^xi):
+//   T_m[e]     = (xi k^(xi-1) z_m[e] - q_i[e] pg) / P * ttab[e]              (desc_backward_kernel's T)
+//   dKe/dc[a,lm] = sum_b T_m[tri(a,b), l] c[b,lm] = alpha_m U_m[a,lm] - beta_m V[a,lm]
+//   U_m = sum_b (z_m ttab)[tri(a,b), l] c[b,lm],  V = sum_b (q_i ttab)[tri(a,b), l] c[b,lm]  (m-independent)
+// and every pair contracts its d c / d r_ij block (radial x harmonic gradients, computed once per pair) against the
+// dKe/dc rows of all LCEs of the tile.  One block per (environment, tile of MT = warps x MM LCEs); warp w owns LCEs
+// w*MM .. w*MM+MM-1 of the tile and each lane one pair of a chunk of 32.
+struct JacArgs {
+    const int* sel;          // [n_sel] sorted inducing positions evaluated, grouped by central species
+    const int* sel_col;      // [n_sel] output column of each
+    int sel_first[kMaxSpecies + 1];
+    int n_tiles;             // blocks per environment
+    int ncol;                // columns of J and W
+    long long n_atoms;       // rows of J
+    double* J;               // [ncol, n_atoms, 3], caller's atom order (accumulated)
+    double* W;               // [B, ncol, 9] (accumulated)
+    const double* cells;     // [B, 9] lattice vectors of the image shifts
+    const int* astr;         // [N] structure of a cell-order atom (nullptr: one structure)
+};
+
+struct JacLayout {
+    int off_V, off_D, off_R;   // doubles from the start of shared memory
+    int prs;                   // stride of a pair record (doubles, odd)
+    int o_Y, o_xyz;            // offsets inside a pair record: f[nb] hh[nb] Y[L2] dYx[L2] dYy[L2] dYz[L2] x y z ru rx ry rz
+    int dpad;                  // per-warp T_m staging stride; 0: T_m is read from global memory
+};
+
+// out[a*L2p + lm] = sum_b T[tri(a,b), l] c[b, lm] for o = a*L2 + lm in [o0, A*L2) step ostep; T from shared memory (Ts)
+// or as zg[e] * ttab[e]
+template <class Store>
+__device__ __forceinline__ void jac_contract(const DescParams& dp, int L, int L2, int L2p, const double* Ts,
+                                             const double* __restrict__ zg, const double* __restrict__ ttab,
+                                             const double* c_s, int o0, int ostep, Store&& store) {
+    const int A = dp.A;
+    for (int o = o0; o < A * L2; o += ostep) {
+        const int a = o / L2, lm = o - a * L2, l = c_l_of_lm[lm];
+        const int rs_a = a * A - ((a * (a - 1)) >> 1);
+        int rs_b = 0;   // rs(b) = b A - b (b-1) / 2
+        double s = 0.0;
+        for (int b = 0; b < A; ++b) {
+            const int e = (b < a ? rs_b + (a - b) : rs_a + (b - a)) * L + l;
+            const double t = Ts ? Ts[e] : zg[e] * ttab[e];
+            s = fma(t, c_s[b * L2p + lm], s);
+            rs_b += A - b;
+        }
+        store(a * L2p + lm, s);
+    }
+}
+
+template <int LMAX, int NB, bool EXACT, int MM>
+__global__ void __launch_bounds__(128, 1) jacobian_kernel(DescParams dp, EnvSrc src, JacLayout lay, JacArgs out,
+                                                          const int* __restrict__ row_of, const double* __restrict__ phat,
+                                                          const double* __restrict__ ttab, const double* __restrict__ prow,
+                                                          const double* __restrict__ zhat, double xi, int xi_int,
+                                                          const double* __restrict__ cbuf,
+                                                          const unsigned char* __restrict__ sflag) {
+    extern __shared__ __align__(16) double smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5, MT = nw * MM;
+    const int env = blockIdx.x / out.n_tiles, tile = blockIdx.x - env * out.n_tiles;
+    const int c = src.active ? src.active[env] : env;
+    const AtomRec ai = src.atoms[c];
+    const int si = meta_species(ai.meta);
+    const long long beg = src.nl_first[env], end = src.nl_first[env + 1];
+    const int t0 = out.sel_first[si] + tile * MT, t1 = out.sel_first[si + 1];
+    // lone centres (constant K), excluded centres (K = 0) and tiles past the species' LCEs: nothing to add
+    if (t0 >= t1 || end == beg || !dp.central_enabled[si]) return;
+    const int L = EXACT ? LMAX + 1 : dp.lmax + 1;
+    const int nbv = EXACT ? NB : dp.nb;
+    const int L2v = EXACT ? (LMAX + 1) * (LMAX + 1) : dp.L2;
+    const int L2p = EXACT ? (((LMAX + 1) * (LMAX + 1)) | 1) : dp.L2p;
+    const int lmaxv = EXACT ? LMAX : dp.lmax;
+    double* c_s = smem;
+    double* V_s = smem + lay.off_V;
+    double* Dt = smem + lay.off_D;   // [MT][csize] dKe/dc of the tile's LCEs
+    double* R = smem + lay.off_R;    // T_m staging, then pair records
+    const int r = row_of[c];
+    const double* q = phat + (size_t)r * dp.ldp;
+    for (int t = threadIdx.x; t < dp.csize; t += blockDim.x) c_s[t] = cbuf[(size_t)env * dp.csize + t];
+    if (lay.dpad)
+        for (int e = threadIdx.x; e < dp.D; e += blockDim.x) R[e] = q[e] * ttab[e];
+    __syncthreads();
+    jac_contract(dp, L, L2v, L2p, lay.dpad ? R : nullptr, q, ttab, c_s, threadIdx.x, blockDim.x,
+                 [&](int o, double s) { V_s[o] = s; });
+    __syncthreads();
+    // chain rule through the normalisation as desc_backward_kernel applies it
+    const double Pn = dp.normalize ? prow[r] : 1.0;
+    const double rP = 1.0 / Pn;
+    const double nfac = (Pn > 2.0 * kEps ? Pn / (Pn - kEps) : 1.0);
+    double* Tw = lay.dpad ? R + (size_t)warp * lay.dpad : nullptr;
+#pragma unroll 1
+    for (int mm = 0; mm < MM; ++mm) {
+        const int t = t0 + warp * MM + mm;
+        if (t >= t1) break;   // warp-uniform
+        const double* z = zhat + (size_t)out.sel[t] * dp.ldp;
+        double k = 0.0;
+        for (int e = lane; e < dp.D; e += 32) {
+            const double zv = z[e];
+            k = fma(q[e], zv, k);
+            if (Tw) Tw[e] = zv * ttab[e];
+        }
+        k = warp_sum(k);
+        double pw = 1.0;
+        if (xi_int >= 1) {
+            for (int u = 1; u < xi_int; ++u) pw *= k;
+        } else {
+            pw = pow(k, xi - 1.0);
+        }
+        const double cm = xi * pw, em = pw * k;
+        const double pg = dp.normalize ? xi * em * nfac : 0.0;
+        const double alpha = cm * rP, beta = pg * rP;
+        double* Dm = Dt + (size_t)(warp * MM + mm) * dp.csize;
+        __syncwarp();
+        jac_contract(dp, L, L2v, L2p, Tw, z, ttab, c_s, lane, 32,
+                     [&](int o, double s) { Dm[o] = alpha * s - beta * V_s[o]; });
+        __syncwarp();
+    }
+    __syncthreads();   // R becomes the pair-record buffer
+
+    const int b = out.astr ? out.astr[c] : 0;
+    const CellRef cref{out.cells + 9 * (size_t)b};
+    const bool flag = sflag[env] != 0;
+    int* pint = reinterpret_cast<int*>(R + 32 * lay.prs);   // [32] species, [32] caller's index of j
+    bool ok[MM];
+    int col[MM];
+#pragma unroll
+    for (int mm = 0; mm < MM; ++mm) {
+        const int t = t0 + warp * MM + mm;
+        ok[mm] = t < t1;
+        col[mm] = ok[mm] ? out.sel_col[t] : 0;
+    }
+    double Gi[MM][3], Wa[MM][9];
+#pragma unroll
+    for (int mm = 0; mm < MM; ++mm) {
+#pragma unroll
+        for (int q3 = 0; q3 < 3; ++q3) Gi[mm][q3] = 0.0;
+#pragma unroll
+        for (int q9 = 0; q9 < 9; ++q9) Wa[mm][q9] = 0.0;
+    }
+    for (long long k0 = beg; k0 < end; k0 += 32) {
+        if (warp == 0) {
+            const long long k = k0 + lane;
+            double* my = R + (size_t)lane * lay.prs;
+            if (k < end) {
+                double rx, ry, rz;
+                int sp, j;
+                Nbr<false>::load_pair(src, cref, ai, src.pairs[k], rx, ry, rz, sp, j);
+                const double u = dp.radii[sp], ru = dp.rinv[sp];
+                const double x = rx * ru, y = ry * ru, z = rz * ru;
+                const double d2 = x * x + y * y + z * z;
+                const double rd = rsqrt(d2);
+                const double d = d2 * rd;
+                double Rr, Rpd;
+                radial_fast(d2, d, rd, u, dp.rc, dp.rc_inv, Rr, Rpd);
+                if (!dp.nbr_enabled[sp]) {
+                    Rr = 0.0;
+                    Rpd = 0.0;
+                }
+                double pw = 1.0;  // d2^(n-1)
+                my[0] = Rr;
+                my[nbv] = Rpd;
+                double fn = Rr;
+                for (int n = 1; n < nbv; ++n) {
+                    fn *= d2;
+                    my[n] = fn;
+                    my[nbv + n] = Rpd * (pw * d2) + 2.0 * n * Rr * pw;
+                    pw *= d2;
+                }
+                double ys = y, zs = z;
+                if (flag) {
+                    ys = y - kTinyAngle * z;
+                    zs = kTinyAngle * y + z;
+                }
+                double* yo = my + lay.o_Y;
+                solid_harmonics<LMAX, true>(c_harm, lmaxv, x, ys, zs,
+                                            [&](int idx, double Y, double dYx, double dYy, double dYz) {
+                                                yo[idx] = Y;
+                                                yo[L2v + idx] = dYx;
+                                                if (flag) {  // transpose of the shear, ylm.py:212-220 (linear: per component)
+                                                    yo[2 * L2v + idx] = dYy + kTinyAngle * dYz;
+                                                    yo[3 * L2v + idx] = -kTinyAngle * dYy + dYz;
+                                                } else {
+                                                    yo[2 * L2v + idx] = dYy;
+                                                    yo[3 * L2v + idx] = dYz;
+                                                }
+                                            });
+                double* xyz = my + lay.o_xyz;
+                xyz[0] = x; xyz[1] = y; xyz[2] = z; xyz[3] = ru;
+                xyz[4] = rx; xyz[5] = ry; xyz[6] = rz;
+                pint[lane] = sp;
+                pint[32 + lane] = meta_orig(src.atoms[j].meta);
+            }
+        }
+        __syncthreads();
+        const int cnt = (int)min((long long)32, end - k0);
+        if (lane < cnt) {
+            const double* my = R + (size_t)lane * lay.prs;
+            const int sp = pint[lane];
+            const long long jo = pint[32 + lane];
+            double f[NB], hh[NB];
+#pragma unroll
+            for (int n = 0; n < NB; ++n) {
+                f[n] = n < nbv ? my[n] : 0.0;
+                hh[n] = n < nbv ? my[nbv + n] : 0.0;
+            }
+            double Tn[MM][NB], gx[MM], gy[MM], gz[MM];
+            const double* Db[MM];
+#pragma unroll
+            for (int mm = 0; mm < MM; ++mm) {
+                gx[mm] = gy[mm] = gz[mm] = 0.0;
+#pragma unroll
+                for (int n = 0; n < NB; ++n) Tn[mm][n] = 0.0;
+                Db[mm] = Dt + (size_t)(warp * MM + mm) * dp.csize + sp * nbv * L2p;
+            }
+            const double* yo = my + lay.o_Y;
+#pragma unroll 2
+            for (int lm = 0; lm < L2v; ++lm) {
+                const double Y = yo[lm], dx = yo[L2v + lm], dy = yo[2 * L2v + lm], dz = yo[3 * L2v + lm];
+#pragma unroll
+                for (int mm = 0; mm < MM; ++mm) {
+                    double B = 0.0;
+#pragma unroll
+                    for (int n = 0; n < NB; ++n) {
+                        if (n < nbv) {
+                            const double dc = Db[mm][n * L2p + lm];
+                            B = fma(dc, f[n], B);
+                            Tn[mm][n] = fma(dc, Y, Tn[mm][n]);
+                        }
+                    }
+                    gx[mm] = fma(B, dx, gx[mm]);
+                    gy[mm] = fma(B, dy, gy[mm]);
+                    gz[mm] = fma(B, dz, gz[mm]);
+                }
+            }
+            const double* xyz = my + lay.o_xyz;
+            const double x = xyz[0], y = xyz[1], z = xyz[2], ru = xyz[3], rx = xyz[4], ry = xyz[5], rz = xyz[6];
+#pragma unroll
+            for (int mm = 0; mm < MM; ++mm) {
+                if (!ok[mm]) continue;
+                double rad = 0.0;
+#pragma unroll
+                for (int n = 0; n < NB; ++n)
+                    if (n < nbv) rad += Tn[mm][n] * hh[n];
+                const double Gx = (rad * x + gx[mm]) * ru, Gy = (rad * y + gy[mm]) * ru, Gz = (rad * z + gz[mm]) * ru;
+                double* Jj = out.J + ((size_t)col[mm] * out.n_atoms + jo) * 3;
+                atomicAdd(Jj, Gx);
+                atomicAdd(Jj + 1, Gy);
+                atomicAdd(Jj + 2, Gz);
+                Gi[mm][0] -= Gx; Gi[mm][1] -= Gy; Gi[mm][2] -= Gz;
+                Wa[mm][0] += rx * Gx; Wa[mm][1] += rx * Gy; Wa[mm][2] += rx * Gz;
+                Wa[mm][3] += ry * Gx; Wa[mm][4] += ry * Gy; Wa[mm][5] += ry * Gz;
+                Wa[mm][6] += rz * Gx; Wa[mm][7] += rz * Gy; Wa[mm][8] += rz * Gz;
+            }
+        }
+        __syncthreads();
+    }
+    const long long io = meta_orig(ai.meta);
+#pragma unroll
+    for (int mm = 0; mm < MM; ++mm) {
+        if (!ok[mm]) continue;   // warp-uniform
+#pragma unroll
+        for (int q3 = 0; q3 < 3; ++q3) Gi[mm][q3] = warp_sum(Gi[mm][q3]);
+#pragma unroll
+        for (int q9 = 0; q9 < 9; ++q9) Wa[mm][q9] = warp_sum(Wa[mm][q9]);
+        if (lane == 0) {
+            double* Ji = out.J + ((size_t)col[mm] * out.n_atoms + io) * 3;
+#pragma unroll
+            for (int q3 = 0; q3 < 3; ++q3) atomicAdd(Ji + q3, Gi[mm][q3]);
+            double* Wb = out.W + ((size_t)b * out.ncol + col[mm]) * 9;
+#pragma unroll
+            for (int q9 = 0; q9 < 9; ++q9) atomicAdd(Wb + q9, Wa[mm][q9]);
+        }
+    }
+}
+
 // packed row -> the reference's dense block layout [S,S,nb,nb,L]
 __global__ void unpack_kernel(DescParams dp, long long rows, const double* __restrict__ packed,
                               const int* __restrict__ src_row, double* __restrict__ full) {
@@ -903,7 +1183,93 @@ int launch_backward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src
     return SGPR_OK;
 }
 
+template <int LMAX, int NB, bool EXACT>
+int launch_jacobian(sgpr_context* h, const EnvSrc& src, const JacArgs& a, int max_sel, cudaStream_t st) {
+    constexpr int MM = NB <= 4 ? 4 : 2;   // LCEs per warp: the register tile of the pair contraction
+    const DescParams& dp = h->dp;
+    const int na = (int)h->n_active;
+    JacLayout lay{};
+    lay.o_Y = 2 * dp.nb;
+    lay.o_xyz = lay.o_Y + 4 * dp.L2;
+    lay.prs = (lay.o_xyz + 7) | 1;
+    const int pair_doubles = 32 * lay.prs + 32;   // records + 64 ints
+    const size_t cap = 220 * 1024;
+    int nw = 4;
+    size_t smem = 0;
+    for (;; nw >>= 1) {
+        const int mt = nw * MM;
+        const int dpad = (dp.D + 1) & ~1;
+        const size_t fixed = (size_t)(2 + mt) * ((dp.csize + 1) & ~1);
+        lay.dpad = dpad;
+        size_t rsz = std::max<size_t>((size_t)nw * dpad, pair_doubles);
+        if ((fixed + rsz) * 8 > cap) {   // read T_m from global memory instead of staging it
+            lay.dpad = 0;
+            rsz = pair_doubles;
+        }
+        smem = (fixed + rsz) * 8;
+        if (smem <= cap) break;
+        if (nw == 1) {
+            set_error("descriptor too large for the Jacobian kernel (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
+            return SGPR_ERR_INVALID;
+        }
+    }
+    const int csp = (dp.csize + 1) & ~1;
+    lay.off_V = csp;
+    lay.off_D = 2 * csp;
+    lay.off_R = (2 + nw * MM) * csp;
+    JacArgs args = a;
+    args.n_tiles = (max_sel + nw * MM - 1) / (nw * MM);
+    const long long grid = (long long)na * args.n_tiles;
+    if (grid == 0) return SGPR_OK;
+    if (grid > 0x7fffffffll) {
+        set_error("too many environments x inducing tiles for one Jacobian launch (%lld)", grid);
+        return SGPR_ERR_INVALID;
+    }
+    auto kern = jacobian_kernel<LMAX, NB, EXACT, MM>;
+    SGPR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)grid, nw * 32, smem, st>>>(dp, src, lay, args, h->rowof.as<int>() + (h->last_N + 1), h->phat.as<double>(),
+                                               h->ttab.as<double>(), h->prow.as<double>(), h->zhat.as<double>(), h->xi,
+                                               h->xi_int, h->cbuf.as<double>(), h->sflag.as<unsigned char>());
+    SGPR_CUDA(cudaGetLastError());
+    h->stats.kernel_launches += 1;
+    return SGPR_OK;
+}
+
 }  // namespace
+
+int descriptor_jacobian_atoms(sgpr_context* h, const JacTarget& t, cudaStream_t st) {
+    if (h->n_active == 0 || t.n_sel == 0) return SGPR_OK;
+    EnvSrc src{};
+    src.atoms = h->atoms.as<AtomRec>();
+    src.pairs = h->nl_pairs.as<PairRec>();
+    src.nl_first = h->nl_first.as<long long>();
+    src.active = h->active_all ? nullptr : h->active_list.as<int>();
+    JacArgs a{};
+    a.sel = t.sel;
+    a.sel_col = t.sel + t.n_sel;
+    int max_sel = 0;
+    for (int s = 0; s <= kMaxSpecies; ++s) a.sel_first[s] = t.sel_first[std::min(s, h->S)];
+    for (int s = 0; s < h->S; ++s) max_sel = std::max(max_sel, t.sel_first[s + 1] - t.sel_first[s]);
+    a.ncol = t.ncol;
+    a.n_atoms = t.n_atoms;
+    a.J = t.J;
+    a.W = t.W;
+    a.cells = t.cells;
+    a.astr = t.astr;
+    const int lmax = h->dp.lmax, nb = h->dp.nb;
+#define JAC(LM, NBB, EX) return launch_jacobian<LM, NBB, EX>(h, src, a, max_sel, st)
+    if (lmax == 3 && nb == 4) JAC(3, 4, true);   // the reference's default
+    if (lmax <= 3 && nb <= 4) JAC(3, 4, false);
+    if (lmax == 6 && nb == 9) JAC(6, 9, true);   // the high-resolution configuration
+    if (lmax <= 3 && nb <= 8) JAC(3, 8, false);
+    if (lmax <= 6 && nb <= 6) JAC(6, 6, false);
+    if (lmax <= 6 && nb <= 9) JAC(6, 9, false);
+    if (lmax <= 6 && nb <= 12) JAC(6, 12, false);
+    if (lmax <= 8 && nb <= 12) JAC(8, 12, false);
+#undef JAC
+    set_error("unsupported descriptor size lmax=%d nmax=%d", lmax, nb - 1);
+    return SGPR_ERR_INVALID;
+}
 
 int descriptor_forward_env(sgpr_context* h, int M, const long long* env_first_d, const double* env_r_d,
                            const unsigned char* env_sp_d, const int* row_of_d, double* phat_d, cudaStream_t st) {

@@ -241,6 +241,7 @@ struct sgpr_context {
     sgpr::DevBuf p2p_local;                      // fused exchange step: [16] partial E/W + step counter
     sgpr::DevBuf b_geom, b_first, b_bins, b_cell, b_err;   // batched prediction: BatchGeom arrays
     sgpr::DevBuf astr, wenv;                     // batched prediction: structure per cell-order atom, [N,9] per-environment virials
+    sgpr::DevBuf jsel, kscr;                     // training-time kernels: inducing selection, K scratch [N, M]
     bool p2p_counter_init = false;
     void* pinned = nullptr;
     size_t pinned_bytes = 0;
@@ -309,6 +310,20 @@ struct P2PStep {
     uint8_t* owned_d;
 };
 int backward_grid(sgpr_context* h);
+// training-time kernels of the step's environments (api.cu: sgpr_kernel_jacobian, sgpr_kernel_jacobian_batch):
+// J [ncol, n_atoms, 3] += d Ke[b(j), m] / d x_j and W [B, ncol, 9] += sum_pairs r (x) dKe/dr, for the inducing LCEs sel
+struct JacTarget {
+    const int* sel;          // device [2 n_sel]: sorted inducing positions grouped by central species, then their columns
+    int n_sel;
+    int sel_first[SGPR_MAX_SPECIES + 1];   // host: range of each central species in sel
+    int ncol;
+    long long n_atoms;
+    double* J;               // zeroed by the caller
+    double* W;               // zeroed by the caller
+    const double* cells;     // device [B, 9]
+    const int* astr;         // device [N] structure of a cell-order atom; nullptr: one structure
+};
+int descriptor_jacobian_atoms(sgpr_context* h, const JacTarget& t, cudaStream_t st);
 int unpack_descriptors(sgpr_context* h, long long rows, const double* packed_d, const int* src_row_d, double* full_d,
                        cudaStream_t st);
 

@@ -60,6 +60,8 @@ EXPORTS = {
     "sgpr_kernel_forward": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_kernel_backward": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_kernel_jacobian": (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
+    "sgpr_kernel_jacobian_batch": (c_int32, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                             c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_neighbors": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_void_p, c_void_p, c_int64, POINTER(c_int64)]),
     "sgpr_descriptors": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -361,6 +363,62 @@ class SgprEngine:
         if want_beta:
             return E, F, W, beta[:N].cpu().numpy()
         return E, F, W
+
+    def training_kernels(self, pos, numbers=None, first=None, cells=None, pbcs=None, m0=0, m1=None, want_jacobian=True):
+        """Training-time kernels of B structures against the inducing LCEs m0 <= m < m1 in one call
+        (``sgpr_kernel_jacobian_batch``): the blocks of ``EnergyForceKernel(first=[...], X, cov=...)``
+        (regression/gppotential.py:63-77) that make_munu stacks.
+
+        Inputs as in ``predict_batch``: concatenated arrays or CUDA tensors with ``first`` [B+1], ``cells`` and ``pbcs``,
+        or a list of structures.  Returns device tensors ``(Ke [B, m], Kf [3 Ntot, m], Kv [6 B, m])``: energy_energy,
+        forces_energy (= -d Ke / d xyz, rows 3i..3i+2 of atom i) and virial_energy (rows 6b..6b+5 of structure b:
+        xx, yy, zz, yz, xz, xy, not divided by the volume), structures stacked in order.  ``want_jacobian=False`` skips
+        the Jacobian and returns ``(Ke, None, None)``.  For B = 1 this is ``kernel_jacobian`` (Ke = K.sum(0))."""
+        import torch
+
+        if first is None:
+            images = list(pos)
+            if numbers is not None or cells is not None or pbcs is not None:
+                raise ValueError("pass either a list of structures or pos, numbers, first, cells, pbcs")
+            counts = [len(a.numbers) for a in images]
+            pos = np.concatenate([np.asarray(a.positions, dtype=np.float64).reshape(-1, 3) for a in images]) if images else np.zeros((0, 3))
+            numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images]) if images else np.zeros(0, dtype=np.int32)
+            first = np.concatenate([[0], np.cumsum(counts)])
+            cells = [np.asarray(a.cell, dtype=np.float64).reshape(3, 3) for a in images]
+            pbcs = [np.broadcast_to(np.asarray(a.pbc), (3,)) for a in images]
+        first_h = np.ascontiguousarray(first, dtype=np.int64).reshape(-1)
+        B = len(first_h) - 1
+        if B < 0:
+            raise ValueError("first must have B+1 >= 1 entries")
+        cell_h = np.ascontiguousarray(np.broadcast_to(np.asarray(cells, dtype=np.float64).reshape(-1, 9), (B, 9)))
+        pb = np.asarray(pbcs).astype(np.int32)
+        pbc_h = np.ascontiguousarray(np.broadcast_to(pb.reshape(-1, 3) if pb.size and pb.size % 3 == 0 else pb.reshape(-1, 1), (B, 3)))
+        pos_t, z_t = self._dev(pos, numbers)
+        N = z_t.numel()
+        if pos_t.shape[0] != N or first_h[-1] != N:
+            raise ValueError(f"first[-1] = {first_h[-1]} does not match {N} atoms")
+        m1 = self.model.M if m1 is None else int(m1)
+        m0 = int(m0)
+        if not 0 <= m0 <= m1 <= self.model.M:
+            raise ValueError(f"inducing range [{m0}, {m1}) outside [0, {self.model.M})")
+        nm = m1 - m0
+        dev = pos_t.device
+        # flat buffers of at least one element: empty outputs still get valid (non-NULL) device pointers
+        buf = lambda n: torch.zeros(max(n, 1), dtype=torch.float64, device=dev)   # noqa: E731
+        Ke = buf(B * nm)
+        J = buf(nm * N * 3) if want_jacobian else None
+        W = buf(B * nm * 9) if want_jacobian else None
+        _check(self.lib, self.lib.sgpr_kernel_jacobian_batch(self._h, B, _ptr(first_h), c_void_p(pos_t.data_ptr()),
+                                                             c_void_p(z_t.data_ptr()), _ptr(cell_h), _ptr(pbc_h), m0, m1,
+                                                             self._stream(), c_void_p(Ke.data_ptr()),
+                                                             c_void_p(J.data_ptr()) if want_jacobian else None,
+                                                             c_void_p(W.data_ptr()) if want_jacobian else None))
+        Ke = Ke[:B * nm].reshape(B, nm)
+        if not want_jacobian:
+            return Ke, None, None
+        Kf = -J[:nm * N * 3].reshape(nm, 3 * N).t().contiguous()
+        Kv = W[:B * nm * 9].reshape(B, nm, 9)[:, :, [0, 4, 8, 5, 2, 1]].permute(0, 2, 1).reshape(6 * B, nm).contiguous()
+        return Ke, Kf, Kv
 
     def predict_p2p(self, pos_t, z_t, cell, pbc, rank, world, peer_ptrs, ew):
         """``sgpr_predict_p2p``: this rank's environments only; forces on every atom are ADDED into the accumulation

@@ -150,7 +150,9 @@ class _SoapKernelBase:
         """``SimilarityKernel.forward(first, second, operation)`` (similarity/similarity.py:17-31).
 
         first : a structure (``TorchAtoms`` / ``ase.Atoms`` / anything with positions, numbers, cell, pbc) -- every atom
-                is a centre -- or ``Local`` / ``LocalsData`` / list of ``Local`` / ``(Z, r, b)`` tuples.
+                is a centre -- or ``Local`` / ``LocalsData`` / list of ``Local`` / ``(Z, r, b)`` tuples, or a list of
+                structures: then "func" gives per-structure sums Ke [B, M] and "leftgrad" / "virial" the structures'
+                rows stacked in order ([3 Ntot, M] / [6 B, M]), all from one batched call.
         second: the same kinds of object (a structure stands for all of its environments).
         operation: "func" -> K [len(first), len(second)];  with a structure as ``first`` also "leftgrad" ->
                 d(sum_i K[i,m]) / d xyz  [3N, M] and "virial" -> [6, M] (similarity/universal.py:124-183; the true
@@ -166,7 +168,13 @@ class _SoapKernelBase:
         else:
             envs2, objs2 = _as_envs(second)
             as_torch = as_torch or any(hasattr(getattr(o, "_r", None), "detach") for o in objs2)
-        if _is_structure(first):
+        if isinstance(first, (list, tuple)) and first and all(_is_structure(a) for a in first):
+            # several structures: one sgpr_kernel_jacobian_batch call; "func" gives one row of Ke per structure, "leftgrad"
+            # and "virial" the structures' rows stacked in order (regression/gppotential.py:63-77)
+            eng = self._engine(envs2, objs2, np.unique(np.concatenate([np.asarray(a.numbers).reshape(-1) for a in first])))
+            Ke, Kf, Kv = eng.training_kernels(list(first), want_jacobian=operation != "func")
+            out = (Ke if operation == "func" else (-Kf if operation == "leftgrad" else Kv)).cpu()
+        elif _is_structure(first):
             eng = self._engine(envs2, objs2, np.unique(first.numbers))
             args = (first.positions, first.numbers, np.asarray(first.cell, dtype=np.float64).reshape(3, 3), first.pbc)
             if operation == "func":

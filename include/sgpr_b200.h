@@ -218,8 +218,30 @@ int sgpr_kernel_backward(sgpr_handle h, const double* gK_d, void* stream, double
  *                         (virial_energy = W.flat[[0,4,8,5,2,1]])
  * These are the true derivatives (they agree with torch.autograd through the reference's forward pass);
  * the reference's hand-written leftgrad drops contributions when an atom occurs twice in one environment
- * (index assignment g[j] += f, universal.py:148) -- see tests/golden/make_golden_train.py. */
+ * (index assignment g[j] += f, universal.py:148) -- see tests/golden/make_golden_train.py.
+ * All m0 <= m < m1 are evaluated by one launch of the Jacobian kernel (as in sgpr_kernel_jacobian_batch); J_d and
+ * W_d agree with it to rounding (atomic accumulation). */
 int sgpr_kernel_jacobian(sgpr_handle h, int32_t m0, int32_t m1, void* stream, double* J_d, double* W_d);
+
+/* Training-time kernels of B independent structures in one call: for every data structure b and every inducing LCE
+ * m0 <= m < m1 the energy_energy, forces_energy and virial_energy blocks that make_munu stacks
+ * (regression/gppotential.py:63-77 EnergyForceKernel(first=[...]), 548-601 make_munu; update_data / update_inducing).
+ * Replaces one sgpr_kernel_forward + sgpr_kernel_jacobian pair per structure.
+ *   first_h [B+1], pos_d, Z_d, cell_h [B,9], pbc_h [B,3]   as in sgpr_predict_batch (0-atom structures, own cells, mixed pbc)
+ *   Ke_d [B, m1-m0]          sum_{i in b} K[i,m], lone-lone term included (K.sum(0) of sgpr_kernel_forward per
+ *                            structure); fixed summation order: bit-identical whatever else is in the batch
+ *   J_d  [m1-m0, Ntot, 3]    d Ke[b(j), m] / d x_j, caller's atom order, layout and sign of sgpr_kernel_jacobian
+ *   W_d  [B, m1-m0, 9]       sum_pairs r (x) dK/dr per structure, NOT divided by the volume (sgpr_kernel_jacobian's W_d)
+ * J_d and W_d both NULL: Ke only (no Jacobian stage); only one of them NULL is SGPR_ERR_INVALID.  J and W are
+ * accumulated with red.global.add.f64 and agree with a call on the structure alone to rounding.
+ * Errors: SGPR_ERR_INVALID for malformed first_h or m0 < 0, m1 > M, m0 > m1; SGPR_ERR_GEOMETRY / _SPECIES name the first
+ * structure that failed in sgpr_last_error().  B = 0 does nothing.
+ * Synchronises the stream once (sizing); never sharded; never replayed as a graph; leaves no state for
+ * sgpr_kernel_backward / sgpr_kernel_jacobian (the next single-structure step sizes again).  sgpr_get_stats reports the
+ * batch's totals. */
+int sgpr_kernel_jacobian_batch(sgpr_handle h, int32_t B, const int64_t* first_h, const double* pos_d, const int32_t* Z_d,
+                               const double* cell_h, const int32_t* pbc_h, int32_t m0, int32_t m1, void* stream,
+                               double* Ke_d, double* J_d, double* W_d);
 
 /* ---- parity hooks (used by tests; same kernels as the hot path) --------------------- */
 
