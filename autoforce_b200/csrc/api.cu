@@ -826,7 +826,8 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
                       &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
-                      &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr};
+                      &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr,
+                      &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part};
     for (DevBuf* b : bufs) b->release();
     if (h->pinned) cudaFreeHost(h->pinned);
     if (h->i8_probs_pinned) cudaFreeHost(h->i8_probs_pinned);
@@ -1261,6 +1262,17 @@ static int predict_impl(sgpr_handle h, int64_t N, const double* pos_d, const int
 static void drop_graphs(sgpr_context* h) {
     for (auto& e : h->graphs) cudaGraphExecDestroy(e.exec);
     h->graphs.clear();
+    md_drop_graphs(h);
+}
+
+bool sgpr::md_warm_possible(sgpr_context* h, int64_t N, const int32_t* pbc_h, bool beta) {
+    return warm_possible(h, N, pbc_h, 0, 1, false, beta);
+}
+
+int sgpr::md_predict(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,
+                     const int32_t* pbc_h, cudaStream_t st, double* E_d, double* F_d, double* W_d, double* beta_d, bool graph) {
+    if (graph) return predict_impl(h, N, pos_d, Z_d, cell_h, pbc_h, 0, 1, st, E_d, F_d, W_d, beta_d, nullptr, nullptr, true);
+    return predict_body(h, N, pos_d, Z_d, cell_h, pbc_h, 0, 1, st, E_d, F_d, W_d, beta_d, nullptr, nullptr, true);
 }
 
 extern "C" __attribute__((visibility("default"))) int sgpr_predict(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,

@@ -258,6 +258,24 @@ struct sgpr_context {
     sgpr_stats stats;
     bool timing = false;
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // ---- MD driver (md.cu): the step in flight is predicted from scratch copies and committed only when it was valid
+    sgpr::DevBuf md_pos, md_mom, md_F, md_beta, md_ew, md_part;
+    struct MdGraphKey {                     // everything a captured MD step bakes into its nodes
+        int64_t N;
+        void* stream;
+        const void* ptr[8];                 // pos, mom, Z, mass, F, thermo, beta, state
+        double cell[9];
+        double prm[5];                      // dt, c1, c2, kT, ediff
+        uint64_t seed;
+        int32_t langevin, stop;
+    };
+    struct MdGraphEntry {
+        MdGraphKey key;
+        cudaGraphExec_t exec;
+        unsigned long long stamp;
+    };
+    std::vector<MdGraphEntry> md_graphs;
+    unsigned long long md_graph_gen = 0;
 };
 
 namespace sgpr {
@@ -345,5 +363,14 @@ int i8_covloss(sgpr_context* h, int64_t n_rows, cudaStream_t st);
 int i8_back_projection(sgpr_context* h, cudaStream_t st);
 int i8_setup_step(sgpr_context* h, cudaStream_t st);   // work lists of this step's GEMMs from row_first_d (one warp)
 int gemm_back_projection(sgpr_context* h, cudaStream_t st);
+
+// ---- api.cu: the prediction step as the MD driver runs it (single structure, no sharding) ---------------------------
+bool md_warm_possible(sgpr_context* h, int64_t N, const int32_t* pbc_h, bool beta);
+// graph = true: sgpr_predict's path (replays its own graph when warm); false: plain launches, for capture by the caller
+int md_predict(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,
+               const int32_t* pbc_h, cudaStream_t st, double* E_d, double* F_d, double* W_d, double* beta_d, bool graph);
+
+// ---- md.cu ----------------------------------------------------------------------------------------------------------
+void md_drop_graphs(sgpr_context* h);
 
 }  // namespace sgpr

@@ -9,6 +9,7 @@
 // descriptor/sesoap.py:172-184 + descriptor/cutoff.py:20-44 (radial part).
 #pragma once
 #include <math.h>
+#include <stdint.h>
 
 #if defined(__CUDACC__)
 #define SGPR_HD __host__ __device__ __forceinline__
@@ -151,6 +152,52 @@ inline double anl(int n, int l) {
     for (int k = 2; k <= n; ++k) f1 *= k;
     for (int k = 2; k <= n + l; ++k) f2 *= k;
     return 1.0 / ((2.0 * l + 1.0) * pow(2.0, 2 * n + l) * f1 * f2);
+}
+
+// Philox4x32-10 (Salmon et al., "Parallel random numbers: as easy as 1, 2, 3", SC'11): counter-based, so the Langevin
+// noise of (atom, step) is a pure function of the seed and needs no generator state in memory.  ctr is replaced by the
+// output block.
+SGPR_HD void philox4x32_10(uint32_t ctr[4], uint32_t k0, uint32_t k1) {
+    for (int r = 0; r < 10; ++r) {
+        if (r > 0) {
+            k0 += 0x9E3779B9u;
+            k1 += 0xBB67AE85u;
+        }
+        const uint64_t p0 = (uint64_t)0xD2511F53u * ctr[0];
+        const uint64_t p1 = (uint64_t)0xCD9E8D57u * ctr[2];
+        const uint32_t hi0 = (uint32_t)(p0 >> 32), lo0 = (uint32_t)p0;
+        const uint32_t hi1 = (uint32_t)(p1 >> 32), lo1 = (uint32_t)p1;
+        const uint32_t c1 = ctr[1], c3 = ctr[3];
+        ctr[0] = hi1 ^ c1 ^ k0;
+        ctr[1] = lo1;
+        ctr[2] = hi0 ^ c3 ^ k1;
+        ctr[3] = lo0;
+    }
+}
+
+// uniform in (0, 1) from the top 53 bits of a 64-bit word (never 0: the logarithm of Box-Muller stays finite)
+SGPR_HD double philox_uniform(uint32_t lo, uint32_t hi) {
+    const uint64_t x = ((uint64_t)hi << 32) | lo;
+    return ((double)(x >> 11) + 0.5) * 1.1102230246251565404e-16;   // 2^-53
+}
+
+// Three standard normal deviates of the Langevin O step for one atom and step.  Key = seed; counter = {atom, call,
+// step low word, step high word}; output words 0,1 and 2,3 of a block are two 64-bit words (low word first).  Box-Muller
+// turns the two uniforms of call 0 into xi[0], xi[1]; the first normal of call 1 is xi[2].
+SGPR_HD void langevin_normals(uint64_t seed, uint32_t atom, uint64_t step, double xi[3]) {
+    const double two_pi = 6.283185307179586476925;
+    for (uint32_t call = 0; call < 2; ++call) {
+        uint32_t c[4] = {atom, call, (uint32_t)step, (uint32_t)(step >> 32)};
+        philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+        const double u0 = philox_uniform(c[0], c[1]), u1 = philox_uniform(c[2], c[3]);
+        const double rad = sqrt(-2.0 * log(u0));
+        if (call == 0) {
+            xi[0] = rad * cos(two_pi * u1);
+            xi[1] = rad * sin(two_pi * u1);
+        } else {
+            xi[2] = rad * cos(two_pi * u1);
+        }
+    }
 }
 
 }  // namespace sgpr

@@ -38,6 +38,13 @@ class sgpr_stats(ctypes.Structure):
     ]
 
 
+class sgpr_md_params(ctypes.Structure):
+    _fields_ = [
+        ("dt", c_double), ("friction", c_double), ("kT", c_double), ("ediff", c_double), ("seed", ctypes.c_uint64),
+        ("langevin", c_int32), ("stop_on_uncertain", c_int32),
+    ]
+
+
 EXPORTS = {
     # name: (restype, argtypes)       -- every symbol include/sgpr_b200.h declares
     "sgpr_create": (c_int32, [POINTER(sgpr_model_desc), POINTER(c_void_p)]),
@@ -67,6 +74,10 @@ EXPORTS = {
     "sgpr_descriptors": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_inducing_descriptors": (c_int32, [c_void_p, c_void_p, c_void_p]),
     "sgpr_kernel_envs": (c_int32, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "sgpr_md_init": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(sgpr_md_params), c_void_p,
+                               c_void_p, c_void_p, c_void_p]),
+    "sgpr_md_steps": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                POINTER(sgpr_md_params), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sgpr_set_async": (c_int32, [c_void_p, c_int32]),
     "sgpr_check": (c_int32, [c_void_p, POINTER(c_int64)]),
     "sgpr_get_stats": (c_int32, [c_void_p, POINTER(sgpr_stats)]),
@@ -631,6 +642,31 @@ class SgprEngine:
         m.ind_b = np.concatenate([m.ind_b, b])
         m.mu = mu
         m.choli = ch
+
+    # ------------------------------------------------------------------ molecular dynamics (md.DeviceMD drives these)
+    def md_init(self, pos_t, z_t, cell, pbc, params, F, beta, state):
+        """``sgpr_md_init``: F [N,3] (and beta [N] when ``params.stop_on_uncertain``) of pos_t, state reset; enqueued on
+        torch's current stream, validated by ``sgpr_check`` after synchronising."""
+        cell_h, pbc_h = self._geom(cell, pbc)
+        _check(self.lib, self.lib.sgpr_md_init(self._h, z_t.numel(), c_void_p(pos_t.data_ptr()), c_void_p(z_t.data_ptr()),
+                                               _ptr(cell_h), _ptr(pbc_h), ctypes.byref(params), self._stream(),
+                                               c_void_p(F.data_ptr()), c_void_p(beta.data_ptr()) if beta is not None else None,
+                                               c_void_p(state.data_ptr())))
+
+    def md_steps(self, pos_t, mom_t, z_t, mass_t, cell, pbc, params, n_steps, F, thermo, beta, state):
+        """``sgpr_md_steps``: enqueue n_steps MD steps on torch's current stream (include/sgpr_b200.h)."""
+        cell_h, pbc_h = self._geom(cell, pbc)
+        _check(self.lib, self.lib.sgpr_md_steps(self._h, z_t.numel(), c_void_p(pos_t.data_ptr()), c_void_p(mom_t.data_ptr()),
+                                                c_void_p(z_t.data_ptr()), c_void_p(mass_t.data_ptr()), _ptr(cell_h), _ptr(pbc_h),
+                                                ctypes.byref(params), int(n_steps), self._stream(), c_void_p(F.data_ptr()),
+                                                c_void_p(thermo.data_ptr()),
+                                                c_void_p(beta.data_ptr()) if beta is not None else None,
+                                                c_void_p(state.data_ptr())))
+
+    def check_status(self):
+        """``sgpr_check`` without raising: (status, message) -- SGPR_ERR_RETRY (-7) is a step to repeat, not a failure."""
+        st = self.lib.sgpr_check(self._h, None)
+        return int(st), (self.lib.sgpr_last_error().decode(errors="replace") if st else "")
 
     def set_async(self, on=True):
         """Device-pointer entry points (predict_device, peer exchange) enqueue warm steps without synchronising; call

@@ -279,6 +279,48 @@ int sgpr_inducing_descriptors(sgpr_handle h, void* stream, double* Zhat_d);
 int sgpr_set_async(sgpr_handle h, int32_t on);
 int sgpr_check(sgpr_handle h, int64_t* n_pairs_out);
 
+/* ---- molecular dynamics on the device ------------------------------------------------
+ * What ASE's VelocityVerlet / Langevin do around ActiveCalculator in prediction mode (calculator/active.py:425-611,
+ * covloss 492-499), with positions, momenta and forces resident on the device.  Units are the caller's (ASE: eV, A, amu,
+ * ASE time); pos_d and mom_d stay unwrapped, as in ASE.
+ *   NVE (langevin = 0), ASE's operation order:   p += dt/2 F;  r += dt p/m;  F = F(r);  p += dt/2 F
+ *   NVT (langevin = 1), BAOAB:  p += dt/2 F;  r += dt/2 p/m;  p = c1 p + c2 sqrt(m kT) xi;  r += dt/2 p/m;  F = F(r);
+ *                               p += dt/2 F    with c1 = exp(-friction dt), c2 = sqrt(1 - c1^2), no centre-of-mass fix;
+ *                               xi = Philox4x32-10 normals keyed by seed and counted by (atom, step): sgpr_math.cuh
+ * Device state state_d [4] int64: 0 steps done (the global step, also the noise counter of the next step), 1 the step
+ * at which max(beta) > ediff first held (0 = the starting structure; -1 = none), 2 = 1 when the step state_d[0]+1 was
+ * not integrated because its prediction was invalid, 3 the step at which the current sgpr_md_steps call began.
+ * Once state_d[1] >= 0 or state_d[2] = 1 every later step leaves positions, momenta, forces and beta unchanged. */
+typedef struct {
+    double   dt;                  /* time step                                                       */
+    double   friction;            /* Langevin friction (1/time); unused for NVE                        */
+    double   kT;                  /* Langevin temperature (energy); unused for NVE                     */
+    double   ediff;               /* stop when max(beta) > ediff (the comparison of prediction mode: NaN does not
+                                     stop, inf does)                                                    */
+    uint64_t seed;                /* Philox key of the Langevin noise                                  */
+    int32_t  langevin;            /* 0 = velocity Verlet, 1 = BAOAB Langevin                           */
+    int32_t  stop_on_uncertain;   /* 1: evaluate covloss every step (beta_d required) and stop          */
+} sgpr_md_params;
+
+/* Start of a run: F_d [N,3] (and beta_d [N] if p->stop_on_uncertain) = forces (covloss) of pos_d, state_d = {0, -1 or 0, 0,
+ * 0}.  Enqueued on `stream` like sgpr_predict in asynchronous mode: after synchronising, sgpr_check reports an invalid
+ * evaluation (SGPR_ERR_RETRY: call sgpr_md_init again). */
+int sgpr_md_init(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,
+                 const int32_t* pbc_h, const sgpr_md_params* p, void* stream, double* F_d, double* beta_d,
+                 int64_t* state_d);
+
+/* Enqueue n_steps MD steps.  pos_d, mom_d [N,3] and F_d (forces of pos_d on entry) are updated in place; mass_d [N];
+ * thermo_d [n_steps, 11] receives one row per step done by this call, {E_pot, E_kin, W[9]} (W as in sgpr_predict; E_kin
+ * = sum p^2/2m in a fixed order); beta_d [N] (or NULL without stop_on_uncertain) the covloss of the current positions.
+ * Warm steps (periodic cell, buffers sized by an earlier step of the same shape) need no host synchronisation: a step is
+ * one CUDA graph launch.  After synchronising the stream, read state_d and call sgpr_check: SGPR_ERR_RETRY means a step
+ * outgrew the buffers and was NOT integrated (state_d[2] = 1): enqueue the remaining steps again; they size first.
+ * Other errors (an atom more than 120 cells outside the cell, unknown species) also leave the state of the last good
+ * step.  Errors found while enqueueing (sizing steps: non-periodic cells size on every step) name the step. */
+int sgpr_md_steps(sgpr_handle h, int64_t N, double* pos_d, double* mom_d, const int32_t* Z_d, const double* mass_d,
+                  const double* cell_h, const int32_t* pbc_h, const sgpr_md_params* p, int32_t n_steps, void* stream,
+                  double* F_d, double* thermo_d, double* beta_d, int64_t* state_d);
+
 /* Explicit local chemical environments (reference `Local` objects: number, _r, _b; descriptor/atoms.py:36-52) against
  * the inducing set -- the similarity interface on LCEs rather than structures:
  *   K_d [n_env, M]   = kern(locs, X)            (similarity/similarity.py:17-43, universal.py:109-122 incl. the
