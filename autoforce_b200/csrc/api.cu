@@ -713,6 +713,7 @@ extern "C" __attribute__((visibility("default"))) int sgpr_create(const sgpr_mod
         set_error("S*(nmax+1) = %d exceeds 255", dp.A);
         return SGPR_ERR_INVALID;
     }
+    SGPR_TRY(descriptor_check_size(dp));
     for (int i = 0; i < 128; ++i) h->z_to_species[i] = -1;
     for (int s = 0; s < SGPR_MAX_SPECIES; ++s) {
         dp.radii[s] = 1.0;

@@ -598,11 +598,15 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
                 const int nm = 2 * l + 1, lm0 = l * l;
 #pragma unroll
                 for (int nn0 = 0; nn0 < nm; nn0 += 8) {
-                    // columns n >= nm and rows a >= A of the product are never stored; k-entries b >= A are zeroed
+                    // columns n >= nm and rows a >= A of the product are never stored; k-entries b >= A are zeroed.
+                    // Columns n >= nm are not read either: past the last l of row b = A-1 they lie beyond the c block,
+                    // and for lmax = 0 with A < 5 beyond this warp's shared-memory slice (for the last warp: past the
+                    // end of the block's allocation)
                     const double* cl = c_s + lm0 + nn0 + g8;
+                    const bool n_ok = nn0 + g8 < nm;
                     double bv[4];
 #pragma unroll
-                    for (int ki = 0; ki < 4; ++ki) bv[ki] = ((okm >> ki) & 1u) ? cl[boff[ki]] : 0.0;
+                    for (int ki = 0; ki < 4; ++ki) bv[ki] = (n_ok && ((okm >> ki) & 1u)) ? cl[boff[ki]] : 0.0;
 #pragma unroll
                     for (int mi = 0; mi < 2; ++mi) {
                         if (mi * 8 < dp.A) {
@@ -1183,20 +1187,15 @@ int launch_backward(sgpr_context* h, const Geom& g, int n_env, const EnvSrc& src
     return SGPR_OK;
 }
 
-template <int LMAX, int NB, bool EXACT>
-int launch_jacobian(sgpr_context* h, const EnvSrc& src, const JacArgs& a, int max_sel, cudaStream_t st) {
-    constexpr int MM = NB <= 4 ? 4 : 2;   // LCEs per warp: the register tile of the pair contraction
-    const DescParams& dp = h->dp;
-    const int na = (int)h->n_active;
-    JacLayout lay{};
+// shared memory of the Jacobian kernel: warps per block, layout and bytes (false: not even one warp fits)
+bool plan_jacobian(const DescParams& dp, int MM, JacLayout& lay, int& nw, size_t& smem) {
+    lay = JacLayout{};
     lay.o_Y = 2 * dp.nb;
     lay.o_xyz = lay.o_Y + 4 * dp.L2;
     lay.prs = (lay.o_xyz + 7) | 1;
     const int pair_doubles = 32 * lay.prs + 32;   // records + 64 ints
     const size_t cap = 220 * 1024;
-    int nw = 4;
-    size_t smem = 0;
-    for (;; nw >>= 1) {
+    for (nw = 4;; nw >>= 1) {
         const int mt = nw * MM;
         const int dpad = (dp.D + 1) & ~1;
         const size_t fixed = (size_t)(2 + mt) * ((dp.csize + 1) & ~1);
@@ -1207,11 +1206,22 @@ int launch_jacobian(sgpr_context* h, const EnvSrc& src, const JacArgs& a, int ma
             rsz = pair_doubles;
         }
         smem = (fixed + rsz) * 8;
-        if (smem <= cap) break;
-        if (nw == 1) {
-            set_error("descriptor too large for the Jacobian kernel (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
-            return SGPR_ERR_INVALID;
-        }
+        if (smem <= cap) return true;
+        if (nw == 1) return false;
+    }
+}
+
+template <int LMAX, int NB, bool EXACT>
+int launch_jacobian(sgpr_context* h, const EnvSrc& src, const JacArgs& a, int max_sel, cudaStream_t st) {
+    constexpr int MM = NB <= 4 ? 4 : 2;   // LCEs per warp: the register tile of the pair contraction
+    const DescParams& dp = h->dp;
+    const int na = (int)h->n_active;
+    JacLayout lay;
+    int nw;
+    size_t smem;
+    if (!plan_jacobian(dp, MM, lay, nw, smem)) {
+        set_error("descriptor too large for the Jacobian kernel (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
+        return SGPR_ERR_INVALID;
     }
     const int csp = (dp.csize + 1) & ~1;
     lay.off_V = csp;
@@ -1236,6 +1246,22 @@ int launch_jacobian(sgpr_context* h, const EnvSrc& src, const JacArgs& a, int ma
 }
 
 }  // namespace
+
+int descriptor_check_size(const DescParams& dp) {
+    if ((size_t)plan_backward(dp).per_warp * 8 > 200 * 1024) {
+        set_error("descriptor too large for shared memory (S=%d nmax=%d lmax=%d): the force kernel needs %zu KB per "
+                  "warp, at most 200 KB fit", dp.S, dp.nb - 1, dp.lmax, (size_t)plan_backward(dp).per_warp * 8 / 1024);
+        return SGPR_ERR_INVALID;
+    }
+    JacLayout lay;
+    int nw;
+    size_t smem;
+    if (!plan_jacobian(dp, (dp.lmax <= 3 && dp.nb <= 4) ? 4 : 2, lay, nw, smem)) {   // MM of descriptor_jacobian_atoms
+        set_error("descriptor too large for the Jacobian kernel (S=%d nmax=%d lmax=%d)", dp.S, dp.nb - 1, dp.lmax);
+        return SGPR_ERR_INVALID;
+    }
+    return SGPR_OK;
+}
 
 int descriptor_jacobian_atoms(sgpr_context* h, const JacTarget& t, cudaStream_t st) {
     if (h->n_active == 0 || t.n_sel == 0) return SGPR_OK;

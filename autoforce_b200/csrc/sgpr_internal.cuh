@@ -300,6 +300,9 @@ int scan_exclusive_ll(sgpr_context* h, const long long* in, long long* out, int 
 
 // ---- descriptor.cu ----------------------------------------------------------------
 int upload_harm_coef();
+// refuses (SGPR_ERR_INVALID, message set) a descriptor size whose shared-memory plans of the force or Jacobian kernel
+// cannot fit one warp
+int descriptor_check_size(const DescParams& dp);
 int descriptor_forward_env(sgpr_context* h, int M, const long long* env_first_d, const double* env_r_d,
                            const unsigned char* env_sp_d, const int* row_of_d, double* phat_d, cudaStream_t st);
 int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st, const BatchGeom* bg = nullptr);
