@@ -10,6 +10,7 @@ from .model import SgprModel  # noqa: F401
 from .engine import SgprEngine, library_path, load_library  # noqa: F401
 from .calculator import B200Calculator  # noqa: F401
 from .md import DeviceMD  # noqa: F401
+from .relax import DeviceRelax  # noqa: F401
 from .kernels import SeSoapKernel, SubSeSoapKernel, HeterogeneousSoapKernel, UniversalSoapKernel, DefaultRadii  # noqa: F401
 
 __version__ = "0.1.0"

@@ -828,7 +828,8 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
                       &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
                       &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr,
-                      &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part};
+                      &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part,
+                      &h->rx_pos, &h->rx_vel, &h->rx_F, &h->rx_beta, &h->rx_ew, &h->rx_part};
     for (DevBuf* b : bufs) b->release();
     if (h->pinned) cudaFreeHost(h->pinned);
     if (h->i8_probs_pinned) cudaFreeHost(h->i8_probs_pinned);
@@ -1263,7 +1264,7 @@ static int predict_impl(sgpr_handle h, int64_t N, const double* pos_d, const int
 static void drop_graphs(sgpr_context* h) {
     for (auto& e : h->graphs) cudaGraphExecDestroy(e.exec);
     h->graphs.clear();
-    md_drop_graphs(h);
+    drop_driver_graphs(h);
 }
 
 bool sgpr::md_warm_possible(sgpr_context* h, int64_t N, const int32_t* pbc_h, bool beta) {

@@ -43,9 +43,6 @@ struct MdArgs {
 
 __device__ __forceinline__ bool md_frozen(const long long* state) { return state[1] >= 0 || state[2] != 0; }
 
-// max that propagates NaN, like torch.max / np.max in prediction mode
-__device__ __forceinline__ double nan_max(double a, double b) { return (b > a || b != b) ? b : a; }
-
 __global__ void md_reset_kernel(long long* state) {
     state[0] = 0;
     state[1] = -1;
@@ -242,25 +239,11 @@ int md_enqueue_step(sgpr_context* h, const MdArgs& a, const int32_t* Z_d, const 
     return md_evaluate(h, a, a.pos_n, Z_d, cell_h, pbc_h, st, graph);
 }
 
-// an error met while enqueueing (sizing steps report geometry and species errors synchronously) names the step
-int md_name_step(sgpr_context* h, int rc, const long long* state_d, cudaStream_t st) {
-    char msg[768];
-    snprintf(msg, sizeof(msg), "%s", sgpr_last_error());
-    long long done = -1;
-    if (cudaStreamSynchronize(st) == cudaSuccess && cudaMemcpy(&done, state_d, sizeof(done), cudaMemcpyDeviceToHost) == cudaSuccess)
-        set_error("MD step %lld: %s", done + 1, msg);
-    else
-        cudaGetLastError();
-    h->warm_ok = false;
-    return rc;
-}
-
 int md_step(sgpr_context* h, const MdArgs& a, const int32_t* Z_d, const double* cell_h, const int32_t* pbc_h,
             cudaStream_t st, const sgpr_md_params* p) {
-    const bool warm = md_warm_possible(h, a.N, pbc_h, a.beta != nullptr);
-    if (!warm || !h->use_graph || h->timing) return md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, true);
-    sgpr_context::MdGraphKey key;
+    sgpr_context::DriverGraphKey key;
     memset(&key, 0, sizeof(key));
+    key.driver = kDriverMd;
     key.N = a.N;
     key.stream = (void*)st;
     key.ptr[0] = a.pos; key.ptr[1] = a.mom; key.ptr[2] = Z_d; key.ptr[3] = a.mass;
@@ -268,15 +251,37 @@ int md_step(sgpr_context* h, const MdArgs& a, const int32_t* Z_d, const double* 
     for (int i = 0; i < 9; ++i) key.cell[i] = cell_h[i];
     key.prm[0] = p->dt; key.prm[1] = a.c1; key.prm[2] = a.c2; key.prm[3] = a.kT; key.prm[4] = a.ediff;
     key.seed = a.seed;
-    key.langevin = a.langevin;
-    key.stop = a.stop_on_uncertain;
+    key.flag[0] = a.langevin;
+    key.flag[1] = a.stop_on_uncertain;
+    return driver_graph_step(h, key, md_warm_possible(h, a.N, pbc_h, a.beta != nullptr),
+                             [&](bool graph) { return md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, graph); });
+}
+
+}  // namespace
+
+int driver_name_step(sgpr_context* h, int rc, const long long* state_d, cudaStream_t st, const char* what) {
+    char msg[768];
+    snprintf(msg, sizeof(msg), "%s", sgpr_last_error());
+    long long done = -1;
+    if (cudaStreamSynchronize(st) == cudaSuccess && cudaMemcpy(&done, state_d, sizeof(done), cudaMemcpyDeviceToHost) == cudaSuccess)
+        set_error("%s %lld: %s", what, done + 1, msg);
+    else
+        cudaGetLastError();
+    h->warm_ok = false;
+    return rc;
+}
+
+int driver_graph_step(sgpr_context* h, const sgpr_context::DriverGraphKey& key, bool warm,
+                      const std::function<int(bool)>& enqueue) {
+    if (!warm || !h->use_graph || h->timing) return enqueue(true);
+    cudaStream_t st = (cudaStream_t)key.stream;
     // a workspace was reallocated since capture: the graphs point at freed memory
     const unsigned long long gen = buf_generation();
-    if (gen != h->md_graph_gen) {
-        md_drop_graphs(h);
-        h->md_graph_gen = gen;
+    if (gen != h->driver_graph_gen) {
+        drop_driver_graphs(h);
+        h->driver_graph_gen = gen;
     }
-    for (auto& e : h->md_graphs) {
+    for (auto& e : h->driver_graphs) {
         if (memcmp(&e.key, &key, sizeof(key)) == 0) {
             e.stamp = ++h->graph_clock;
             h->step_was_warm = true;
@@ -287,9 +292,9 @@ int md_step(sgpr_context* h, const MdArgs& a, const int32_t* Z_d, const double* 
     cudaGraph_t graph = nullptr;
     if (cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed) != cudaSuccess) {
         cudaGetLastError();   // e.g. the legacy default stream cannot be captured
-        return md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, true);
+        return enqueue(true);
     }
-    const int rc = md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, false);
+    const int rc = enqueue(false);
     const cudaError_t ce = cudaStreamEndCapture(st, &graph);
     if (rc != SGPR_OK || ce != cudaSuccess || !graph || !h->step_was_warm) {
         if (graph) cudaGraphDestroy(graph);
@@ -297,38 +302,36 @@ int md_step(sgpr_context* h, const MdArgs& a, const int32_t* Z_d, const double* 
         h->use_graph = false;   // plain launches from now on (as predict_impl does)
         h->warm_ok = false;     // whatever was enqueued during the failed capture never ran
         if (rc != SGPR_OK) return rc;
-        return md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, false);
+        return enqueue(false);
     }
     cudaGraphExec_t exec = nullptr;
-    if (buf_generation() != h->md_graph_gen || cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) {
+    if (buf_generation() != h->driver_graph_gen || cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) {
         // (a workspace grown during the capture would leave a graph that points at freed memory)
         cudaGraphDestroy(graph);
         cudaGetLastError();
         h->warm_ok = false;
-        return md_enqueue_step(h, a, Z_d, cell_h, pbc_h, st, false);
+        return enqueue(false);
     }
     cudaGraphDestroy(graph);
-    if (h->md_graphs.size() >= 4) {   // evict the least recently used entry
+    if (h->driver_graphs.size() >= 4) {   // evict the least recently used entry
         size_t lru = 0;
-        for (size_t i = 1; i < h->md_graphs.size(); ++i)
-            if (h->md_graphs[i].stamp < h->md_graphs[lru].stamp) lru = i;
-        cudaGraphExecDestroy(h->md_graphs[lru].exec);
-        h->md_graphs.erase(h->md_graphs.begin() + lru);
+        for (size_t i = 1; i < h->driver_graphs.size(); ++i)
+            if (h->driver_graphs[i].stamp < h->driver_graphs[lru].stamp) lru = i;
+        cudaGraphExecDestroy(h->driver_graphs[lru].exec);
+        h->driver_graphs.erase(h->driver_graphs.begin() + lru);
     }
-    sgpr_context::MdGraphEntry e;
+    sgpr_context::DriverGraphEntry e;
     e.key = key;
     e.exec = exec;
     e.stamp = ++h->graph_clock;
-    h->md_graphs.push_back(e);
+    h->driver_graphs.push_back(e);
     SGPR_CUDA(cudaGraphLaunch(exec, st));
     return SGPR_OK;
 }
 
-}  // namespace
-
-void md_drop_graphs(sgpr_context* h) {
-    for (auto& e : h->md_graphs) cudaGraphExecDestroy(e.exec);
-    h->md_graphs.clear();
+void drop_driver_graphs(sgpr_context* h) {
+    for (auto& e : h->driver_graphs) cudaGraphExecDestroy(e.exec);
+    h->driver_graphs.clear();
 }
 
 }  // namespace sgpr
@@ -367,7 +370,7 @@ extern "C" __attribute__((visibility("default"))) int sgpr_md_steps(sgpr_handle 
     SGPR_CUDA(cudaGetLastError());
     for (int32_t k = 0; k < n_steps; ++k) {
         const int rc = md_step(h, a, Z_d, cell_h, pbc_h, st, p);
-        if (rc != SGPR_OK) return md_name_step(h, rc, a.state, st);
+        if (rc != SGPR_OK) return driver_name_step(h, rc, a.state, st, "MD step");
     }
     return SGPR_OK;
 }

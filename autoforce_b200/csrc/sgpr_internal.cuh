@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -111,6 +112,9 @@ struct BatchGeom {
 // Number of DevBuf reallocations so far: CUDA graphs of warm steps bake the workspaces' addresses into their nodes and
 // must not outlive them (api.cu: predict_impl).
 unsigned long long buf_generation();
+
+// max that propagates NaN, like torch.max / np.max in prediction mode (the device drivers' reductions)
+__device__ __forceinline__ double nan_max(double a, double b) { return (b > a || b != b) ? b : a; }
 
 // host-side mirror of a grow-only device buffer
 struct DevBuf {
@@ -260,22 +264,26 @@ struct sgpr_context {
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     // ---- MD driver (md.cu): the step in flight is predicted from scratch copies and committed only when it was valid
     sgpr::DevBuf md_pos, md_mom, md_F, md_beta, md_ew, md_part;
-    struct MdGraphKey {                     // everything a captured MD step bakes into its nodes
+    // ---- relaxation driver (relax.cu), same rule: scratch positions (first the step dr), velocities, forces, beta
+    sgpr::DevBuf rx_pos, rx_vel, rx_F, rx_beta, rx_ew, rx_part;
+    // ---- CUDA graphs of warm driver steps (md.cu: driver_graph_step), MD and relaxation in one LRU cache
+    struct DriverGraphKey {                 // everything a captured driver step bakes into its nodes
+        int32_t driver;                     // kDriverMd / kDriverRelax: keeps the two drivers' graphs apart
+        int32_t flag[3];
         int64_t N;
         void* stream;
-        const void* ptr[8];                 // pos, mom, Z, mass, F, thermo, beta, state
+        const void* ptr[10];
         double cell[9];
-        double prm[5];                      // dt, c1, c2, kT, ediff
+        double prm[10];
         uint64_t seed;
-        int32_t langevin, stop;
     };
-    struct MdGraphEntry {
-        MdGraphKey key;
+    struct DriverGraphEntry {
+        DriverGraphKey key;
         cudaGraphExec_t exec;
         unsigned long long stamp;
     };
-    std::vector<MdGraphEntry> md_graphs;
-    unsigned long long md_graph_gen = 0;
+    std::vector<DriverGraphEntry> driver_graphs;
+    unsigned long long driver_graph_gen = 0;
 };
 
 namespace sgpr {
@@ -374,6 +382,14 @@ int md_predict(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z
                const int32_t* pbc_h, cudaStream_t st, double* E_d, double* F_d, double* W_d, double* beta_d, bool graph);
 
 // ---- md.cu ----------------------------------------------------------------------------------------------------------
-void md_drop_graphs(sgpr_context* h);
+enum { kDriverMd = 1, kDriverRelax = 2 };
+void drop_driver_graphs(sgpr_context* h);
+// one step of a device driver: enqueue(true) runs it with plain launches (sizing steps, no graph); when warm, the step
+// enqueued by enqueue(false) is captured once per key and replayed (key zero-filled before its fields are set: compared
+// with memcmp)
+int driver_graph_step(sgpr_context* h, const sgpr_context::DriverGraphKey& key, bool warm,
+                      const std::function<int(bool)>& enqueue);
+// an error met while enqueueing a driver step names the step: "<what> <state_d[0] + 1>: <message>"
+int driver_name_step(sgpr_context* h, int rc, const long long* state_d, cudaStream_t st, const char* what);
 
 }  // namespace sgpr

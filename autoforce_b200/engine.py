@@ -45,6 +45,14 @@ class sgpr_md_params(ctypes.Structure):
     ]
 
 
+class sgpr_relax_params(ctypes.Structure):
+    _fields_ = [
+        ("dt", c_double), ("maxstep", c_double), ("dtmax", c_double), ("finc", c_double), ("fdec", c_double),
+        ("astart", c_double), ("fa", c_double), ("a", c_double), ("fmax", c_double), ("ediff", c_double),
+        ("Nmin", c_int32), ("stop_on_uncertain", c_int32),
+    ]
+
+
 EXPORTS = {
     # name: (restype, argtypes)       -- every symbol include/sgpr_b200.h declares
     "sgpr_create": (c_int32, [POINTER(sgpr_model_desc), POINTER(c_void_p)]),
@@ -78,6 +86,11 @@ EXPORTS = {
                                c_void_p, c_void_p, c_void_p]),
     "sgpr_md_steps": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                 POINTER(sgpr_md_params), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "sgpr_relax_init": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  POINTER(sgpr_relax_params), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "sgpr_relax_steps": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   POINTER(sgpr_relax_params), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p]),
     "sgpr_set_async": (c_int32, [c_void_p, c_int32]),
     "sgpr_check": (c_int32, [c_void_p, POINTER(c_int64)]),
     "sgpr_get_stats": (c_int32, [c_void_p, POINTER(sgpr_stats)]),
@@ -662,6 +675,29 @@ class SgprEngine:
                                                 c_void_p(thermo.data_ptr()),
                                                 c_void_p(beta.data_ptr()) if beta is not None else None,
                                                 c_void_p(state.data_ptr())))
+
+    # ------------------------------------------------------------------ geometry relaxation (relax.DeviceRelax drives these)
+    def relax_init(self, pos_t, z_t, fixed, cell, pbc, params, F, beta, fire, state):
+        """``sgpr_relax_init``: F [N,3] (and beta [N] when ``params.stop_on_uncertain``) of pos_t with the rows of
+        ``fixed`` (uint8 [N] or None) zeroed, FIRE scalars and state reset; validated by ``sgpr_check`` after
+        synchronising."""
+        cell_h, pbc_h = self._geom(cell, pbc)
+        _check(self.lib, self.lib.sgpr_relax_init(self._h, z_t.numel(), c_void_p(pos_t.data_ptr()), c_void_p(z_t.data_ptr()),
+                                                  c_void_p(fixed.data_ptr()) if fixed is not None else None, _ptr(cell_h),
+                                                  _ptr(pbc_h), ctypes.byref(params), self._stream(), c_void_p(F.data_ptr()),
+                                                  c_void_p(beta.data_ptr()) if beta is not None else None,
+                                                  c_void_p(fire.data_ptr()), c_void_p(state.data_ptr())))
+
+    def relax_steps(self, pos_t, vel_t, z_t, fixed, cell, pbc, params, n_steps, F, trace, beta, fire, state):
+        """``sgpr_relax_steps``: enqueue n_steps FIRE steps on torch's current stream (include/sgpr_b200.h)."""
+        cell_h, pbc_h = self._geom(cell, pbc)
+        _check(self.lib, self.lib.sgpr_relax_steps(self._h, z_t.numel(), c_void_p(pos_t.data_ptr()), c_void_p(vel_t.data_ptr()),
+                                                   c_void_p(z_t.data_ptr()),
+                                                   c_void_p(fixed.data_ptr()) if fixed is not None else None, _ptr(cell_h),
+                                                   _ptr(pbc_h), ctypes.byref(params), int(n_steps), self._stream(),
+                                                   c_void_p(F.data_ptr()), c_void_p(trace.data_ptr()),
+                                                   c_void_p(beta.data_ptr()) if beta is not None else None,
+                                                   c_void_p(fire.data_ptr()), c_void_p(state.data_ptr())))
 
     def check_status(self):
         """``sgpr_check`` without raising: (status, message) -- SGPR_ERR_RETRY (-7) is a step to repeat, not a failure."""

@@ -24,6 +24,25 @@ KB = 8.617330337217213e-05    # ase.units.kB: Boltzmann constant in eV/K
 SGPR_ERR_RETRY = -7
 
 
+def check_driver(calc, name):
+    """What the device drivers (DeviceMD, DeviceRelax) refuse: kernel sums and torch.distributed sharding."""
+    if len(getattr(calc, "models", ())) != 1:
+        raise NotImplementedError(f"{name} runs a single model handle: kernel sums are not supported")
+    _, _, world = calc._dist()
+    if world > 1:
+        raise NotImplementedError(f"{name} runs on one GPU: torch.distributed sharding is not supported")
+
+
+def check_species(calc, atoms):
+    """atoms.numbers as a flat array; unknown species are refused before any device work."""
+    numbers = np.asarray(atoms.numbers).reshape(-1)
+    species = set(int(z) for z in calc.model.species()) | set(int(z) for z in numbers)
+    if any(z < 1 or z > 118 for z in species) or len(species) > MAX_SPECIES:
+        raise ValueError(f"unknown species: atomic numbers {sorted(set(int(z) for z in numbers))} with the model's "
+                         f"{sorted(calc.model.species())} (at most {MAX_SPECIES} species of Z 1..118)")
+    return numbers
+
+
 class DeviceMD:
     """MD of one structure on the GPU of ``calc`` (a ``B200Calculator``).
 
@@ -34,19 +53,11 @@ class DeviceMD:
     def __init__(self, calc, atoms, timestep=1.0, temperature_K=None, friction=None, seed=0, masses=None):
         import torch
 
-        if len(getattr(calc, "models", ())) != 1:
-            raise NotImplementedError("DeviceMD runs a single model handle: kernel sums are not supported")
-        _, _, world = calc._dist()
-        if world > 1:
-            raise NotImplementedError("DeviceMD runs on one GPU: torch.distributed sharding is not supported")
+        check_driver(calc, "DeviceMD")
         if getattr(atoms, "constraints", None):
             raise NotImplementedError("DeviceMD does not support ASE constraints")
-        numbers = np.asarray(atoms.numbers).reshape(-1)
+        numbers = check_species(calc, atoms)
         N = len(numbers)
-        species = set(int(z) for z in calc.model.species()) | set(int(z) for z in numbers)
-        if any(z < 1 or z > 118 for z in species) or len(species) > MAX_SPECIES:
-            raise ValueError(f"unknown species: atomic numbers {sorted(set(int(z) for z in numbers))} with the model's "
-                             f"{sorted(calc.model.species())} (at most {MAX_SPECIES} species of Z 1..118)")
         if masses is None:
             if not hasattr(atoms, "get_masses"):
                 raise ValueError("masses are required when atoms has no get_masses()")

@@ -321,6 +321,49 @@ int sgpr_md_steps(sgpr_handle h, int64_t N, double* pos_d, double* mom_d, const 
                   const double* cell_h, const int32_t* pbc_h, const sgpr_md_params* p, int32_t n_steps, void* stream,
                   double* F_d, double* thermo_d, double* beta_d, int64_t* state_d);
 
+/* ---- geometry relaxation on the device ------------------------------------------------
+ * ASE's FIRE optimiser (ase/optimize/fire.py of ASE 3.22-3.23, downhill_check=False) around the prediction step, with
+ * positions, velocities and forces resident on the device.  Iteration k, with the forces F of the positions r known:
+ *   converged <=> max_i |F_i|^2 < fmax^2   (tested before every step, the starting structure included)
+ *   first step: v = 0;  later: if F.v > 0:  v = (1-a) v + a |v| F/|F|;  if Nsteps > Nmin: dt = min(dt finc, dtmax),
+ *                                          a *= fa;  Nsteps += 1
+ *                               else:     v *= 0;  a = astart;  dt *= fdec;  Nsteps = 0
+ *   v += dt F;  dr = dt v;  if |dr| > maxstep: dr *= maxstep/|dr| (norm over all atoms);  r += dr;  F = F(r)
+ * fixed_d (uint8 [N], or NULL): the forces of atoms with fixed_d[i] != 0 are zero in every use above (ASE's FixAtoms
+ * through get_forces()), so they never move; energy and virial are those of all atoms.
+ * fire_d [6] double: {dt, a, F.v, F.F, v.v, max_i |F_i|^2} -- the FIRE scalars and the reductions of the current F, v.
+ * state_d [6] int64: 0 steps done, 1 the step at which max(beta) > ediff first held (-1 = none), 2 = 1 when the step
+ * state_d[0]+1 was not done because its prediction was invalid, 3 the step at which the current sgpr_relax_steps call
+ * began, 4 the step whose forces met fmax (-1 = none), 5 FIRE's Nsteps.  Once state_d[1] >= 0, state_d[2] = 1 or
+ * state_d[4] >= 0 every later step leaves positions, velocities, forces, beta and fire_d unchanged. */
+typedef struct {
+    double   dt;                  /* FIRE (ASE's names and defaults): initial time step, 0.1                */
+    double   maxstep;             /* largest |dr| of a step (norm over all atoms), 0.2                       */
+    double   dtmax;               /* 1.0                                                                   */
+    double   finc, fdec;          /* 1.1, 0.5                                                              */
+    double   astart, fa, a;       /* 0.1, 0.99, 0.1 (a: initial mixing)                                    */
+    double   fmax;                /* convergence: max_i |F_i| < fmax                                        */
+    double   ediff;               /* stop when max(beta) > ediff (as sgpr_md_params)                        */
+    int32_t  Nmin;                /* 5                                                                     */
+    int32_t  stop_on_uncertain;   /* 1: evaluate covloss every step (beta_d required) and stop               */
+} sgpr_relax_params;
+
+/* Start of a relaxation: F_d [N,3] (and beta_d [N] if p->stop_on_uncertain) of pos_d, fixed rows zeroed; fire_d = {p->dt,
+ * p->a, ...}; state_d = {0, -1 or 0, 0, 0, 0 if the start meets p->fmax else -1, 0}.  Enqueued on `stream`; after
+ * synchronising, sgpr_check reports an invalid evaluation (SGPR_ERR_RETRY: call sgpr_relax_init again). */
+int sgpr_relax_init(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d, const uint8_t* fixed_d,
+                    const double* cell_h, const int32_t* pbc_h, const sgpr_relax_params* p, void* stream, double* F_d,
+                    double* beta_d, double* fire_d, int64_t* state_d);
+
+/* Enqueue n_steps FIRE steps.  pos_d, vel_d [N,3], F_d (forces of pos_d on entry), beta_d, fire_d and state_d are
+ * updated in place.  The call first re-tests the current forces against p->fmax (state_d[4]), as ASE's run(fmax) does.
+ * trace_d [n_steps, 13] receives one row per step done by this call: {E_pot, max_i |F_i|, dt, a, W[9]} (dt and a after
+ * the step's update).  Warm steps replay one CUDA graph each; the overflow protocol and the errors are sgpr_md_steps':
+ * SGPR_ERR_RETRY with state_d[2] = 1 means the step was not done: enqueue the remaining steps again. */
+int sgpr_relax_steps(sgpr_handle h, int64_t N, double* pos_d, double* vel_d, const int32_t* Z_d, const uint8_t* fixed_d,
+                     const double* cell_h, const int32_t* pbc_h, const sgpr_relax_params* p, int32_t n_steps,
+                     void* stream, double* F_d, double* trace_d, double* beta_d, double* fire_d, int64_t* state_d);
+
 /* Explicit local chemical environments (reference `Local` objects: number, _r, _b; descriptor/atoms.py:36-52) against
  * the inducing set -- the similarity interface on LCEs rather than structures:
  *   K_d [n_env, M]   = kern(locs, X)            (similarity/similarity.py:17-43, universal.py:109-122 incl. the
