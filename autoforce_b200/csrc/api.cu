@@ -1032,6 +1032,19 @@ static int covloss_stage(sgpr_context* h, cudaStream_t st, int64_t N, const int*
     return SGPR_OK;
 }
 
+// stage times of a call from the events ev[0..4] recorded on its way and ev[5] recorded here (synchronises)
+static int read_stage_times(sgpr_context* h, cudaStream_t st) {
+    cudaEventRecord(h->ev[5], st);
+    SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
+    cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
+    cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
+    cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
+    cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
+    cudaEventElapsedTime(&h->stats.ms_beta, h->ev[4], h->ev[5]);
+    cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
+    return SGPR_OK;
+}
+
 static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d, const double* cell_h,
                         const int32_t* pbc_h, int32_t rank, int32_t world, void* stream, double* E_d, double* F_d,
                         double* W_d, double* beta_d, uint8_t* owned_d, const uint64_t* peer_f_h, bool allow_warm,
@@ -1162,16 +1175,7 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
     } else {
         h->warm_ok = false;
     }
-    if (h->timing) {
-        cudaEventRecord(h->ev[5], st);
-        SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
-        cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
-        cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
-        cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
-        cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
-        cudaEventElapsedTime(&h->stats.ms_beta, h->ev[4], h->ev[5]);
-        cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
-    }
+    if (h->timing) SGPR_TRY(read_stage_times(h, st));
     return SGPR_OK;
 }
 
@@ -1454,18 +1458,8 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_host(sgpr_han
     return SGPR_OK;
 }
 
-// B independent structures in one call (include/sgpr_b200.h).  Same stages as a sizing step of sgpr_predict over the
-// concatenated atoms; what differs is per-structure geometry (batched cell sort, neighbour search and image shifts) and
-// the per-structure reductions.  The rows are ordinary descriptor rows: GEMMs, covloss and force scatter are shared.
-extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_handle h, int32_t B, const int64_t* first_h,
-                                                                         const double* pos_d, const int32_t* Z_d,
-                                                                         const double* cell_h, const int32_t* pbc_h,
-                                                                         void* stream, double* E_d, double* F_d,
-                                                                         double* W_d, double* beta_d) {
-    if (!h || B < 0 || !first_h || (B > 0 && (!cell_h || !pbc_h || !E_d || !W_d))) {
-        set_error("null argument");
-        return SGPR_ERR_INVALID;
-    }
+// Atom offsets of a batch of B structures: first_h[0] = 0 and non-decreasing; *N = first_h[B], the batch's atom count.
+static int check_batch_first(int B, const int64_t* first_h, int64_t* N) {
     if (first_h[0] != 0) {
         set_error("first_h[0] = %lld, must be 0", (long long)first_h[0]);
         return SGPR_ERR_INVALID;
@@ -1475,26 +1469,24 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_ha
             set_error("first_h is not monotone at structure %d (%lld > %lld)", b, (long long)first_h[b], (long long)first_h[b + 1]);
             return SGPR_ERR_INVALID;
         }
-    const int64_t N = first_h[B];
-    if (N > 0x7fffff00ll) {
+    *N = first_h[B];
+    if (*N > 0x7fffff00ll) {
         set_error("bad atom count");
         return SGPR_ERR_INVALID;
     }
-    if (N > 0 && (!pos_d || !Z_d || !F_d)) {
-        set_error("null argument");
-        return SGPR_ERR_INVALID;
-    }
-    if (beta_d && !h->has_choli) {
-        set_error("covloss requested but the model has no choli");
-        return SGPR_ERR_INVALID;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    SGPR_CUDA(cudaSetDevice(h->device));
-    h->fwd_valid = false;   // no state for sgpr_kernel_backward
+    return SGPR_OK;
+}
+
+// Front end of the batched entry points, from the state reset to the descriptors of the batch's N atoms: per-structure
+// geometry, batched cell sort and neighbour list, descriptors; fills bg.  i8: the step may use the int8 GEMM engine
+// (when the handle does).  B == 0 stops after the state reset: the caller has nothing more to do.
+static int batch_front(sgpr_context* h, int B, const int64_t* first_h, int64_t N, const double* pos_d, const int32_t* Z_d,
+                       const double* cell_h, const int32_t* pbc_h, cudaStream_t st, bool i8, bool with_k8, BatchGeom* bg) {
+    h->fwd_valid = false;   // no state for sgpr_kernel_backward / sgpr_kernel_jacobian
     h->warm_ok = false;     // the next single-structure step sizes its buffers again
     h->step_was_warm = false;
     if (B == 0) return SGPR_OK;
-    h->use_i8_now = h->use_i8;
+    h->use_i8_now = i8 && h->use_i8;
     h->stats.i8_ops = 0.0;
     h->stats.gemm_flops = 0.0;
     h->stats.covloss_flops = 0.0;
@@ -1527,29 +1519,60 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_ha
     SGPR_CUDA(cudaMemcpyAsync(h->b_first.p, first_h, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
     SGPR_CUDA(cudaMemcpyAsync(h->b_bins.p, bin_base.data(), sizeof(int) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
     SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, cells.data(), sizeof(double) * 9 * (size_t)B, cudaMemcpyHostToDevice, st));
-    BatchGeom bg{};
-    bg.B = B;
-    bg.ncell = (int)ncell;
-    bg.geoms = h->b_geom.as<Geom>();
-    bg.first = h->b_first.as<long long>();
-    bg.bin_base = h->b_bins.as<int>();
-    bg.cells = h->b_cell.as<double>();
-    bg.astr = h->astr.as<int>();
-    bg.err = h->b_err.as<unsigned long long>();
+    *bg = BatchGeom{};
+    bg->B = B;
+    bg->ncell = (int)ncell;
+    bg->geoms = h->b_geom.as<Geom>();
+    bg->first = h->b_first.as<long long>();
+    bg->bin_base = h->b_bins.as<int>();
+    bg->cells = h->b_cell.as<double>();
+    bg->astr = h->astr.as<int>();
+    bg->err = h->b_err.as<unsigned long long>();
     const Geom unused{};
     // cell sort -> neighbour list (the call's one sizing synchronisation) -> descriptors
     if (h->timing) cudaEventRecord(h->ev[0], st);
-    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, bg, st));
+    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, *bg, st));
     int64_t n_pairs = 0;
-    SGPR_TRY(batch_neighbor_build(h, N, bg, st, &n_pairs));
+    SGPR_TRY(batch_neighbor_build(h, N, *bg, st, &n_pairs));
     h->stats.n_active = h->n_active;
     h->stats.n_pairs = n_pairs;
     if (h->timing) cudaEventRecord(h->ev[1], st);
-    const size_t nrows = (size_t)N + 1;
-    SGPR_TRY(h->phat.ensure(sizeof(double) * nrows * h->dp.ldp));
-    if (h->use_i8_now) SGPR_TRY(i8_ensure_step_buffers(h, (size_t)N, beta_d != nullptr));
-    SGPR_TRY(descriptor_forward_atoms(h, unused, st, &bg));
+    SGPR_TRY(h->phat.ensure(sizeof(double) * ((size_t)N + 1) * h->dp.ldp));
+    if (h->use_i8_now) SGPR_TRY(i8_ensure_step_buffers(h, (size_t)N, with_k8));
+    SGPR_TRY(descriptor_forward_atoms(h, unused, st, bg));
     if (h->timing) cudaEventRecord(h->ev[2], st);
+    return SGPR_OK;
+}
+
+// B independent structures in one call (include/sgpr_b200.h).  Same stages as a sizing step of sgpr_predict over the
+// concatenated atoms; what differs is per-structure geometry (batched cell sort, neighbour search and image shifts) and
+// the per-structure reductions.  The rows are ordinary descriptor rows: GEMMs, covloss and force scatter are shared.
+extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_handle h, int32_t B, const int64_t* first_h,
+                                                                         const double* pos_d, const int32_t* Z_d,
+                                                                         const double* cell_h, const int32_t* pbc_h,
+                                                                         void* stream, double* E_d, double* F_d,
+                                                                         double* W_d, double* beta_d) {
+    if (!h || B < 0 || !first_h || (B > 0 && (!cell_h || !pbc_h || !E_d || !W_d))) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    int64_t N = 0;
+    SGPR_TRY(check_batch_first(B, first_h, &N));
+    if (N > 0 && (!pos_d || !Z_d || !F_d)) {
+        set_error("null argument");
+        return SGPR_ERR_INVALID;
+    }
+    if (beta_d && !h->has_choli) {
+        set_error("covloss requested but the model has no choli");
+        return SGPR_ERR_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    SGPR_CUDA(cudaSetDevice(h->device));
+    BatchGeom bg;
+    SGPR_TRY(batch_front(h, B, first_h, N, pos_d, Z_d, cell_h, pbc_h, st, /*i8=*/true, /*with_k8=*/beta_d != nullptr, &bg));
+    if (B == 0) return SGPR_OK;
+    const Geom unused{};
+    const size_t nrows = (size_t)N + 1;
     if (h->use_i8_now) SGPR_TRY(i8_setup_step(h, st));
     int max_part = 1;
     const RowSpecies rs = row_species(h, &max_part);
@@ -1579,15 +1602,33 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_ha
     }
     if (h->timing) cudaEventRecord(h->ev[4], st);
     if (beta_d) SGPR_TRY(covloss_stage(h, st, N, nullptr, nullptr, beta_d));
-    if (h->timing) {
-        cudaEventRecord(h->ev[5], st);
-        SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
-        cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
-        cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
-        cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
-        cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
-        cudaEventElapsedTime(&h->stats.ms_beta, h->ev[4], h->ev[5]);
-        cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
+    if (h->timing) SGPR_TRY(read_stage_times(h, st));
+    return SGPR_OK;
+}
+
+// K [N, M] of the N atoms of the last front end into K (caller's rows and columns, lone-lone term included), FP64 GEMM
+static int kernel_matrix_caller_order(sgpr_context* h, int64_t N, cudaStream_t st, double* K) {
+    SGPR_TRY(h->gmat.ensure(sizeof(double) * ((size_t)N + 1) * h->ldg));
+    {
+        int max_part = 1;
+        for (int s = 0; s < h->S; ++s) max_part = std::max(max_part, gemm_energy_parts(h->m_first[s + 1] - h->m_first[s]));
+        SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * ((size_t)N + 1)));
+    }
+    SGPR_TRY(h->rowmap.ensure(sizeof(int) * ((size_t)N + 1)));
+    SGPR_CUDA(cudaMemsetAsync(K, 0, sizeof(double) * (size_t)N * h->M, st));
+    if (N > 0 && h->M > 0) {
+        row_to_orig_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(),
+                                                                   h->rowof.as<int>() + (N + 1), h->rowmap.as<int>());
+        SGPR_TRY(gemm_kernel_matrix(h, K, h->M, h->rowmap.as<int>(), false, st));
+        // lone-lone term, in the caller's inducing order
+        bool any = false;
+        for (int p = 0; p < h->M; ++p) any |= h->ind_lone[p] != 0;
+        if (any) {
+            lone_k_kernel<<<h->sm_count, 128, 0, st>>>((int)h->n_active, nullptr, h->atoms.as<AtomRec>(),
+                                                       h->nl_first.as<long long>(), h->M, h->ind_sp_d.as<int>(),
+                                                       h->ind_lone_d.as<unsigned char>(), K, h->lone_w);
+        }
+        h->stats.kernel_launches += 2;
     }
     return SGPR_OK;
 }
@@ -1602,28 +1643,7 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_forward(sgpr_h
     SGPR_CUDA(cudaSetDevice(h->device));
     Geom g;
     SGPR_TRY(stage_front(h, N, pos_d, Z_d, cell_h, pbc_h, st, &g));
-    SGPR_TRY(h->gmat.ensure(sizeof(double) * ((size_t)N + 1) * h->ldg));
-    {
-        int max_part = 1;
-        for (int s = 0; s < h->S; ++s) max_part = std::max(max_part, gemm_energy_parts(h->m_first[s + 1] - h->m_first[s]));
-        SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * ((size_t)N + 1)));
-    }
-    SGPR_TRY(h->rowmap.ensure(sizeof(int) * ((size_t)N + 1)));
-    SGPR_CUDA(cudaMemsetAsync(K_d, 0, sizeof(double) * (size_t)N * h->M, st));
-    if (N > 0 && h->M > 0) {
-        row_to_orig_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(),
-                                                                   h->rowof.as<int>() + (N + 1), h->rowmap.as<int>());
-        SGPR_TRY(gemm_kernel_matrix(h, K_d, h->M, h->rowmap.as<int>(), false, st));
-        // lone-lone term, in the caller's inducing order
-        bool any = false;
-        for (int p = 0; p < h->M; ++p) any |= h->ind_lone[p] != 0;
-        if (any) {
-            lone_k_kernel<<<h->sm_count, 128, 0, st>>>((int)h->n_active, nullptr, h->atoms.as<AtomRec>(),
-                                                       h->nl_first.as<long long>(), h->M, h->ind_sp_d.as<int>(),
-                                                       h->ind_lone_d.as<unsigned char>(), K_d, h->lone_w);
-        }
-        h->stats.kernel_launches += 2;
-    }
+    SGPR_TRY(kernel_matrix_caller_order(h, N, st, K_d));
     SGPR_CUDA(cudaGetLastError());
     SGPR_CUDA(cudaStreamSynchronize(st));
     h->fwd_valid = true;
@@ -1648,14 +1668,9 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_backward(sgpr_
     const Geom g = h->last_geom;
     const size_t nrows = (size_t)h->n_active + 1;
     const int nblk_b = backward_grid(h), grid_e = 128, nblk_x = 64;
-    RowSpecies rs{};
-    rs.S = h->S;
+    h->use_i8_now = false;   // the VJP runs the FP64 GEMM (row_species() reads this)
     int max_part = 1;
-    for (int s = 0; s < h->S; ++s) {
-        const int Ms = h->m_first[s + 1] - h->m_first[s];
-        rs.n_part[s] = (Ms > 0 && h->dp.central_enabled[s]) ? gemm_energy_parts(Ms) : 0;
-        max_part = std::max(max_part, rs.n_part[s]);
-    }
+    const RowSpecies rs = row_species(h, &max_part);
     SGPR_TRY(h->gmat.ensure(sizeof(double) * nrows * h->ldg));
     SGPR_TRY(h->gvec.ensure(sizeof(double) * nrows * h->dp.ldp));
     SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * nrows));
@@ -1666,7 +1681,6 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_backward(sgpr_
     SGPR_CUDA(cudaMemsetAsync(h->wpart.p, 0, sizeof(double) * 9 * nblk_b, st));
     SGPR_CUDA(cudaMemsetAsync(h->fcell.p, 0, sizeof(double) * 3 * ((size_t)N + 1), st));
     SGPR_CUDA(cudaMemsetAsync(h->epart.p, 0, sizeof(double) * (grid_e + 16 + 9 * nblk_x), st));
-    h->use_i8_now = false;
     if (N > 0 && h->M > 0) {
         SGPR_TRY(gemm_kernel_matrix(h, nullptr, h->M, h->rowmap.as<int>(), false, st, gK_d));
         row_energy_kernel<<<grid_e, 256, 0, st>>>((int)h->n_active, rs, h->row_first_d.as<int>(), h->erow_part.as<double>(),
@@ -1724,6 +1738,26 @@ static int upload_selection(sgpr_context* h, int m0, int m1, cudaStream_t st, Ja
     return SGPR_OK;
 }
 
+// Jacobian kernel of the last front end's atoms against inducing LCEs m0 <= m < m1 into J_d [ncol, N, 3] and W_d
+// [B, ncol, 9], both zeroed here.  cells_d [B, 9]: the structures' cells; astr_d: structure of each cell-order atom
+// (nullptr: one structure).
+static int jacobian_stage(sgpr_context* h, int m0, int m1, int B, const double* cells_d, const int* astr_d, double* J_d,
+                          double* W_d, cudaStream_t st) {
+    const int64_t N = h->last_N;
+    const int ncol = m1 - m0;
+    JacTarget t{};
+    SGPR_TRY(upload_selection(h, m0, m1, st, &t));
+    t.n_atoms = N;
+    t.J = J_d;
+    t.W = W_d;
+    t.cells = cells_d;
+    t.astr = astr_d;
+    if (N > 0) SGPR_CUDA(cudaMemsetAsync(J_d, 0, sizeof(double) * 3 * (size_t)N * ncol, st));
+    SGPR_CUDA(cudaMemsetAsync(W_d, 0, sizeof(double) * 9 * (size_t)B * ncol, st));
+    if (N > 0) SGPR_TRY(descriptor_jacobian_atoms(h, t, st));
+    return SGPR_OK;
+}
+
 // Training-time kernels of the structure of the LAST sgpr_kernel_forward against inducing LCEs m0 <= m < m1
 // (caller's order): the Jacobian of Ke[m] = sum_i K[i,m] for all of them in one launch (descriptor.cu: jacobian_kernel).
 extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian(sgpr_handle h, int32_t m0, int32_t m1, void* stream, double* J_d, double* W_d) {
@@ -1741,22 +1775,11 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian(sgpr_
     }
     cudaStream_t st = (cudaStream_t)stream;
     SGPR_CUDA(cudaSetDevice(h->device));
-    const int64_t N = h->last_N;
-    const int ncol = m1 - m0;
-    if (ncol == 0) return SGPR_OK;
+    if (m1 == m0) return SGPR_OK;
     h->use_i8_now = false;
-    JacTarget t{};
-    SGPR_TRY(upload_selection(h, m0, m1, st, &t));
     SGPR_TRY(h->b_cell.ensure(sizeof(double) * 9));
     SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, h->last_geom.cell, sizeof(double) * 9, cudaMemcpyHostToDevice, st));
-    t.n_atoms = N;
-    t.J = J_d;
-    t.W = W_d;
-    t.cells = h->b_cell.as<double>();
-    t.astr = nullptr;
-    if (N > 0) SGPR_CUDA(cudaMemsetAsync(J_d, 0, sizeof(double) * 3 * (size_t)N * ncol, st));
-    SGPR_CUDA(cudaMemsetAsync(W_d, 0, sizeof(double) * 9 * (size_t)ncol, st));
-    if (N > 0) SGPR_TRY(descriptor_jacobian_atoms(h, t, st));
+    SGPR_TRY(jacobian_stage(h, m0, m1, 1, h->b_cell.as<double>(), nullptr, J_d, W_d, st));
     SGPR_CUDA(cudaGetLastError());
     SGPR_CUDA(cudaStreamSynchronize(st));
     return SGPR_OK;
@@ -1781,108 +1804,22 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian_batch
         set_error("inducing range [%d, %d) outside [0, %d)", m0, m1, h->M);
         return SGPR_ERR_INVALID;
     }
-    if (first_h[0] != 0) {
-        set_error("first_h[0] = %lld, must be 0", (long long)first_h[0]);
-        return SGPR_ERR_INVALID;
-    }
-    for (int b = 0; b < B; ++b)
-        if (first_h[b + 1] < first_h[b]) {
-            set_error("first_h is not monotone at structure %d (%lld > %lld)", b, (long long)first_h[b], (long long)first_h[b + 1]);
-            return SGPR_ERR_INVALID;
-        }
-    const int64_t N = first_h[B];
-    if (N > 0x7fffff00ll) {
-        set_error("bad atom count");
-        return SGPR_ERR_INVALID;
-    }
+    int64_t N = 0;
+    SGPR_TRY(check_batch_first(B, first_h, &N));
     if (N > 0 && (!pos_d || !Z_d)) {
         set_error("null argument");
         return SGPR_ERR_INVALID;
     }
     cudaStream_t st = (cudaStream_t)stream;
     SGPR_CUDA(cudaSetDevice(h->device));
-    h->fwd_valid = false;   // no state for sgpr_kernel_backward / sgpr_kernel_jacobian
-    h->warm_ok = false;     // the next single-structure step sizes its buffers again
-    h->step_was_warm = false;
+    BatchGeom bg;
+    SGPR_TRY(batch_front(h, B, first_h, N, pos_d, Z_d, cell_h, pbc_h, st, /*i8=*/false, /*with_k8=*/false, &bg));
     if (B == 0) return SGPR_OK;
     const int ncol = m1 - m0;
-    h->use_i8_now = false;
-    h->stats.i8_ops = 0.0;
-    h->stats.gemm_flops = 0.0;
-    h->stats.covloss_flops = 0.0;
-    h->stats.kernel_launches = 0;
-    h->stats.n_atoms = N;
-    h->last_N = N;
-    std::vector<Geom> gs;
-    SGPR_TRY(build_geometry_batch(h, B, first_h, pos_d, cell_h, pbc_h, st, &gs));
-    std::vector<int> bin_base(B + 1, 0);
-    std::vector<double> cells(9 * (size_t)B);
-    long long ncell = 0;
-    for (int b = 0; b < B; ++b) {
-        bin_base[b] = (int)ncell;
-        ncell += gs[b].ncell;
-        for (int q = 0; q < 9; ++q) cells[9 * (size_t)b + q] = gs[b].cell[q];
-    }
-    if ((ncell + 1) * h->S > 0x7fffffffll) {
-        set_error("batch too large: %lld bins", ncell);
-        return SGPR_ERR_INVALID;
-    }
-    bin_base[B] = (int)ncell;
-    SGPR_TRY(h->b_geom.ensure(sizeof(Geom) * (size_t)B));
-    SGPR_TRY(h->b_first.ensure(sizeof(long long) * ((size_t)B + 1)));
-    SGPR_TRY(h->b_bins.ensure(sizeof(int) * ((size_t)B + 1)));
-    SGPR_TRY(h->b_cell.ensure(sizeof(double) * 9 * (size_t)B));
-    SGPR_TRY(h->b_err.ensure(sizeof(unsigned long long) * 2));
-    SGPR_TRY(h->astr.ensure(sizeof(int) * ((size_t)N + 1)));
-    SGPR_CUDA(cudaMemcpyAsync(h->b_geom.p, gs.data(), sizeof(Geom) * (size_t)B, cudaMemcpyHostToDevice, st));
-    SGPR_CUDA(cudaMemcpyAsync(h->b_first.p, first_h, sizeof(long long) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
-    SGPR_CUDA(cudaMemcpyAsync(h->b_bins.p, bin_base.data(), sizeof(int) * ((size_t)B + 1), cudaMemcpyHostToDevice, st));
-    SGPR_CUDA(cudaMemcpyAsync(h->b_cell.p, cells.data(), sizeof(double) * 9 * (size_t)B, cudaMemcpyHostToDevice, st));
-    BatchGeom bg{};
-    bg.B = B;
-    bg.ncell = (int)ncell;
-    bg.geoms = h->b_geom.as<Geom>();
-    bg.first = h->b_first.as<long long>();
-    bg.bin_base = h->b_bins.as<int>();
-    bg.cells = h->b_cell.as<double>();
-    bg.astr = h->astr.as<int>();
-    bg.err = h->b_err.as<unsigned long long>();
-    const Geom unused{};
-    // cell sort -> neighbour list (the call's one sizing synchronisation) -> descriptors
-    if (h->timing) cudaEventRecord(h->ev[0], st);
-    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, bg, st));
-    int64_t n_pairs = 0;
-    SGPR_TRY(batch_neighbor_build(h, N, bg, st, &n_pairs));
-    h->stats.n_active = h->n_active;
-    h->stats.n_pairs = n_pairs;
-    if (h->timing) cudaEventRecord(h->ev[1], st);
-    const size_t nrows = (size_t)N + 1;
-    SGPR_TRY(h->phat.ensure(sizeof(double) * nrows * h->dp.ldp));
-    SGPR_TRY(descriptor_forward_atoms(h, unused, st, &bg));
-    if (h->timing) cudaEventRecord(h->ev[2], st);
     // K [N, M] (caller's rows and columns, lone-lone term included) -> Ke
-    SGPR_TRY(h->gmat.ensure(sizeof(double) * nrows * h->ldg));
-    {
-        int max_part = 1;
-        for (int s = 0; s < h->S; ++s) max_part = std::max(max_part, gemm_energy_parts(h->m_first[s + 1] - h->m_first[s]));
-        SGPR_TRY(h->erow_part.ensure(sizeof(double) * (size_t)max_part * nrows));
-    }
-    SGPR_TRY(h->rowmap.ensure(sizeof(int) * nrows));
     SGPR_TRY(h->kscr.ensure(sizeof(double) * ((size_t)N * h->M + 1)));
     double* K = h->kscr.as<double>();
-    SGPR_CUDA(cudaMemsetAsync(K, 0, sizeof(double) * (size_t)N * h->M, st));
-    if (N > 0 && h->M > 0) {
-        row_to_orig_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1),
-                                                                   h->rowmap.as<int>());
-        SGPR_TRY(gemm_kernel_matrix(h, K, h->M, h->rowmap.as<int>(), false, st));
-        bool any = false;
-        for (int p = 0; p < h->M; ++p) any |= h->ind_lone[p] != 0;
-        if (any)
-            lone_k_kernel<<<h->sm_count, 128, 0, st>>>((int)h->n_active, nullptr, h->atoms.as<AtomRec>(),
-                                                       h->nl_first.as<long long>(), h->M, h->ind_sp_d.as<int>(),
-                                                       h->ind_lone_d.as<unsigned char>(), K, h->lone_w);
-        h->stats.kernel_launches += 2;
-    }
+    SGPR_TRY(kernel_matrix_caller_order(h, N, st, K));
     if (ncol > 0) {
         const long long n = (long long)B * ncol;
         ke_reduce_kernel<<<(int)std::min<long long>((n + 255) / 256, (long long)h->sm_count * 16), 256, 0, st>>>(
@@ -1892,28 +1829,13 @@ extern "C" __attribute__((visibility("default"))) int sgpr_kernel_jacobian_batch
     if (h->timing) cudaEventRecord(h->ev[3], st);
     if (J_d && ncol > 0) {
         NvtxRange jac_range("sgpr:jacobian");
-        JacTarget t{};
-        SGPR_TRY(upload_selection(h, m0, m1, st, &t));
-        t.n_atoms = N;
-        t.J = J_d;
-        t.W = W_d;
-        t.cells = bg.cells;
-        t.astr = bg.astr;
-        if (N > 0) SGPR_CUDA(cudaMemsetAsync(J_d, 0, sizeof(double) * 3 * (size_t)N * ncol, st));
-        SGPR_CUDA(cudaMemsetAsync(W_d, 0, sizeof(double) * 9 * (size_t)B * ncol, st));
-        if (N > 0) SGPR_TRY(descriptor_jacobian_atoms(h, t, st));
+        SGPR_TRY(jacobian_stage(h, m0, m1, B, bg.cells, bg.astr, J_d, W_d, st));
     }
     SGPR_CUDA(cudaGetLastError());
     if (h->timing) {
         cudaEventRecord(h->ev[4], st);
-        cudaEventRecord(h->ev[5], st);
-        SGPR_CUDA(cudaEventSynchronize(h->ev[5]));
-        cudaEventElapsedTime(&h->stats.ms_nl, h->ev[0], h->ev[1]);
-        cudaEventElapsedTime(&h->stats.ms_desc, h->ev[1], h->ev[2]);
-        cudaEventElapsedTime(&h->stats.ms_gemm, h->ev[2], h->ev[3]);
-        cudaEventElapsedTime(&h->stats.ms_force, h->ev[3], h->ev[4]);
+        SGPR_TRY(read_stage_times(h, st));
         h->stats.ms_beta = 0.0f;
-        cudaEventElapsedTime(&h->stats.ms_total, h->ev[0], h->ev[5]);
     }
     return SGPR_OK;
 }

@@ -284,6 +284,33 @@ class SgprEngine:
         z_t = torch.as_tensor(np.ascontiguousarray(numbers, dtype=np.int32)).to(dev) if not torch.is_tensor(numbers) else numbers.to(dev, torch.int32).contiguous()
         return pos_t.reshape(-1, 3), z_t.reshape(-1)
 
+    def _batch(self, pos, numbers, first, cells, pbcs):
+        """Inputs of the batched entry points (``predict_batch``, ``training_kernels``): a list of structures, or
+        concatenated ``pos`` / ``numbers`` with ``first`` [B+1] and ``cells`` / ``pbcs`` (one value for all, or one per
+        structure).  Returns first_h int64 [B+1], B, N, cell_h [B,9], pbc_h int32 [B,3] (host) and pos_t, z_t (device)."""
+        if first is None:
+            images = list(pos)
+            if numbers is not None or cells is not None or pbcs is not None:
+                raise ValueError("pass either a list of structures or pos, numbers, first, cells, pbcs")
+            counts = [len(a.numbers) for a in images]
+            pos = np.concatenate([np.asarray(a.positions, dtype=np.float64).reshape(-1, 3) for a in images]) if images else np.zeros((0, 3))
+            numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images]) if images else np.zeros(0, dtype=np.int32)
+            first = np.concatenate([[0], np.cumsum(counts)])
+            cells = [np.asarray(a.cell, dtype=np.float64).reshape(3, 3) for a in images]
+            pbcs = [np.broadcast_to(np.asarray(a.pbc), (3,)) for a in images]
+        first_h = np.ascontiguousarray(first, dtype=np.int64).reshape(-1)
+        B = len(first_h) - 1
+        if B < 0:
+            raise ValueError("first must have B+1 >= 1 entries")
+        cell_h = np.ascontiguousarray(np.broadcast_to(np.asarray(cells, dtype=np.float64).reshape(-1, 9), (B, 9)))
+        pb = np.asarray(pbcs).astype(np.int32)
+        pbc_h = np.ascontiguousarray(np.broadcast_to(pb.reshape(-1, 3) if pb.size and pb.size % 3 == 0 else pb.reshape(-1, 1), (B, 3)))
+        pos_t, z_t = self._dev(pos, numbers)
+        N = z_t.numel()
+        if pos_t.shape[0] != N or first_h[-1] != N:
+            raise ValueError(f"first[-1] = {first_h[-1]} does not match {N} atoms")
+        return first_h, B, N, cell_h, pbc_h, pos_t, z_t
+
     @staticmethod
     def _stream():
         import torch
@@ -353,27 +380,7 @@ class SgprEngine:
         when ``want_beta``)."""
         import torch
 
-        if first is None:
-            images = list(pos)
-            if numbers is not None or cells is not None or pbcs is not None:
-                raise ValueError("pass either a list of structures or pos, numbers, first, cells, pbcs")
-            counts = [len(a.numbers) for a in images]
-            pos = np.concatenate([np.asarray(a.positions, dtype=np.float64).reshape(-1, 3) for a in images]) if images else np.zeros((0, 3))
-            numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images]) if images else np.zeros(0, dtype=np.int32)
-            first = np.concatenate([[0], np.cumsum(counts)])
-            cells = [np.asarray(a.cell, dtype=np.float64).reshape(3, 3) for a in images]
-            pbcs = [np.broadcast_to(np.asarray(a.pbc), (3,)) for a in images]
-        first_h = np.ascontiguousarray(first, dtype=np.int64).reshape(-1)
-        B = len(first_h) - 1
-        if B < 0:
-            raise ValueError("first must have B+1 >= 1 entries")
-        cell_h = np.ascontiguousarray(np.broadcast_to(np.asarray(cells, dtype=np.float64).reshape(-1, 9), (B, 9)))
-        pb = np.asarray(pbcs).astype(np.int32)
-        pbc_h = np.ascontiguousarray(np.broadcast_to(pb.reshape(-1, 3) if pb.size and pb.size % 3 == 0 else pb.reshape(-1, 1), (B, 3)))
-        pos_t, z_t = self._dev(pos, numbers)
-        N = z_t.numel()
-        if pos_t.shape[0] != N or first_h[-1] != N:
-            raise ValueError(f"first[-1] = {first_h[-1]} does not match {N} atoms")
+        first_h, B, N, cell_h, pbc_h, pos_t, z_t = self._batch(pos, numbers, first, cells, pbcs)
         dev = pos_t.device
         E = torch.zeros(max(B, 1), dtype=torch.float64, device=dev)
         F = torch.zeros((N, 3), dtype=torch.float64, device=dev)
@@ -400,27 +407,7 @@ class SgprEngine:
         the Jacobian and returns ``(Ke, None, None)``.  For B = 1 this is ``kernel_jacobian`` (Ke = K.sum(0))."""
         import torch
 
-        if first is None:
-            images = list(pos)
-            if numbers is not None or cells is not None or pbcs is not None:
-                raise ValueError("pass either a list of structures or pos, numbers, first, cells, pbcs")
-            counts = [len(a.numbers) for a in images]
-            pos = np.concatenate([np.asarray(a.positions, dtype=np.float64).reshape(-1, 3) for a in images]) if images else np.zeros((0, 3))
-            numbers = np.concatenate([np.asarray(a.numbers).reshape(-1) for a in images]) if images else np.zeros(0, dtype=np.int32)
-            first = np.concatenate([[0], np.cumsum(counts)])
-            cells = [np.asarray(a.cell, dtype=np.float64).reshape(3, 3) for a in images]
-            pbcs = [np.broadcast_to(np.asarray(a.pbc), (3,)) for a in images]
-        first_h = np.ascontiguousarray(first, dtype=np.int64).reshape(-1)
-        B = len(first_h) - 1
-        if B < 0:
-            raise ValueError("first must have B+1 >= 1 entries")
-        cell_h = np.ascontiguousarray(np.broadcast_to(np.asarray(cells, dtype=np.float64).reshape(-1, 9), (B, 9)))
-        pb = np.asarray(pbcs).astype(np.int32)
-        pbc_h = np.ascontiguousarray(np.broadcast_to(pb.reshape(-1, 3) if pb.size and pb.size % 3 == 0 else pb.reshape(-1, 1), (B, 3)))
-        pos_t, z_t = self._dev(pos, numbers)
-        N = z_t.numel()
-        if pos_t.shape[0] != N or first_h[-1] != N:
-            raise ValueError(f"first[-1] = {first_h[-1]} does not match {N} atoms")
+        first_h, B, N, cell_h, pbc_h, pos_t, z_t = self._batch(pos, numbers, first, cells, pbcs)
         m1 = self.model.M if m1 is None else int(m1)
         m0 = int(m0)
         if not 0 <= m0 <= m1 <= self.model.M:
