@@ -75,7 +75,7 @@ __global__ void transpose_zhat_kernel(int D, int ldp, int m0, int Ms, int ld_zt,
 // per-atom terms outside the GEMM: constant mean (gppotential.py:219-227), the
 // "lone atoms" kernel term (similarity.py:94-103), scatter of forces to caller order
 __global__ void atom_terms_kernel(int64_t N, int n_active, const int* __restrict__ active,
-                                  const AtomRec* __restrict__ atoms, const long long* __restrict__ nl_first,
+                                  const AtomRec* __restrict__ atoms, const longlong2* __restrict__ nl_rows,
                                   const unsigned char* __restrict__ owned, const double* __restrict__ mean_w,
                                   const double* __restrict__ lone_mu, double* __restrict__ part) {
     __shared__ double red[256];
@@ -85,7 +85,7 @@ __global__ void atom_terms_kernel(int64_t N, int n_active, const int* __restrict
         if (owned && !owned[c]) continue;
         const int sp = meta_species(atoms[c].meta);
         s += mean_w[sp];
-        if (nl_first[env + 1] == nl_first[env]) s += lone_mu[sp];
+        if (nl_rows[env].y == nl_rows[env].x) s += lone_mu[sp];
     }
     red[threadIdx.x] = s;
     __syncthreads();
@@ -98,7 +98,7 @@ __global__ void atom_terms_kernel(int64_t N, int n_active, const int* __restrict
 
 // covloss (calculator/active.py:781-804): beta_i = sqrt(clamp(1 - c_i, 0)) * sqrt(vscale[Z_i])
 __global__ void beta_finish_kernel(int n_active, const int* __restrict__ active, const AtomRec* __restrict__ atoms,
-                                   const int* __restrict__ rowof, const long long* __restrict__ nl_first,
+                                   const int* __restrict__ rowof, const longlong2* __restrict__ nl_rows,
                                    const unsigned char* __restrict__ owned, const unsigned char* __restrict__ sp_on,
                                    const int* __restrict__ sp_enabled, const double* __restrict__ cpart, int n_part,
                                    int part_ld, const double* __restrict__ clone, const double* __restrict__ vscale,
@@ -109,7 +109,7 @@ __global__ void beta_finish_kernel(int n_active, const int* __restrict__ active,
         const unsigned long long meta = atoms[c].meta;
         const int sp = meta_species(meta);
         double cc = 0.0;
-        const bool lone = nl_first[env + 1] == nl_first[env];
+        const bool lone = nl_rows[env].y == nl_rows[env].x;
         if (lone) {
             cc = clone[sp];
         } else if (sp_on[sp]) {
@@ -250,11 +250,11 @@ __global__ void orig_to_row_kernel(int64_t N, const AtomRec* __restrict__ atoms,
 }
 
 __global__ void lone_k_kernel(int n_active, const int* __restrict__ active, const AtomRec* __restrict__ atoms,
-                              const long long* __restrict__ nl_first, int M, const int* __restrict__ ind_sp,
+                              const longlong2* __restrict__ nl_rows, int M, const int* __restrict__ ind_sp,
                               const unsigned char* __restrict__ ind_lone, double* __restrict__ K, double lone_w) {
     // K[i,m] += 1 when both LCEs have no neighbours and the same species (similarity.py:94-103)
     for (int env = blockIdx.x; env < n_active; env += gridDim.x) {
-        if (nl_first[env + 1] != nl_first[env]) continue;
+        if (nl_rows[env].y != nl_rows[env].x) continue;
         const int c = active ? active[env] : env;
         const int sp = meta_species(atoms[c].meta);
         const int i = meta_orig(atoms[c].meta);
@@ -381,7 +381,7 @@ __global__ void p2p_publish_wait_kernel(int rank, int world, P2PPeers peers, con
 }
 
 // CSR neighbour list in the caller's atom order (parity hook)
-__global__ void nl_count_orig_kernel(int64_t N, const AtomRec* __restrict__ atoms, const long long* __restrict__ nl_first,
+__global__ void nl_count_orig_kernel(int64_t N, const AtomRec* __restrict__ atoms, const longlong2* __restrict__ nl_rows,
                                      long long* __restrict__ cnt) {
     int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (c > N) return;
@@ -389,17 +389,17 @@ __global__ void nl_count_orig_kernel(int64_t N, const AtomRec* __restrict__ atom
         cnt[N] = 0;
         return;
     }
-    cnt[meta_orig(atoms[c].meta)] = nl_first[c + 1] - nl_first[c];
+    cnt[meta_orig(atoms[c].meta)] = nl_rows[c].y - nl_rows[c].x;
 }
 __global__ void nl_export_kernel(int64_t N, const AtomRec* __restrict__ atoms, const PairRec* __restrict__ pairs,
-                                 const long long* __restrict__ nl_first, const long long* __restrict__ first_out,
+                                 const longlong2* __restrict__ nl_rows, const long long* __restrict__ first_out,
                                  int32_t* __restrict__ j_out, int8_t* __restrict__ S_out) {
     const int lane = threadIdx.x & 31;
     const int64_t c = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     if (c >= N) return;
     const AtomRec ai = atoms[c];
     const long long o = first_out[meta_orig(ai.meta)];
-    const long long beg = nl_first[c], end = nl_first[c + 1];
+    const long long beg = nl_rows[c].x, end = nl_rows[c].y;
     for (long long k = beg + lane; k < end; k += 32) {
         const PairRec pr = pairs[k];
         const AtomRec aj = atoms[pr.j];
@@ -414,7 +414,7 @@ __global__ void nl_export_kernel(int64_t N, const AtomRec* __restrict__ atoms, c
 // first[b+1]-1 (structure-major keys), whose order depends on that structure alone; lane-strided partial sums and a
 // fixed shuffle tree make E and W reproducible and independent of the rest of the batch.
 __global__ void batch_reduce_kernel(int B, const long long* __restrict__ first, const AtomRec* __restrict__ atoms,
-                                    const int* __restrict__ rowof, const long long* __restrict__ nl_first,
+                                    const int* __restrict__ rowof, const longlong2* __restrict__ nl_rows,
                                     const double* __restrict__ erow, const double* __restrict__ mean_w,
                                     const double* __restrict__ lone_mu, const double* __restrict__ wenv,
                                     double* __restrict__ E, double* __restrict__ W) {
@@ -426,7 +426,7 @@ __global__ void batch_reduce_kernel(int B, const long long* __restrict__ first, 
         const int sp = meta_species(atoms[c].meta);
         e += erow[rowof[c]];
         e += mean_w[sp];
-        if (nl_first[c + 1] == nl_first[c]) e += lone_mu[sp];
+        if (nl_rows[c].y == nl_rows[c].x) e += lone_mu[sp];
 #pragma unroll
         for (int q = 0; q < 9; ++q) w[q] += wenv[9 * c + q];
     }
@@ -739,7 +739,7 @@ extern "C" __attribute__((visibility("default"))) int sgpr_create(const sgpr_mod
     h->lone_w = d->lone_weight > 0 ? d->lone_weight : (d->lone_weight < 0 ? 0.0 : 1.0);
     h->xi_int = (d->xi == std::floor(d->xi) && d->xi >= 1 && d->xi <= 64) ? (int)d->xi : -1;
     SGPR_TRY(upload(h->ztab, h->z_to_species, sizeof(int) * 128));
-    SGPR_TRY(h->errflag.ensure(sizeof(int) * 4));
+    SGPR_TRY(h->errflag.ensure(kErrflagBytes));
     SGPR_TRY(h->status_d.ensure(sizeof(long long) * 8));
     SGPR_CUDA(cudaMemset(h->status_d.p, 0, sizeof(long long) * 8));
     SGPR_CUDA(cudaMallocHost((void**)&h->status_pinned, sizeof(long long) * 8));
@@ -826,7 +826,7 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->nl_first, &h->nl_pairs, &h->scan_tmp, &h->phat, &h->cbuf, &h->pnorm, &h->sflag, &h->gmat,
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
-                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_run, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
+                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_rows, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
                       &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr,
                       &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part,
                       &h->rx_pos, &h->rx_vel, &h->rx_F, &h->rx_beta, &h->rx_ew, &h->rx_part};
@@ -1023,7 +1023,7 @@ static int covloss_stage(sgpr_context* h, cudaStream_t st, int64_t N, const int*
         SGPR_CUDA(cudaMemcpyAsync(h->misc.p, h->dp.central_enabled, sizeof(int) * SGPR_MAX_SPECIES,
                                   cudaMemcpyHostToDevice, st));
         beta_finish_kernel<<<h->sm_count * 2, 256, 0, st>>>(
-            (int)h->n_active, active, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1), h->nl_first.as<long long>(),
+            (int)h->n_active, active, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1), h->nl_rows.as<longlong2>(),
             owned, h->sp_on.as<unsigned char>(), h->misc.as<int>(), h->cpart.as<double>(), n_part, (int)nrows,
             h->clone_d.as<double>(), h->vscale_d.as<double>(), h->prow.as<double>(), h->dp.normalize, h->xi, beta_d);
         h->stats.kernel_launches += 1;
@@ -1085,7 +1085,7 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
         W_d = h->p2p_local.as<double>() + 1;
     }
     // Sync-free ("warm") step: every size the host needs was fixed by an earlier sizing step of the same shape; the
-    // pair count, the species row ranges and the error flags stay on the device (nl.cu: nl_status_kernel).
+    // pair count, the species row ranges and the error flags stay on the device (nl.cu: nl_finish_kernel).
     const bool halo_mode = world > 1 && peer_f_h == nullptr;
     const bool shape_ok = h->use_i8 && pbc_h[0] && pbc_h[1] && pbc_h[2] && !halo_mode;
     const bool warm = allow_warm && warm_possible(h, N, pbc_h, rank, world, peer_f_h != nullptr, beta_d != nullptr);
@@ -1137,7 +1137,7 @@ static int predict_body(sgpr_handle h, int64_t N, const double* pos_d, const int
     }
     if (N > 0) {
         atom_terms_kernel<<<nblk_x, 256, 0, st>>>(N, (int)h->n_active, active, h->atoms.as<AtomRec>(),
-                                                  h->nl_first.as<long long>(), owned, h->mean_w_d.as<double>(),
+                                                  h->nl_rows.as<longlong2>(), owned, h->mean_w_d.as<double>(),
                                                   h->lone_mu.as<double>(),
                                                   h->epart.as<double>() + (size_t)grid_g);
         if (!peer_f_h)
@@ -1594,7 +1594,7 @@ extern "C" __attribute__((visibility("default"))) int sgpr_predict_batch(sgpr_ha
             scatter_forces_kernel<<<(int)((N + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->fcell.as<double>(),
                                                                           nullptr, F_d, nullptr);
         batch_reduce_kernel<<<(B + 7) / 8, 256, 0, st>>>(B, bg.first, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1),
-                                                        h->nl_first.as<long long>(), h->erow.as<double>(),
+                                                        h->nl_rows.as<longlong2>(), h->erow.as<double>(),
                                                         h->mean_w_d.as<double>(), h->lone_mu.as<double>(),
                                                         h->wenv.as<double>(), E_d, W_d);
         h->stats.kernel_launches += 2;
@@ -1625,7 +1625,7 @@ static int kernel_matrix_caller_order(sgpr_context* h, int64_t N, cudaStream_t s
         for (int p = 0; p < h->M; ++p) any |= h->ind_lone[p] != 0;
         if (any) {
             lone_k_kernel<<<h->sm_count, 128, 0, st>>>((int)h->n_active, nullptr, h->atoms.as<AtomRec>(),
-                                                       h->nl_first.as<long long>(), h->M, h->ind_sp_d.as<int>(),
+                                                       h->nl_rows.as<longlong2>(), h->M, h->ind_sp_d.as<int>(),
                                                        h->ind_lone_d.as<unsigned char>(), K, h->lone_w);
         }
         h->stats.kernel_launches += 2;
@@ -1866,11 +1866,11 @@ extern "C" __attribute__((visibility("default"))) int sgpr_neighbors(sgpr_handle
     SGPR_TRY(h->misc.ensure(sizeof(long long) * ((size_t)N + 2)));
     long long* cnt = h->misc.as<long long>();
     nl_count_orig_kernel<<<(int)((N + 1 + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(),
-                                                                     h->nl_first.as<long long>(), cnt);
+                                                                     h->nl_rows.as<longlong2>(), cnt);
     SGPR_TRY(scan_exclusive_ll(h, cnt, (long long*)first_d, (int)N + 1, st));
     if (n_pairs <= capacity && N > 0 && j_d && S_d) {
         nl_export_kernel<<<(int)((N * 32 + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->nl_pairs.as<PairRec>(),
-                                                                      h->nl_first.as<long long>(), (const long long*)first_d,
+                                                                      h->nl_rows.as<longlong2>(), (const long long*)first_d,
                                                                       j_d, S_d);
     }
     SGPR_CUDA(cudaGetLastError());

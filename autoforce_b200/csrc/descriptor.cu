@@ -50,7 +50,7 @@ struct EnvSrc {
     // atoms mode
     const AtomRec* atoms;
     const PairRec* pairs;
-    const long long* nl_first;
+    const longlong2* nl_rows;   // (begin, end) of each environment's row in pairs
     const int* active;   // env -> cell-order index (nullptr: identity)
     // explicit-environment mode (inducing LCEs)
     const long long* env_first;
@@ -191,8 +191,9 @@ __global__ void __launch_bounds__(128, (LMAX <= 3 ? 7 : 4)) desc_forward_kernel(
         } else {
             c = src.active ? src.active[env] : env;
             ai = src.atoms[c];
-            beg = src.nl_first[env];
-            end = src.nl_first[env + 1];
+            const longlong2 row = src.nl_rows[env];
+            beg = row.x;
+            end = row.y;
         }
         [[maybe_unused]] CellRef cref{nullptr};
         if constexpr (BATCH) cref.cell = bcell + 9 * (size_t)astr[c];
@@ -566,7 +567,7 @@ __global__ void __launch_bounds__(128, (NB <= 4 ? 4 : 3)) desc_backward_kernel(D
 #pragma unroll
             for (int q = 0; q < 9; ++q) Wacc[q] = 0.0;
         }
-        const long long beg = src.nl_first[env], end = src.nl_first[env + 1];
+        const long long beg = src.nl_rows[env].x, end = src.nl_rows[env].y;
         const bool skip = end == beg || !out.sp_on[si];   // warp-uniform
         const bool flag = sflag[env] != 0;
         // chain rule through the normalisation (sesoap.py:229-235): dE/dq = (g - q_hat (q_hat.g)) / P with
@@ -847,7 +848,7 @@ __global__ void __launch_bounds__(128, 1) jacobian_kernel(DescParams dp, EnvSrc 
     const int c = src.active ? src.active[env] : env;
     const AtomRec ai = src.atoms[c];
     const int si = meta_species(ai.meta);
-    const long long beg = src.nl_first[env], end = src.nl_first[env + 1];
+    const long long beg = src.nl_rows[env].x, end = src.nl_rows[env].y;
     const int t0 = out.sel_first[si] + tile * MT, t1 = out.sel_first[si + 1];
     // lone centres (constant K), excluded centres (K = 0) and tiles past the species' LCEs: nothing to add
     if (t0 >= t1 || end == beg || !dp.central_enabled[si]) return;
@@ -1268,7 +1269,7 @@ int descriptor_jacobian_atoms(sgpr_context* h, const JacTarget& t, cudaStream_t 
     EnvSrc src{};
     src.atoms = h->atoms.as<AtomRec>();
     src.pairs = h->nl_pairs.as<PairRec>();
-    src.nl_first = h->nl_first.as<long long>();
+    src.nl_rows = h->nl_rows.as<longlong2>();
     src.active = h->active_all ? nullptr : h->active_list.as<int>();
     JacArgs a{};
     a.sel = t.sel;
@@ -1317,7 +1318,7 @@ int descriptor_forward_atoms(sgpr_context* h, const Geom& g, cudaStream_t st, co
     EnvSrc src{};
     src.atoms = h->atoms.as<AtomRec>();
     src.pairs = h->nl_pairs.as<PairRec>();
-    src.nl_first = h->nl_first.as<long long>();
+    src.nl_rows = h->nl_rows.as<longlong2>();
     src.active = h->active_all ? nullptr : h->active_list.as<int>();
     if (bg)
         return dispatch_forward<false, true>(h, g, na, src, h->rowof.as<int>() + (h->last_N + 1), h->phat.as<double>(),
@@ -1354,7 +1355,7 @@ int descriptor_backward_atoms(sgpr_context* h, const Geom& g, const unsigned cha
     EnvSrc src{};
     src.atoms = h->atoms.as<AtomRec>();
     src.pairs = h->nl_pairs.as<PairRec>();
-    src.nl_first = h->nl_first.as<long long>();
+    src.nl_rows = h->nl_rows.as<longlong2>();
     src.active = h->active_all ? nullptr : h->active_list.as<int>();
     BackOut out{};
     if (peers) out.peers = *peers;

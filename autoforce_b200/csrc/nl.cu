@@ -537,7 +537,7 @@ int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_
     int* rank = key + (N + 1);
     int* err = h->errflag.as<int>();
     SGPR_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (nkeys + 1), st));
-    SGPR_CUDA(cudaMemsetAsync(err, 0, sizeof(int) * 4, st));
+    SGPR_CUDA(cudaMemsetAsync(err, 0, kErrflagBytes, st));   // error flags and the pair cursor
     const int T = 256;
     const int nblkN = (int)((N + T - 1) / T);
     const int nblkK = (nkeys + T - 1) / T;
@@ -655,7 +655,7 @@ int batch_cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32
     int* key = h->keyrank.as<int>();
     int* rank = key + (N + 1);
     SGPR_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (nkeys + 1), st));
-    SGPR_CUDA(cudaMemsetAsync(h->errflag.p, 0, sizeof(int) * 4, st));
+    SGPR_CUDA(cudaMemsetAsync(h->errflag.p, 0, kErrflagBytes, st));   // error flags and the pair cursor
     SGPR_CUDA(cudaMemsetAsync(bg.err, 0x7f, sizeof(unsigned long long) * 2, st));
     const int T = 256;
     const int nblkN = (int)((N + T - 1) / T);
@@ -756,11 +756,14 @@ __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, cons
                                                        const AtomRec* __restrict__ atoms, const int* __restrict__ abin,
                                                        const int* __restrict__ cstart, Geom g_call, int S,
                                                        int* __restrict__ nl_cnt, const long long* __restrict__ nl_first,
-                                                       PairRec* __restrict__ pairs, unsigned char* __restrict__ mark,
-                                                       unsigned* __restrict__ masks, BatchGeom bg = BatchGeom{}) {
+                                                       const long long* __restrict__ cursor, long long cap,
+                                                       longlong2* __restrict__ rows, PairRec* __restrict__ pairs,
+                                                       unsigned char* __restrict__ mark, unsigned* __restrict__ masks,
+                                                       BatchGeom bg = BatchGeom{}) {
     const int lane = threadIdx.x & 31;
     int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (wid >= n_env) return;
+    const int k_env = wid;   // index among this launch's environments (nl_first)
     wid += env0;  // index into the active list / the neighbour-list rows
     const int c = active ? active[wid] : wid;
     int sb = 0, bbase = 0;
@@ -784,13 +787,18 @@ __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, cons
     const double rc2_lo = rc2 * (1.0 - 1e-14), rc2_hi = rc2 * (1.0 + 1e-14);
 #pragma unroll
     for (int s = 0; s < NS; ++s) count[s] = 0;
+    bool fits = true;
     if (FILL) {
-        long long o = nl_first[wid];
+        // this launch's rows follow the pairs already reserved on the cursor (block-per-bin rows of the same step)
+        const long long row0 = *cursor + nl_first[k_env];
+        long long o = row0;
 #pragma unroll
         for (int s = 0; s < NS; ++s) {
             base[s] = o;
             if (s < S) o += nl_cnt[(long long)wid * S + s];
         }
+        if (lane == 0) rows[wid] = make_longlong2(row0, o);
+        fits = o <= cap;   // an invalid warm step writes no pairs (nl_finish_kernel empties its rows)
     }
     for (int dx = -g.reach[0]; dx <= g.reach[0]; ++dx) {
         int nx, sx;
@@ -844,7 +852,7 @@ __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, cons
 #pragma unroll
                         for (int s = 0; s < NS; ++s) {
                             const unsigned m = __ballot_sync(0xffffffffu, acc && sp == s);
-                            if (acc && sp == s) {
+                            if (fits && acc && sp == s) {
                                 PairRec pr;
                                 pr.j = p;
                                 pr.sb[0] = (signed char)sx;
@@ -877,23 +885,27 @@ __global__ void __launch_bounds__(256) neighbor_kernel(int env0, int n_env, cons
 }
 
 // ---------------------------------------------------------------------------------
-// neighbour search, one BLOCK per bin (the path for all but tiny systems): every atom of a bin walks the
-// same stencil, so the block gathers the candidates of the stencil once into shared memory -- already
-// shifted to the right periodic image -- and its warps then test their atoms against that tile without
-// touching global memory.  Same two passes, masks, pair order and exact accept rule as neighbor_kernel:
-// the shared-memory test decides everything except d^2 within 1e-11 of rc^2, which goes through
-// pair_test (the reference's rounding sequence).
+// neighbour search, one BLOCK per bin (the path for all but tiny systems), in ONE pass: every atom of a bin walks the
+// same stencil, so the block gathers the candidates of the stencil once into shared memory -- already shifted to the
+// right periodic image -- and its warps test their atoms against that tile without touching global memory.  The
+// accept bits stay in shared memory; the block then reserves the rows of its atoms in nl_pairs with one atomicAdd on
+// the pair cursor and writes the pairs from the bits.  Inside a row the pairs are ordered by species, then tile, then
+// lane, then slot (the descriptor kernels sum a row in this order); the accept rule is neighbor_kernel's: the
+// shared-memory test decides everything except d^2 within 1e-11 of rc^2, which goes through pair_test (the reference's
+// rounding sequence).
+// Rows land in nl_pairs in whatever order the atomics hand out the segments: consumers read [begin, end) of a row.
 // ---------------------------------------------------------------------------------
 constexpr int kBinThreads = 256, kBinCap = 1024, kRunChunk = 128;
+constexpr int kBinAtoms = 32;   // atoms per round of a block (one lane each in the reservation); crowded bins take several
 
-template <bool FILL, int NS>
+template <int NS>
 __global__ void __launch_bounds__(kBinThreads, 4) neighbor_bin_kernel(int c_begin, int c_end, int env0,
                                                                    const AtomRec* __restrict__ atoms,
-                                                                   const int* __restrict__ cstart, Geom g, int S,
-                                                                   int* __restrict__ nl_cnt,
-                                                                   const long long* __restrict__ nl_first,
-                                                                   PairRec* __restrict__ pairs, unsigned char* __restrict__ mark,
-                                                                   unsigned* __restrict__ masks, int* __restrict__ nl_run) {
+                                                                   const int* __restrict__ cstart,
+                                                                   const __grid_constant__ Geom g, int S,
+                                                                   long long* __restrict__ cursor, long long cap,
+                                                                   longlong2* __restrict__ rows, PairRec* __restrict__ pairs,
+                                                                   unsigned char* __restrict__ mark) {
     // candidate image relative to the bin's first atom, in float (x, y, z), and w = |x| + |y| + |z| of the unshifted and
     // shifted absolute coordinates (rounding bound of the double-precision test)
     __shared__ float4 rel[kBinCap];
@@ -902,6 +914,12 @@ __global__ void __launch_bounds__(kBinThreads, 4) neighbor_bin_kernel(int c_begi
     __shared__ unsigned code[kBinCap];       // bin shift (3 x int8) | species << 24
     __shared__ int run_beg[kRunChunk], run_pre[kRunChunk + 1];
     __shared__ unsigned run_sh[kRunChunk];
+    __shared__ unsigned long long acc_s[kBinAtoms][32];   // accept bits of an atom: bit k of lane l = candidate (slot k, l)
+    __shared__ int cnt_s[kBinAtoms][NS];     // accepted candidates per species over the whole stencil
+    __shared__ int done_s[kBinAtoms][NS];    // pairs per species written by earlier tiles
+    __shared__ long long row_s[kBinAtoms];   // first pair of the row
+    __shared__ int fits_s;                   // the round's segment lies inside nl_pairs
+    __shared__ unsigned smask_s[NS][32];     // bit b of [s][l]: candidate (batch b, lane l) of the tile has species s
     const int bin = blockIdx.x;
     const int lo = max(cstart[bin * S], c_begin), hi = min(cstart[(bin + 1) * S], c_end);
     if (lo >= hi) return;
@@ -925,10 +943,11 @@ __global__ void __launch_bounds__(kBinThreads, 4) neighbor_bin_kernel(int c_begi
     const double rc2 = g.rc * g.rc;
     const double fast_lo = rc2 * (1.0 - 1e-11), fast_hi = rc2 * (1.0 + 1e-11);
     const double rc2_lo = rc2 * (1.0 - 1e-14), rc2_hi = rc2 * (1.0 + 1e-14);
-    int slot_base = 0, tile_no = 0;
-    for (int r0 = 0; r0 < nruns; r0 += kRunChunk) {
-        const int nr = min(kRunChunk, nruns - r0);
-        __syncthreads();
+
+    // runs r0 .. r0+nr-1 of the stencil: first candidate, count (run_pre: exclusive prefix) and bin shift
+    auto stage_runs = [&](int r0, int nr) {
+        __syncthreads();   // the previous tile is still being read
+        for (int t = threadIdx.x; t < NS * 32; t += kBinThreads) smask_s[t >> 5][t & 31] = 0u;
         for (int t = threadIdx.x; t < nr; t += kBinThreads) {
             const int r = r0 + t;
             const int iz = r % nzr, iy = (r / nzr) % nyr, ix = r / (nzr * nyr);
@@ -955,277 +974,308 @@ __global__ void __launch_bounds__(kBinThreads, 4) neighbor_bin_kernel(int c_begi
             for (int t = 0; t < nr; ++t) run_pre[t + 1] += run_pre[t];
         }
         __syncthreads();
-        const int total = run_pre[nr];
-        for (int t0 = 0; t0 < total; t0 += kBinCap) {
-            const int n = min(kBinCap, total - t0);
-            const bool last_tile = (r0 + kRunChunk >= nruns) && (t0 + kBinCap >= total);
-            if (t0 > 0) __syncthreads();   // the previous tile is still being read
-            float my_max = 0.0f;
-            for (int q = threadIdx.x; q < n; q += kBinThreads) {
-                const int gq = t0 + q;
-                int a = 0, b = nr;          // last run with run_pre[a] <= gq
-                while (b - a > 1) {
-                    const int mid = (a + b) >> 1;
-                    if (run_pre[mid] <= gq) a = mid;
-                    else b = mid;
-                }
-                const int p = run_beg[a] + (gq - run_pre[a]);
-                const AtomRec aj = atoms[p];
-                const unsigned sh = run_sh[a];
-                double s0, s1, s2;
-                shift_vec(g, (int)(signed char)(sh & 0xff) - meta_w(aj.meta, 0), (int)(signed char)((sh >> 8) & 0xff) - meta_w(aj.meta, 1),
-                          (int)(signed char)((sh >> 16) & 0xff) - meta_w(aj.meta, 2), s0, s1, s2);
-                const float fx = (float)((aj.x + s0) - refx), fy = (float)((aj.y + s1) - refy), fz = (float)((aj.z + s2) - refz);
-                rel[q] = make_float4(fx, fy, fz,
-                                     (float)(fabs(aj.x) + fabs(aj.y) + fabs(aj.z) + fabs(s0) + fabs(s1) + fabs(s2)) * 1.0001f);
-                my_max = fmaxf(my_max, fabsf(fx) + fabsf(fy) + fabsf(fz));
-                pj[q] = p;
-                code[q] = sh | ((unsigned)meta_species(aj.meta) << 24);
-            }
-            {
-                const unsigned m = __reduce_max_sync(0xffffffffu, __float_as_uint(my_max));   // floats >= 0 order as uints
-                if (lane == 0 && m > 0u) atomicMax(&maxabs_u, m);
-            }
+    };
+    // candidates t0 .. t0+n-1 of the staged runs into the tile
+    auto stage_tile = [&](int nr, int t0, int n) {
+        if (t0 > 0) {
+            __syncthreads();   // the previous tile is still being read
+            for (int t = threadIdx.x; t < NS * 32; t += kBinThreads) smask_s[t >> 5][t & 31] = 0u;
             __syncthreads();
-            const float maxabs = __uint_as_float(maxabs_u);
-            // accept bits of an environment: one 64-bit word per lane, bit k = candidate (slot k, this lane)
-            const int nb_tile = (n + 31) >> 5;
-            const int nb_masked = max(0, min(nb_tile, kMaskSlots - slot_base));   // batches of this tile covered by the word
-            for (int c = lo + warp; c < hi; c += NW) {
-                const int wid = c - c_begin + env0;
-                const AtomRec ai = atoms[c];
-                unsigned long long* my_word = reinterpret_cast<unsigned long long*>(masks) + (size_t)wid * 32 + lane;
-                unsigned long long accw = 0ull;
-                long long first_pair = 0;
-                int cnt_s[NS];
-                if (FILL) {
-                    accw = *my_word;
-                    first_pair = nl_first[wid];
+        }
+        float my_max = 0.0f;
+        for (int q = threadIdx.x; q < n; q += kBinThreads) {
+            const int gq = t0 + q;
+            int a = 0, b = nr;          // last run with run_pre[a] <= gq
+            while (b - a > 1) {
+                const int mid = (a + b) >> 1;
+                if (run_pre[mid] <= gq) a = mid;
+                else b = mid;
+            }
+            const int p = run_beg[a] + (gq - run_pre[a]);
+            const AtomRec aj = atoms[p];
+            const unsigned sh = run_sh[a];
+            double s0, s1, s2;
+            shift_vec(g, (int)(signed char)(sh & 0xff) - meta_w(aj.meta, 0), (int)(signed char)((sh >> 8) & 0xff) - meta_w(aj.meta, 1),
+                      (int)(signed char)((sh >> 16) & 0xff) - meta_w(aj.meta, 2), s0, s1, s2);
+            const float fx = (float)((aj.x + s0) - refx), fy = (float)((aj.y + s1) - refy), fz = (float)((aj.z + s2) - refz);
+            rel[q] = make_float4(fx, fy, fz,
+                                 (float)(fabs(aj.x) + fabs(aj.y) + fabs(aj.z) + fabs(s0) + fabs(s1) + fabs(s2)) * 1.0001f);
+            my_max = fmaxf(my_max, fabsf(fx) + fabsf(fy) + fabsf(fz));
+            pj[q] = p;
+            code[q] = sh | ((unsigned)meta_species(aj.meta) << 24);
+            atomicOr(&smask_s[meta_species(aj.meta)][q & 31], 1u << (q >> 5));
+        }
+        {
+            const unsigned m = __reduce_max_sync(0xffffffffu, __float_as_uint(my_max));   // floats >= 0 order as uints
+            if (lane == 0 && m > 0u) atomicMax(&maxabs_u, m);
+        }
+        __syncthreads();
+    };
+    // one atom against the tile: COUNT pass (accept bits, per-species counts, halo marks) or EMIT pass (pairs)
+    auto visit = [&](bool emit, int c, int a, int n, int slot_base) {
+        const AtomRec ai = atoms[c];
+        const float maxabs = __uint_as_float(maxabs_u);
+        double w0, w1, w2;
+        shift_vec(g, meta_w(ai.meta, 0), meta_w(ai.meta, 1), meta_w(ai.meta, 2), w0, w1, w2);
+        const double xi = ai.x - w0, yi = ai.y - w1, zi = ai.z - w2;   // the atom's image inside the box
+        // |d2 - d2_reference| <= ~2 rc sqrt(3) * (rounding of the coordinates involved): the band in which the
+        // shared-memory test may disagree with the reference's rounding sequence grows with the coordinates'
+        // magnitude (unwrapped trajectories far from the origin)
+        const double imag = fabs(ai.x) + fabs(ai.y) + fabs(ai.z) + fabs(w0) + fabs(w1) + fabs(w2);
+        // distance test of candidate q.  Float coordinates relative to the bin decide everything farther from the
+        // cutoff sphere than their rounding error: with coordinates of 1-norm <= m the float d2 is off by less
+        // than 2^-24 (7 m |d| + 5 d^2) <= 2^-19 (m^2 + rc^2) wherever a decision is taken -- the margin is 4x
+        // that.  Inside the margin (and for d2 ~ 0: the atom itself) the double-precision test decides, with the
+        // reference's exact rounding sequence only in its own, much narrower band.
+        const float fxi = (float)(xi - refx), fyi = (float)(yi - refy), fzi = (float)(zi - refz);
+        const float mx = fmaxf(maxabs, fabsf(fxi) + fabsf(fyi) + fabsf(fzi));
+        const float margin = 7.62939453125e-6f * (mx * mx + (float)rc2);   // 2^-17
+        const float lo_f = (float)rc2 - margin, hi_f = (float)rc2 + margin;
+        // candidates the float test leaves undecided (rare)
+        auto exact = [&](int q) -> bool {
+            const float4 cq = rel[q];
+            const unsigned cd = code[q];
+            const int p = pj[q];
+            if (p == c && (cd & 0xffffffu) == 0u) return false;   // the atom itself (zero image shift)
+            const AtomRec aj = atoms[p];
+            const int sx = (int)(signed char)(cd & 0xff), sy = (int)(signed char)((cd >> 8) & 0xff),
+                      sz = (int)(signed char)((cd >> 16) & 0xff);
+            double s0, s1, s2;
+            shift_vec(g, sx - meta_w(aj.meta, 0), sy - meta_w(aj.meta, 1), sz - meta_w(aj.meta, 2), s0, s1, s2);
+            const double dx = (aj.x + s0) - xi, dy = (aj.y + s1) - yi, dz = (aj.z + s2) - zi;
+            const double d2 = dx * dx + dy * dy + dz * dz;
+            const double band = 3.6e-15 * g.rc * ((double)cq.w + imag);   // 2^-48 rc (|x_j| + |x_i| + shifts)
+            if (d2 < fast_lo - band) return true;
+            if (d2 > fast_hi + band) return false;
+            double sh0, sh1, sh2;
+            shift_vec(g, sx, sy, sz, sh0, sh1, sh2);
+            return pair_test(g, ai, aj, sx, sy, sz, sh0, sh1, sh2, rc2_lo, rc2_hi, false);
+        };
+        auto test = [&](int q) -> bool {
+            const float4 cq = rel[q];
+            const float ex = cq.x - fxi, ey = cq.y - fyi, ez = cq.z - fzi;
+            const float d2f = fmaf(ex, ex, fmaf(ey, ey, ez * ez));
+            if (d2f > hi_f) return false;
+            if (d2f < lo_f && d2f > margin) return true;
+            return exact(q);
+        };
+        // per-lane counts of the accepted candidates in w by species, packed 16 bits per species
+        auto species_counts = [&](unsigned w, unsigned long long& pc0, unsigned long long& pc1) {
+            pc0 = pc1 = 0ull;
 #pragma unroll
-                    for (int s = 0; s < NS; ++s) cnt_s[s] = s < S ? nl_cnt[(long long)wid * S + s] : 0;
-                } else if (tile_no > 0 && slot_base < kMaskSlots) {
-                    accw = *my_word;
-                }
-                double w0, w1, w2;
-                shift_vec(g, meta_w(ai.meta, 0), meta_w(ai.meta, 1), meta_w(ai.meta, 2), w0, w1, w2);
-                const double xi = ai.x - w0, yi = ai.y - w1, zi = ai.z - w2;   // the atom's image inside the box
-                // |d2 - d2_reference| <= ~2 rc sqrt(3) * (rounding of the coordinates involved): the band in which the
-                // shared-memory test may disagree with the reference's rounding sequence grows with the coordinates'
-                // magnitude (unwrapped trajectories far from the origin)
-                const double imag = fabs(ai.x) + fabs(ai.y) + fabs(ai.z) + fabs(w0) + fabs(w1) + fabs(w2);
-                // distance test of candidate q.  Float coordinates relative to the bin decide everything farther from the
-                // cutoff sphere than their rounding error: with coordinates of 1-norm <= m the float d2 is off by less
-                // than 2^-24 (7 m |d| + 5 d^2) <= 2^-19 (m^2 + rc^2) wherever a decision is taken -- the margin is 4x
-                // that.  Inside the margin (and for d2 ~ 0: the atom itself) the double-precision test decides, with the
-                // reference's exact rounding sequence only in its own, much narrower band.
-                const float fxi = (float)(xi - refx), fyi = (float)(yi - refy), fzi = (float)(zi - refz);
-                const float mx = fmaxf(maxabs, fabsf(fxi) + fabsf(fyi) + fabsf(fzi));
-                const float margin = 7.62939453125e-6f * (mx * mx + (float)rc2);   // 2^-17
-                const float lo_f = (float)rc2 - margin, hi_f = (float)rc2 + margin;
-                auto test = [&](int q) -> bool {
+            for (int s = 0; s < NS; ++s) {
+                const unsigned long long v = (unsigned long long)__popc(w & smask_s[s][lane]) << (16 * (s & 3));
+                if (s < 4) pc0 += v;
+                else pc1 += v;
+            }
+        };
+        // accept bits of an atom: one 64-bit word per lane, bit k = candidate (slot k, this lane); slots beyond the
+        // word (more than 2048 candidates) are tested again by the EMIT pass
+        const int nb_tile = (n + 31) >> 5;
+        const int nb_masked = max(0, min(nb_tile, 64 - slot_base));   // batches of this tile covered by the word
+        if (!emit) {
+            // the float test over the tile (a tile has at most 32 batches: one bit each), undecided candidates after it
+            unsigned w = 0u, undecided = 0u;
+            for (int b = 0; b < nb_tile; ++b) {
+                const int q = b * 32 + lane;
+                if (q < n) {
                     const float4 cq = rel[q];
                     const float ex = cq.x - fxi, ey = cq.y - fyi, ez = cq.z - fzi;
                     const float d2f = fmaf(ex, ex, fmaf(ey, ey, ez * ez));
-                    if (d2f > hi_f) return false;
-                    if (d2f < lo_f && d2f > margin) return true;
-                    const unsigned cd = code[q];
-                    const int p = pj[q];
-                    if (p == c && (cd & 0xffffffu) == 0u) return false;   // the atom itself (zero image shift)
-                    const AtomRec aj = atoms[p];
-                    const int sx = (int)(signed char)(cd & 0xff), sy = (int)(signed char)((cd >> 8) & 0xff),
-                              sz = (int)(signed char)((cd >> 16) & 0xff);
-                    double s0, s1, s2;
-                    shift_vec(g, sx - meta_w(aj.meta, 0), sy - meta_w(aj.meta, 1), sz - meta_w(aj.meta, 2), s0, s1, s2);
-                    const double dx = (aj.x + s0) - xi, dy = (aj.y + s1) - yi, dz = (aj.z + s2) - zi;
-                    const double d2 = dx * dx + dy * dy + dz * dz;
-                    const double band = 3.6e-15 * g.rc * ((double)cq.w + imag);   // 2^-48 rc (|x_j| + |x_i| + shifts)
-                    if (d2 < fast_lo - band) return true;
-                    if (d2 > fast_hi + band) return false;
-                    double sh0, sh1, sh2;
-                    shift_vec(g, sx, sy, sz, sh0, sh1, sh2);
-                    return pair_test(g, ai, aj, sx, sy, sz, sh0, sh1, sh2, rc2_lo, rc2_hi, false);
-                };
-                if (!FILL) {
-                    unsigned long long pc0 = 0ull, pc1 = 0ull;   // packed per-lane counters, 16 bits per species
-                    for (int b = 0; b < nb_tile; ++b) {
-                        const int q = b * 32 + lane;
-                        if (q < n && test(q)) {
-                            const int sp = (int)(code[q] >> 24);
-                            if (mark) mark[pj[q]] = 1;   // atoms whose environment the owner needs (halo)
-                            const unsigned long long one = 1ull << (16 * (sp & 3));
-                            if (NS <= 4 || sp < 4) pc0 += one;
-                            else pc1 += one;
-                            if (b < nb_masked) accw |= 1ull << (slot_base + b);
-                        }
-                    }
-                    if (nb_masked > 0) *my_word = accw;
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) {
-                        pc0 += __shfl_xor_sync(0xffffffffu, pc0, o);
-                        if (NS > 4) pc1 += __shfl_xor_sync(0xffffffffu, pc1, o);
-                    }
-                    if (lane == 0) {
-#pragma unroll
-                        for (int s = 0; s < NS; ++s)
-                            if (s < S) {
-                                const int v = (int)(((s < 4 ? pc0 : pc1) >> (16 * (s & 3))) & 0xffffull);
-                                int* dst = nl_cnt + (long long)wid * S + s;
-                                *dst = tile_no > 0 ? *dst + v : v;
-                            }
-                    }
-                } else {
-                    // pairs of one species are contiguous; inside a species: tile, then lane, then slot
-                    long long start[NS];
-                    {
-                        long long o = first_pair;
-#pragma unroll
-                        for (int s = 0; s < NS; ++s) {
-                            start[s] = o + ((tile_no > 0 && s < S) ? nl_run[(long long)wid * S + s] : 0);
-                            o += cnt_s[s];
-                        }
-                    }
-                    auto emit = [&](int q, unsigned long long& run0, unsigned long long& run1) {
-                        const unsigned cd = code[q];
-                        const int sp = (int)(cd >> 24);
-                        long long b = 0;
-#pragma unroll
-                        for (int s = 0; s < NS; ++s)
-                            if (sp == s) b = start[s];
-                        unsigned long long& run = (NS <= 4 || sp < 4) ? run0 : run1;
-                        const int r = (int)((run >> (16 * (sp & 3))) & 0xffffull);
-                        run += 1ull << (16 * (sp & 3));
-                        PairRec pr;
-                        pr.j = pj[q];
-                        pr.sb[0] = (signed char)(cd & 0xff);
-                        pr.sb[1] = (signed char)((cd >> 8) & 0xff);
-                        pr.sb[2] = (signed char)((cd >> 16) & 0xff);
-                        pr.sp = (unsigned char)sp;
-                        pairs[b + r] = pr;
-                    };
-                    // this lane's accepted candidates of the tile: stored bits, recomputed beyond the word's reach
-                    unsigned long long wt = nb_masked > 0 ? (accw >> slot_base) : 0ull;
-                    if (nb_masked < 64) wt &= (1ull << nb_masked) - 1ull;
-                    unsigned long long pc0 = 0ull, pc1 = 0ull;
-                    for (unsigned long long t = wt; t; t &= t - 1) {
-                        const int sp = (int)(code[(__ffsll((long long)t) - 1) * 32 + lane] >> 24);
-                        const unsigned long long one = 1ull << (16 * (sp & 3));
-                        if (NS <= 4 || sp < 4) pc0 += one;
-                        else pc1 += one;
-                    }
-                    for (int b = nb_masked; b < nb_tile; ++b) {   // rare: more than kMaskSlots batches
-                        const int q = b * 32 + lane;
-                        if (q < n && test(q)) {
-                            const int sp = (int)(code[q] >> 24);
-                            const unsigned long long one = 1ull << (16 * (sp & 3));
-                            if (NS <= 4 || sp < 4) pc0 += one;
-                            else pc1 += one;
-                        }
-                    }
-                    // exclusive prefix over lanes (16-bit fields cannot carry: totals < 65536)
-                    unsigned long long in0 = pc0, in1 = pc1;
-#pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) {
-                        const unsigned long long u0 = __shfl_up_sync(0xffffffffu, in0, o);
-                        const unsigned long long u1 = NS > 4 ? __shfl_up_sync(0xffffffffu, in1, o) : 0ull;
-                        if (lane >= o) {
-                            in0 += u0;
-                            in1 += u1;
-                        }
-                    }
-                    unsigned long long run0 = in0 - pc0, run1 = in1 - pc1;
-                    const unsigned long long tot0 = __shfl_sync(0xffffffffu, in0, 31);
-                    const unsigned long long tot1 = NS > 4 ? __shfl_sync(0xffffffffu, in1, 31) : 0ull;
-                    for (unsigned long long t = wt; t; t &= t - 1) emit((__ffsll((long long)t) - 1) * 32 + lane, run0, run1);
-                    for (int b = nb_masked; b < nb_tile; ++b) {
-                        const int q = b * 32 + lane;
-                        if (q < n && test(q)) emit(q, run0, run1);
-                    }
-                    if (!last_tile && lane == 0) {
-#pragma unroll
-                        for (int s = 0; s < NS; ++s)
-                            if (s < S) {
-                                const int prev = tile_no > 0 ? nl_run[(long long)wid * S + s] : 0;
-                                nl_run[(long long)wid * S + s] = prev + (int)(((s < 4 ? tot0 : tot1) >> (16 * (s & 3))) & 0xffffull);
-                            }
+                    if (d2f <= hi_f) {
+                        if (d2f < lo_f && d2f > margin) w |= 1u << b;
+                        else undecided |= 1u << b;
                     }
                 }
             }
-            slot_base += (n + 31) >> 5;
-            ++tile_no;
+            for (unsigned t = undecided; t; t &= t - 1) {
+                const int b = __ffs(t) - 1;
+                if (exact(b * 32 + lane)) w |= 1u << b;
+            }
+            if (mark)   // atoms whose environment the owner needs (halo)
+                for (unsigned t = w; t; t &= t - 1) mark[pj[(__ffs(t) - 1) * 32 + lane]] = 1;
+            if (nb_masked > 0) acc_s[a][lane] = (slot_base > 0 ? acc_s[a][lane] : 0ull) | ((unsigned long long)w << slot_base);
+            unsigned long long pc0, pc1;
+            species_counts(w, pc0, pc1);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                pc0 += __shfl_xor_sync(0xffffffffu, pc0, o);
+                if (NS > 4) pc1 += __shfl_xor_sync(0xffffffffu, pc1, o);
+            }
+            if (lane == 0) {
+#pragma unroll
+                for (int s = 0; s < NS; ++s) cnt_s[a][s] += (int)(((s < 4 ? pc0 : pc1) >> (16 * (s & 3))) & 0xffffull);
+            }
+            return;
         }
+        // pairs of one species are contiguous; inside a species: tile, then lane, then slot
+        long long start[NS];
+        {
+            long long o = row_s[a];
+#pragma unroll
+            for (int s = 0; s < NS; ++s) {
+                start[s] = o + done_s[a][s];
+                o += cnt_s[a][s];
+            }
+        }
+        auto emit_pair = [&](int q, unsigned long long& run0, unsigned long long& run1) {
+            const unsigned cd = code[q];
+            const int sp = (int)(cd >> 24);
+            long long b = 0;
+#pragma unroll
+            for (int s = 0; s < NS; ++s)
+                if (sp == s) b = start[s];
+            unsigned long long& run = (NS <= 4 || sp < 4) ? run0 : run1;
+            const int r = (int)((run >> (16 * (sp & 3))) & 0xffffull);
+            run += 1ull << (16 * (sp & 3));
+            PairRec pr;
+            pr.j = pj[q];
+            pr.sb[0] = (signed char)(cd & 0xff);
+            pr.sb[1] = (signed char)((cd >> 8) & 0xff);
+            pr.sb[2] = (signed char)((cd >> 16) & 0xff);
+            pr.sp = (unsigned char)sp;
+            pairs[b + r] = pr;
+        };
+        // this lane's accepted candidates of the tile: stored bits, tested again beyond the word's reach (rare)
+        unsigned w = nb_masked > 0 ? (unsigned)(acc_s[a][lane] >> slot_base) : 0u;
+        if (nb_tile < 32) w &= (1u << nb_tile) - 1u;   // drop the next tile's bits
+        for (int b = nb_masked; b < nb_tile; ++b) {
+            const int q = b * 32 + lane;
+            if (q < n && test(q)) w |= 1u << b;
+        }
+        unsigned long long pc0, pc1;
+        species_counts(w, pc0, pc1);
+        // exclusive prefix over lanes (16-bit fields cannot carry: totals < 65536)
+        unsigned long long in0 = pc0, in1 = pc1;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long u0 = __shfl_up_sync(0xffffffffu, in0, o);
+            const unsigned long long u1 = NS > 4 ? __shfl_up_sync(0xffffffffu, in1, o) : 0ull;
+            if (lane >= o) {
+                in0 += u0;
+                in1 += u1;
+            }
+        }
+        unsigned long long run0 = in0 - pc0, run1 = in1 - pc1;
+        const unsigned long long tot0 = __shfl_sync(0xffffffffu, in0, 31);
+        const unsigned long long tot1 = NS > 4 ? __shfl_sync(0xffffffffu, in1, 31) : 0ull;
+        for (unsigned t = w; t; t &= t - 1) emit_pair((__ffs(t) - 1) * 32 + lane, run0, run1);
+        if (lane == 0) {
+#pragma unroll
+            for (int s = 0; s < NS; ++s) done_s[a][s] += (int)(((s < 4 ? tot0 : tot1) >> (16 * (s & 3))) & 0xffffull);
+        }
+    };
+    // A bin whose stencil is one tile (the common case) stages it once; otherwise both passes stage every tile.
+    bool resident = false;
+    auto walk = [&](bool emit, int a0, int a1) {
+        int slot_base = 0;
+        for (int r0 = 0; r0 < nruns; r0 += kRunChunk) {
+            const int nr = min(kRunChunk, nruns - r0);
+            if (!resident) stage_runs(r0, nr);
+            const int total = run_pre[nr];
+            for (int t0 = 0; t0 < total; t0 += kBinCap) {
+                const int n = min(kBinCap, total - t0);
+                if (!resident) stage_tile(nr, t0, n);
+                for (int c = a0 + warp; c < a1; c += NW) visit(emit, c, c - a0, n, slot_base);
+                slot_base += (n + 31) >> 5;
+            }
+            resident = nruns <= kRunChunk && total <= kBinCap;
+        }
+    };
+    for (int a0 = lo; a0 < hi; a0 += kBinAtoms) {
+        const int a1 = min(hi, a0 + kBinAtoms);
+        if (a0 > lo) __syncthreads();   // the previous round still reads cnt_s / done_s
+        for (int t = threadIdx.x; t < kBinAtoms * NS; t += kBinThreads) {
+            cnt_s[t / NS][t % NS] = 0;
+            done_s[t / NS][t % NS] = 0;
+        }
+        __syncthreads();
+        walk(false, a0, a1);
+        __syncthreads();
+        // reserve the round's rows: one atomic per round, rows in cell order inside the segment
+        if (warp == 0) {
+            int tot = 0;
+            if (lane < a1 - a0)
+                for (int s = 0; s < S; ++s) tot += cnt_s[lane][s];
+            int inc = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int u = __shfl_up_sync(0xffffffffu, inc, o);
+                if (lane >= o) inc += u;
+            }
+            unsigned long long base = 0ull;
+            if (lane == 31) base = atomicAdd(reinterpret_cast<unsigned long long*>(cursor), (unsigned long long)inc);
+            base = __shfl_sync(0xffffffffu, base, 31);
+            const long long b0 = (long long)base + (inc - tot);
+            if (lane < a1 - a0) {
+                row_s[lane] = b0;
+                rows[a0 + lane - c_begin + env0] = make_longlong2(b0, b0 + tot);
+            }
+            if (lane == 31) fits_s = (long long)base + inc <= cap ? 1 : 0;   // else: count only (the sizing step re-runs)
+        }
+        __syncthreads();
+        if (fits_s) walk(true, a0, a1);
     }
 }
 
-template <bool FILL>
-static void launch_neighbor_bins(cudaStream_t st, int S, int c_begin, int c_end, int env0, const AtomRec* atoms,
-                                 const int* cstart, const Geom& g, int* nl_cnt, const long long* nl_first, PairRec* pairs,
-                                 unsigned char* mark, unsigned* masks, int* nl_run) {
-    const int nblk = g.ncell, T = kBinThreads;
+static void launch_neighbor_bins(sgpr_context* h, const Geom& g, int c_begin, int c_end, int env0, unsigned char* mark,
+                                 cudaStream_t st) {
+    const int nblk = g.ncell, T = kBinThreads, S = h->S;
+    const AtomRec* atoms = h->atoms.as<AtomRec>();
+    const int* cstart = h->cstart.as<int>();
+    long long* cursor = pair_cursor(h);
+    longlong2* rows = h->nl_rows.as<longlong2>();
+    PairRec* pairs = h->nl_pairs.as<PairRec>();
+    const long long cap = h->pairs_cap;
     if (S <= 1)
-        neighbor_bin_kernel<FILL, 1><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, nl_run);
+        neighbor_bin_kernel<1><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, cursor, cap, rows, pairs, mark);
     else if (S <= 2)
-        neighbor_bin_kernel<FILL, 2><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, nl_run);
+        neighbor_bin_kernel<2><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, cursor, cap, rows, pairs, mark);
     else if (S <= 4)
-        neighbor_bin_kernel<FILL, 4><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, nl_run);
+        neighbor_bin_kernel<4><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, cursor, cap, rows, pairs, mark);
     else
-        neighbor_bin_kernel<FILL, 8><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, nl_run);
+        neighbor_bin_kernel<8><<<nblk, T, 0, st>>>(c_begin, c_end, env0, atoms, cstart, g, S, cursor, cap, rows, pairs, mark);
+    h->stats.kernel_launches += 1;
 }
 
 // the block-per-bin kernels need enough bins to fill the machine; tiny systems keep one warp per environment
 static bool use_bin_kernels(const sgpr_context* h, const Geom& g) { return h->nl_mode == 2 || (g.ncell >= 64 && h->nl_mode != 1); }
 
+// one warp per environment, environments env0 .. env0+n_env-1 (FILL: nl_first = exclusive scan of their row lengths)
 template <bool FILL>
-static void launch_neighbor(int nblk, int T, cudaStream_t st, int S, int env0, int n_env, const int* active,
-                            const AtomRec* atoms, const int* abin, const int* cstart, const Geom& g, int* nl_cnt,
-                            const long long* nl_first, PairRec* pairs, unsigned char* mark, unsigned* masks,
-                            const BatchGeom* bg = nullptr) {
-    if (bg) {
-        if (S <= 1)
-            neighbor_kernel<FILL, 1, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
-        else if (S <= 2)
-            neighbor_kernel<FILL, 2, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
-        else if (S <= 4)
-            neighbor_kernel<FILL, 4, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
-        else
-            neighbor_kernel<FILL, 8, true><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks, *bg);
-        return;
-    }
-    if (S <= 1)
-        neighbor_kernel<FILL, 1><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks);
-    else if (S <= 2)
-        neighbor_kernel<FILL, 2><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks);
-    else if (S <= 4)
-        neighbor_kernel<FILL, 4><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks);
-    else
-        neighbor_kernel<FILL, 8><<<nblk, T, 0, st>>>(env0, n_env, active, atoms, abin, cstart, g, S, nl_cnt, nl_first, pairs, mark, masks);
-}
-
-__global__ void row_total_kernel(int n, int S, const int* __restrict__ nl_cnt, long long* __restrict__ tot) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i > n) return;
-    long long t = 0;
-    if (i < n)
-        for (int s = 0; s < S; ++s) t += nl_cnt[(long long)i * S + s];
-    tot[i] = t;
-}
-
-// contig_c0 >= 0: environments env0 .. env0+n_env-1 are the atoms contig_c0 .. of the cell order
-static int launch_count(sgpr_context* h, int env0, int n_env, const Geom& g, unsigned char* mark, cudaStream_t st,
-                        int contig_c0, const BatchGeom* bg = nullptr) {
-    if (n_env <= 0) return SGPR_OK;
-    if (contig_c0 >= 0 && !bg && use_bin_kernels(h, g)) {
-        launch_neighbor_bins<false>(st, h->S, contig_c0, contig_c0 + n_env, env0, h->atoms.as<AtomRec>(), h->cstart.as<int>(), g,
-                                    h->nl_cnt.as<int>(), nullptr, nullptr, mark, h->nl_masks.as<unsigned>(), nullptr);
-        h->stats.kernel_launches += 1;
-        return SGPR_OK;
-    }
-    const int T = 256;
+static void launch_neighbor(sgpr_context* h, cudaStream_t st, int env0, int n_env, const Geom& g, const long long* nl_first,
+                            unsigned char* mark, const BatchGeom* bg) {
+    const int T = 256, S = h->S;
     const int nblk = (int)(((int64_t)n_env * 32 + T - 1) / T);
-    launch_neighbor<false>(nblk, T, st, h->S, env0, n_env, h->active_all ? nullptr : h->active_list.as<int>(),
-                           h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->cstart.as<int>(), g, h->nl_cnt.as<int>(), nullptr,
-                           nullptr, mark, h->nl_masks.as<unsigned>(), bg);
+    const int* active = h->active_all ? nullptr : h->active_list.as<int>();
+    auto go = [&](auto kernel) {
+        kernel<<<nblk, T, 0, st>>>(env0, n_env, active, h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->cstart.as<int>(), g, S,
+                                   h->nl_cnt.as<int>(), nl_first, pair_cursor(h), h->pairs_cap, h->nl_rows.as<longlong2>(),
+                                   h->nl_pairs.as<PairRec>(), mark, h->nl_masks.as<unsigned>(), bg ? *bg : BatchGeom{});
+    };
+    if (bg) {
+        if (S <= 1) go(neighbor_kernel<FILL, 1, true>);
+        else if (S <= 2) go(neighbor_kernel<FILL, 2, true>);
+        else if (S <= 4) go(neighbor_kernel<FILL, 4, true>);
+        else go(neighbor_kernel<FILL, 8, true>);
+    } else {
+        if (S <= 1) go(neighbor_kernel<FILL, 1>);
+        else if (S <= 2) go(neighbor_kernel<FILL, 2>);
+        else if (S <= 4) go(neighbor_kernel<FILL, 4>);
+        else go(neighbor_kernel<FILL, 8>);
+    }
     h->stats.kernel_launches += 1;
-    return SGPR_OK;
+}
+
+// contig_c0 >= 0: environments env0 .. env0+n_env-1 are the atoms contig_c0 .. of the cell order -- the block-per-bin
+// kernel writes their rows and pairs in one pass.  Otherwise the warp kernel counts them and nl_finish fills their rows.
+static void launch_count(sgpr_context* h, int env0, int n_env, const Geom& g, unsigned char* mark, cudaStream_t st,
+                         int contig_c0, const BatchGeom* bg = nullptr) {
+    if (n_env <= 0) return;
+    if (contig_c0 >= 0 && !bg && use_bin_kernels(h, g))
+        launch_neighbor_bins(h, g, contig_c0, contig_c0 + n_env, env0, mark, st);
+    else
+        launch_neighbor<false>(h, st, env0, n_env, g, nullptr, mark, bg);
 }
 
 static int check_err_flags(const int* err) {
@@ -1255,45 +1305,25 @@ static int check_batch_err(const unsigned long long* berr) {
     return SGPR_OK;
 }
 
-// Sync-free steps: the pair count and the error flags stay on the device.  One thread records them in the status
-// block and decides whether the step is valid (the pair list fits the capacity sized by an earlier step, no error
-// flag); an invalid step gets EMPTY neighbour rows, so that every later kernel stays inside its buffers -- the step's
-// results are then meaningless and the sticky counter status[1] says so (sgpr_check / the host entry point re-run it).
-__global__ void nl_status_kernel(int na, const long long* __restrict__ first, long long cap, const int* __restrict__ err,
-                                 long long* __restrict__ status) {
-    const long long total = first[na];
-    const bool bad = total > cap || err[0] != 0;
-    status[0] = total;
-    status[6] = bad ? 1 : 0;
-    if (bad) {
-        status[1] += 1;
-        status[2] = err[0];
-        status[3] = err[1];
-        status[4] = total;
-        status[5] = cap;
-    }
-}
-__global__ void nl_clamp_kernel(int na, long long* __restrict__ first, const long long* __restrict__ status) {
-    if (status[6] == 0) return;
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i <= na) first[i] = 0;
+__global__ void row_total_kernel(int n, int S, const int* __restrict__ nl_cnt, long long* __restrict__ tot) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n) return;
+    long long t = 0;
+    if (i < n)
+        for (int s = 0; s < S; ++s) t += nl_cnt[(long long)i * S + s];
+    tot[i] = t;
 }
 
-// Lean form of row totals -> exclusive scan -> species row ranges -> (sync-free steps) status + clamp: one block walks the
-// rows in coalesced tiles of 1024 with a running carry.  (A few microseconds for 1e5 rows, and one graph node instead of
-// six: what matters for small systems and for the per-rank share of a sharded one.)
-constexpr int kRowsScanMax = 1 << 16;   // beyond: row_total + cub scan + status + clamp (one SM would be the bottleneck)
-__global__ void __launch_bounds__(1024) rows_scan_kernel(int na, int S, const int* __restrict__ nl_cnt,
-                                                         long long* __restrict__ first, const int* __restrict__ row_first_src,
-                                                         int row_first_pitch_ints, int* __restrict__ row_first_d, int do_status,
-                                                         long long cap, const int* __restrict__ err,
-                                                         long long* __restrict__ status) {
-    __shared__ int bad_s;
-    if ((int)threadIdx.x <= S) row_first_d[threadIdx.x] = row_first_src[(size_t)threadIdx.x * row_first_pitch_ints];
-    const long long total = block_scan_exclusive<long long>(
-        na + 1,
+// Lean form of row totals -> exclusive scan for the rows of the warp kernel: one block walks the rows in coalesced tiles
+// of 1024 with a running carry.  (A few microseconds for 1e5 rows, and one graph node instead of three: what matters for
+// small systems and for the halo rows of a sharded one.)
+constexpr int kRowsScanMax = 1 << 16;   // beyond: row_total + cub scan (one SM would be the bottleneck)
+__global__ void __launch_bounds__(1024) rows_scan_kernel(int n, int S, const int* __restrict__ nl_cnt,
+                                                         long long* __restrict__ first) {
+    block_scan_exclusive<long long>(
+        n + 1,
         [&](int i) -> long long {
-            if (i >= na) return 0;
+            if (i >= n) return 0;
             if (S == 4) {
                 const int4 c = *reinterpret_cast<const int4*>(nl_cnt + 4 * (long long)i);
                 return (long long)c.x + c.y + c.z + c.w;
@@ -1303,8 +1333,25 @@ __global__ void __launch_bounds__(1024) rows_scan_kernel(int na, int S, const in
             return t;
         },
         [&](int i, long long v) { first[i] = v; });
+}
+
+// Last node of the neighbour stage: the species row ranges go to their canonical device location (read by the GEMM set-up
+// kernel and row_energy_kernel) and, on sync-free steps, the pair total and the error flags to the status block.  The
+// total is the pair cursor (block-per-bin rows) plus the rows of the warp kernel.  A step is valid when the pair list fits
+// the capacity sized by an earlier step and no error flag is set; an invalid step gets EMPTY rows, so that every later
+// kernel stays inside its buffers -- its results are then meaningless and the sticky counter status[1] says so
+// (sgpr_check / the host entry point re-run it).
+__global__ void __launch_bounds__(1024) nl_finish_kernel(int na, int S, const int* __restrict__ row_first_src, int pitch_ints,
+                                                         int* __restrict__ row_first_d, int do_status,
+                                                         const long long* __restrict__ cursor,
+                                                         const long long* __restrict__ warp_total, long long cap,
+                                                         const int* __restrict__ err, long long* __restrict__ status,
+                                                         longlong2* __restrict__ rows) {
+    __shared__ int bad_s;
+    if ((int)threadIdx.x <= S) row_first_d[threadIdx.x] = row_first_src[(size_t)threadIdx.x * pitch_ints];
     if (!do_status) return;
     if (threadIdx.x == 0) {
+        const long long total = *cursor + (warp_total ? *warp_total : 0);
         const bool bad = total > cap || err[0] != 0;
         status[0] = total;
         status[6] = bad ? 1 : 0;
@@ -1319,46 +1366,48 @@ __global__ void __launch_bounds__(1024) rows_scan_kernel(int na, int S, const in
     }
     __syncthreads();
     if (bad_s)
-        for (int i = threadIdx.x; i <= na; i += 1024) first[i] = 0;
+        for (int i = threadIdx.x; i < na; i += blockDim.x) rows[i] = make_longlong2(0, 0);
 }
 
-// row totals -> exclusive scan -> (sizing step: sync for pair count, error flags, species row ranges) -> fill
+// Rows of the environments the block-per-bin kernel has not written (it writes the first n_contig, a contiguous range of
+// the cell order from contig_c0, when use_bin_kernels): per-environment counts of the warp kernel -> exclusive scan ->
+// fill behind the cursor.  A sizing step (warm = false) then synchronises for the pair total, the error flags and the
+// species row ranges; when the list does not fit it grows the capacity with head room (the following steps of a
+// trajectory reuse it without asking the device) and runs the block-per-bin kernel again, whose pairs did not fit.
 static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int* row_first_src, int row_first_pitch,
                      int64_t* n_pairs, int contig_c0, int n_contig, bool warm, const BatchGeom* bg = nullptr) {
     const int S = h->S;
     const int na = (int)h->n_active;
-    SGPR_TRY(h->nl_first.ensure(sizeof(long long) * 2 * ((size_t)na + 1)));
+    const int done = (n_contig > 0 && !bg && use_bin_kernels(h, g)) ? n_contig : 0;
+    const int nw = na - done;
+    SGPR_TRY(h->nl_first.ensure(sizeof(long long) * 2 * ((size_t)nw + 1)));
     SGPR_TRY(h->row_first_d.ensure(sizeof(int) * (SGPR_MAX_SPECIES + 2)));
     SGPR_TRY(h->status_d.ensure(sizeof(long long) * 8));
     long long* first = h->nl_first.as<long long>();
-    long long* tot = first + (na + 1);
+    long long* cursor = pair_cursor(h);
     const int T = 256;
-    const bool lean = h->nl_lean && na + 1 <= kRowsScanMax && row_first_pitch % (int)sizeof(int) == 0;
-    if (lean) {
-        rows_scan_kernel<<<1, 1024, 0, st>>>(na, S, h->nl_cnt.as<int>(), first, row_first_src,
-                                             row_first_pitch / (int)sizeof(int), h->row_first_d.as<int>(), warm ? 1 : 0,
-                                             h->pairs_cap, h->errflag.as<int>(), h->status_d.as<long long>());
-        h->stats.kernel_launches += 1;
-    } else {
-        row_total_kernel<<<(na + 1 + T - 1) / T, T, 0, st>>>(na, S, h->nl_cnt.as<int>(), tot);
-        SGPR_TRY(scan_exclusive_ll(h, tot, first, na + 1, st));
-        // species row ranges in their canonical device location (read by the GEMM set-up kernel and row_energy_kernel)
-        SGPR_CUDA(cudaMemcpy2DAsync(h->row_first_d.p, sizeof(int), row_first_src, (size_t)row_first_pitch, sizeof(int), S + 1,
-                                    cudaMemcpyDeviceToDevice, st));
+    if (nw > 0) {
+        const int* cnt = h->nl_cnt.as<int>() + (size_t)done * S;
+        if (h->nl_lean && nw + 1 <= kRowsScanMax) {
+            rows_scan_kernel<<<1, 1024, 0, st>>>(nw, S, cnt, first);
+            h->stats.kernel_launches += 1;
+        } else {
+            long long* tot = first + (nw + 1);
+            row_total_kernel<<<(nw + 1 + T - 1) / T, T, 0, st>>>(nw, S, cnt, tot);
+            SGPR_TRY(scan_exclusive_ll(h, tot, first, nw + 1, st));
+            h->stats.kernel_launches += 3;
+        }
     }
     long long total = 0;
     if (warm) {
         h->row_first_host_valid = false;
-        if (!lean) {
-            nl_status_kernel<<<1, 1, 0, st>>>(na, first, h->pairs_cap, h->errflag.as<int>(), h->status_d.as<long long>());
-            nl_clamp_kernel<<<(na + 1 + T - 1) / T, T, 0, st>>>(na, first, h->status_d.as<long long>());
-            h->stats.kernel_launches += 2;
-        }
     } else {
+        long long part[2] = {0, 0};   // block-per-bin pairs (cursor), warp-kernel pairs
         int err[4] = {0, 0, 0, 0};
         unsigned long long berr[2] = {0, 0};
         int rf[SGPR_MAX_SPECIES + 1];
-        SGPR_CUDA(cudaMemcpyAsync(&total, first + na, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        SGPR_CUDA(cudaMemcpyAsync(&part[0], cursor, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        if (nw > 0) SGPR_CUDA(cudaMemcpyAsync(&part[1], first + nw, sizeof(long long), cudaMemcpyDeviceToHost, st));
         SGPR_CUDA(cudaMemcpyAsync(err, h->errflag.p, sizeof(int) * 4, cudaMemcpyDeviceToHost, st));
         if (bg) SGPR_CUDA(cudaMemcpyAsync(berr, bg->err, sizeof(berr), cudaMemcpyDeviceToHost, st));
         SGPR_CUDA(cudaMemcpy2DAsync(rf, sizeof(int), row_first_src, (size_t)row_first_pitch, sizeof(int), S + 1,
@@ -1367,42 +1416,37 @@ static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int*
         SGPR_TRY(bg ? check_batch_err(berr) : check_err_flags(err));
         for (int s = 0; s <= S; ++s) h->row_first[s] = rf[s];
         h->row_first_host_valid = true;
-        // capacity with head room: the following steps of a trajectory reuse it without asking the device
+        total = part[0] + part[1];
         if (total + 1 > h->pairs_cap) {
             const long long want = total + total / 4 + 4096;
             SGPR_TRY(h->nl_pairs.ensure(sizeof(PairRec) * (size_t)want));
             h->pairs_cap = (long long)(h->nl_pairs.bytes / sizeof(PairRec)) - 1;
+            if (done > 0) {
+                SGPR_CUDA(cudaMemsetAsync(cursor, 0, sizeof(long long), st));
+                launch_neighbor_bins(h, g, contig_c0, contig_c0 + done, 0, nullptr, st);
+            }
         }
     }
-    int done = 0;   // environments 0 .. n_contig-1 are a contiguous range of the cell order: block-per-bin fill
-    if (n_contig > 0 && !bg && use_bin_kernels(h, g)) {
-        SGPR_TRY(h->nl_run.ensure(sizeof(int) * ((size_t)n_contig * S + 1)));
-        launch_neighbor_bins<true>(st, S, contig_c0, contig_c0 + n_contig, 0, h->atoms.as<AtomRec>(), h->cstart.as<int>(), g,
-                                   h->nl_cnt.as<int>(), first, h->nl_pairs.as<PairRec>(), nullptr,
-                                   h->nl_masks.as<unsigned>(), h->nl_run.as<int>());
-        done = n_contig;
-    }
-    if (na > done) {
-        const int nblk = (int)(((int64_t)(na - done) * 32 + T - 1) / T);
-        launch_neighbor<true>(nblk, T, st, S, done, na - done, h->active_all ? nullptr : h->active_list.as<int>(),
-                              h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->cstart.as<int>(), g, h->nl_cnt.as<int>(), first,
-                              h->nl_pairs.as<PairRec>(), nullptr, h->nl_masks.as<unsigned>(), bg);
-    }
-    h->stats.kernel_launches += lean ? 1 : 4;  // fill (+ row totals, cub scan (2) when not the one-kernel scan)
+    if (nw > 0) launch_neighbor<true>(h, st, done, nw, g, first, nullptr, bg);
+    nl_finish_kernel<<<1, 1024, 0, st>>>(na, S, row_first_src, row_first_pitch / (int)sizeof(int), h->row_first_d.as<int>(),
+                                         warm ? 1 : 0, cursor, nw > 0 ? first + nw : nullptr, h->pairs_cap,
+                                         h->errflag.as<int>(), h->status_d.as<long long>(), h->nl_rows.as<longlong2>());
+    h->stats.kernel_launches += 1;
     SGPR_CUDA(cudaGetLastError());
     *n_pairs = total;
     return SGPR_OK;
 }
 
-// Neighbour list of ALL atoms (single-GPU path): rows in cell order, descriptor rows from the
-// species-major scan of cell_sort.  Output: nl_cnt [N,S], nl_first [N+1] (int64), nl_pairs,
-// rows ordered by neighbour species, then bin traversal order, then cell order; h->row_first.
+// Neighbour list of ALL atoms (single-GPU path): rows in cell order, descriptor rows from the species-major scan of
+// cell_sort.  Output: nl_rows [N] (begin, end) into nl_pairs, each row ordered by neighbour species, then bin traversal
+// order, then cell order; h->row_first.
 int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, int64_t* n_pairs, bool warm) {
     h->active_all = true;
     h->n_active = N;
     SGPR_TRY(h->nl_cnt.ensure(sizeof(int) * ((size_t)N * h->S + 1)));
     SGPR_TRY(h->nl_masks.ensure(sizeof(unsigned) * kMaskSlots * ((size_t)N + 1)));
-    SGPR_TRY(launch_count(h, 0, (int)N, g, nullptr, st, 0));
+    SGPR_TRY(h->nl_rows.ensure(sizeof(longlong2) * ((size_t)N + 1)));
+    launch_count(h, 0, (int)N, g, nullptr, st, 0);
     const int nkeys = g.ncell * h->S;
     const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
     return nl_finish(h, g, st, rstartT, (int)sizeof(int) * g.ncell, n_pairs, 0, (int)N, warm);
@@ -1415,8 +1459,9 @@ int batch_neighbor_build(sgpr_context* h, int64_t N, const BatchGeom& bg, cudaSt
     h->n_active = N;
     SGPR_TRY(h->nl_cnt.ensure(sizeof(int) * ((size_t)N * h->S + 1)));
     SGPR_TRY(h->nl_masks.ensure(sizeof(unsigned) * kMaskSlots * ((size_t)N + 1)));
+    SGPR_TRY(h->nl_rows.ensure(sizeof(longlong2) * ((size_t)N + 1)));
     const Geom unused{};
-    SGPR_TRY(launch_count(h, 0, (int)N, unused, nullptr, st, -1, &bg));
+    launch_count(h, 0, (int)N, unused, nullptr, st, -1, &bg);
     const int nkeys = bg.ncell * h->S;
     const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
     return nl_finish(h, unused, st, rstartT, (int)sizeof(int) * bg.ncell, n_pairs, 0, 0, false, &bg);
@@ -1544,7 +1589,8 @@ int neighbor_build_sharded(sgpr_context* h, int64_t N, const Geom& g, int rank, 
     const int nblkN = (int)((N + 1 + T - 1) / T);
     shard_init_kernel<<<nblkN, T, 0, st>>>(N, c0, c1, owned, mark, active, rowof);
     h->n_active = n_own;
-    SGPR_TRY(launch_count(h, 0, n_own, g, with_halo ? mark : nullptr, st, c0));
+    SGPR_TRY(h->nl_rows.ensure(sizeof(longlong2) * ((size_t)N + 1)));
+    launch_count(h, 0, n_own, g, with_halo ? mark : nullptr, st, c0);
     int n_halo = 0;
     if (with_halo) {
         halo_flag_kernel<<<nblkN, T, 0, st>>>(N, owned, mark, flag);
@@ -1558,7 +1604,7 @@ int neighbor_build_sharded(sgpr_context* h, int64_t N, const Geom& g, int rank, 
     }
     const int na = n_own + n_halo;
     h->n_active = na;
-    SGPR_TRY(launch_count(h, n_own, n_halo, g, nullptr, st, -1));
+    launch_count(h, n_own, n_halo, g, nullptr, st, -1);
     // species-major rows over the active list
     SGPR_CUDA(cudaMemsetAsync(row_first_d, 0, sizeof(int) * (SGPR_MAX_SPECIES + 1), st));
     const int nblkA = (na + 1 + T - 1) / T;

@@ -169,7 +169,6 @@ struct sgpr_context {
     // ---- tcgen05 int8-sliced GEMM path (i8gemm.cu)
     bool nl_lean = true;        // SGPR_NL_LEAN=0: force the many-kernel cell sort / row scan that very large systems use -- test hook
     int nl_mode = 0;            // SGPR_NL: 0 auto, 1 "warp" (one warp per environment), 2 "bins" (one block per bin) -- test hook
-    sgpr::DevBuf nl_run;        // running per-species fill offsets across candidate tiles (block-per-bin fill)
     bool use_i8 = false;        // GEMMs on tcgen05 (int8 digit slices) instead of FP64 DMMA
     bool use_i8_now = false;    // ... for the current call (compat / K-matrix calls use the DMMA path)
     int i8_tr = 7;              // kernel matrix: truncation t + u <= i8_tr (7: 21 slice products, 8: 26)
@@ -235,10 +234,11 @@ struct sgpr_context {
     sgpr::DevBuf ind_perm_d;  // [M]
     sgpr::DevBuf ind_sp_d, ind_lone_d;  // [M] caller's order (lone-lone kernel term)
     sgpr::DevBuf sp_on;       // [S] species has usable inducing points and is enabled as a centre
-    sgpr::DevBuf errflag;     // [4] ints
+    sgpr::DevBuf errflag;     // [4] ints of error flags, then the pair cursor (long long); the cell sort zeroes both
     // ---- per-call workspaces (grow-only)
     sgpr::DevBuf cnt, cstart, rstart, keyrank, atoms, order, rowof, active_list, rowmap;
-    sgpr::DevBuf nl_cnt, nl_first, nl_pairs, nl_masks, scan_tmp;
+    sgpr::DevBuf nl_cnt, nl_first, nl_pairs, nl_masks, scan_tmp;   // nl_first: row offsets of the warp-kernel rows
+    sgpr::DevBuf nl_rows;     // [N] longlong2: (begin, end) of each environment's row in nl_pairs
     sgpr::DevBuf owned, shard_tmp, row_owned;    // atom sharding: owned/mark masks, scans, per-row ownership
     sgpr::DevBuf phat, cbuf, pnorm, sflag, gmat, gvec, epart, wpart, fcell, misc;
     sgpr::DevBuf stage_pos, stage_z, stage_out;  // device staging for the host API
@@ -287,6 +287,10 @@ struct sgpr_context {
 };
 
 namespace sgpr {
+
+// errflag: error flags of the cell sort, then the neighbour list's pair cursor (next free record of nl_pairs)
+constexpr size_t kErrflagBytes = sizeof(int) * 4 + sizeof(long long);
+inline long long* pair_cursor(sgpr_context* h) { return reinterpret_cast<long long*>(h->errflag.as<int>() + 4); }
 
 // ---- nl.cu ------------------------------------------------------------------------
 int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double* cell_h, const int32_t* pbc_h,
