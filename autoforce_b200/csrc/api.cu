@@ -393,7 +393,7 @@ __global__ void nl_count_orig_kernel(int64_t N, const AtomRec* __restrict__ atom
 }
 __global__ void nl_export_kernel(int64_t N, const AtomRec* __restrict__ atoms, const PairRec* __restrict__ pairs,
                                  const longlong2* __restrict__ nl_rows, const long long* __restrict__ first_out,
-                                 int32_t* __restrict__ j_out, int8_t* __restrict__ S_out) {
+                                 int32_t* __restrict__ j_out, int8_t* __restrict__ S_out, int* __restrict__ wide) {
     const int lane = threadIdx.x & 31;
     const int64_t c = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     if (c >= N) return;
@@ -404,8 +404,12 @@ __global__ void nl_export_kernel(int64_t N, const AtomRec* __restrict__ atoms, c
         const PairRec pr = pairs[k];
         const AtomRec aj = atoms[pr.j];
         j_out[o + (k - beg)] = meta_orig(aj.meta);
-        for (int q = 0; q < 3; ++q)
-            S_out[3 * (o + (k - beg)) + q] = (int8_t)(pr.sb[q] - meta_w(aj.meta, q) + meta_w(ai.meta, q));
+        for (int q = 0; q < 3; ++q) {
+            // the shift relative to the given positions spans up to 2 x 120 cells; int8 holds it only near the cell
+            const int s = pr.sb[q] - meta_w(aj.meta, q) + meta_w(ai.meta, q);
+            if (s < -128 || s > 127) *wide = 1;
+            S_out[3 * (o + (k - beg)) + q] = (int8_t)s;
+        }
     }
 }
 
@@ -1863,18 +1867,27 @@ extern "C" __attribute__((visibility("default"))) int sgpr_neighbors(sgpr_handle
     SGPR_TRY(neighbor_build(h, N, g, st, &n_pairs));
     *nnz_h = n_pairs;
     // counts in caller order -> exclusive scan -> export
-    SGPR_TRY(h->misc.ensure(sizeof(long long) * ((size_t)N + 2)));
+    SGPR_TRY(h->misc.ensure(sizeof(long long) * ((size_t)N + 3)));
     long long* cnt = h->misc.as<long long>();
+    int* wide = reinterpret_cast<int*>(cnt + N + 2);   // set when a shift does not fit in int8
+    SGPR_CUDA(cudaMemsetAsync(wide, 0, sizeof(int), st));
     nl_count_orig_kernel<<<(int)((N + 1 + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(),
                                                                      h->nl_rows.as<longlong2>(), cnt);
     SGPR_TRY(scan_exclusive_ll(h, cnt, (long long*)first_d, (int)N + 1, st));
     if (n_pairs <= capacity && N > 0 && j_d && S_d) {
         nl_export_kernel<<<(int)((N * 32 + 255) / 256), 256, 0, st>>>(N, h->atoms.as<AtomRec>(), h->nl_pairs.as<PairRec>(),
                                                                       h->nl_rows.as<longlong2>(), (const long long*)first_d,
-                                                                      j_d, S_d);
+                                                                      j_d, S_d, wide);
     }
     SGPR_CUDA(cudaGetLastError());
+    int wide_h = 0;
+    SGPR_CUDA(cudaMemcpyAsync(&wide_h, wide, sizeof(int), cudaMemcpyDeviceToHost, st));
     SGPR_CUDA(cudaStreamSynchronize(st));
+    if (wide_h) {
+        set_error("an image shift between two neighbours exceeds the int8 range of the exported list (atoms more than "
+                  "~127 cells apart); wrap positions first");
+        return SGPR_ERR_GEOMETRY;
+    }
     return SGPR_OK;
 }
 

@@ -250,7 +250,9 @@ int sgpr_kernel_jacobian_batch(sgpr_handle h, int32_t B, const int64_t* first_h,
  * CSR over atoms in the caller's order, offsets relative to the given positions.
  *   first_d [N+1] int64;  j_d [capacity] int32;  S_d [capacity,3] int8
  *   *nnz_h receives the number of pairs; if it exceeds `capacity` nothing is written to
- *   j_d/S_d and the call still returns SGPR_OK (call again with a larger buffer). */
+ *   j_d/S_d and the call still returns SGPR_OK (call again with a larger buffer).
+ *   An offset outside the int8 range (the two atoms of a pair stored ~128 or more cells
+ *   apart, e.g. +70 and -70 cells out) is SGPR_ERR_GEOMETRY: wrap positions first. */
 int sgpr_neighbors(sgpr_handle h, int64_t N, const double* pos_d, const int32_t* Z_d,
                    const double* cell_h, const int32_t* pbc_h, void* stream,
                    int64_t* first_d, int32_t* j_d, int8_t* S_d, int64_t capacity, int64_t* nnz_h);

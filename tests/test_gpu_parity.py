@@ -36,20 +36,44 @@ def stress_of(W, cell):
     return (W / vol).reshape(-1)[[0, 4, 8, 5, 2, 1]]
 
 
-@pytest.fixture(params=golden_cases())
-def case(request):
+def golden_engine(name):
     import autoforce_b200 as ab
 
-    g = load_golden(request.param)
+    g = load_golden(name)
     if g["meta"]["kernel"]["kind"] == "multi":
         pytest.skip("kernel sums run through one handle per kernel: test_kernel_sum_with_different_hyperparameters")
-    eng = ab.SgprEngine(model_from_golden(g), species=g["meta"]["species"])
+    return g, ab.SgprEngine(model_from_golden(g), species=g["meta"]["species"])
+
+
+@pytest.fixture(params=golden_cases())
+def case(request):
+    g, eng = golden_engine(request.param)
     yield g, eng
     eng.close()
 
 
-def test_neighbor_list_bit_exact(case):
-    g, eng = case
+# The golden cells have 1-9 bins (cluster_lone: 1,700), so the automatic choice runs them through the warp-per-atom
+# neighbour kernel; "<name>-bins" runs the same case through the block-per-bin kernel (SGPR_NL is read when the handle
+# is created).  Tests that depend on the neighbour list take this fixture instead of `case`.
+@pytest.fixture(params=golden_cases() + [n + "-bins" for n in golden_cases()])
+def nl_case(request, monkeypatch):
+    name, _, mode = request.param.partition("-")
+    if mode:
+        monkeypatch.setenv("SGPR_NL", mode)
+    g, eng = golden_engine(name)
+    yield g, eng
+    eng.close()
+
+
+def assert_golden_efs(g, E, F, W):
+    N = len(g["numbers"])
+    assert abs(E - float(g["energy"])) / N < TOL_E_PER_ATOM
+    assert np.abs(F - g["forces"]).max() < TOL_F
+    assert np.abs(stress_of(W, g["cell"]) - g["stress"]).max() < TOL_S
+
+
+def test_neighbor_list_bit_exact(nl_case):
+    g, eng = nl_case
     first, J, S = eng.neighbors(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
     assert len(J) == len(g["nl_j"])
     a, b = sorted_rows(first, J, S), sorted_rows(g["nl_first"], g["nl_j"], g["nl_S"])
@@ -84,8 +108,8 @@ def test_kernel_matrix(case):
     assert np.abs(K - g["K"]).max() < 1e-12
 
 
-def test_energy_forces_stress(case):
-    g, eng = case
+def test_energy_forces_stress(nl_case):
+    g, eng = nl_case
     N = len(g["numbers"])
     E, F, W, owned = eng.predict(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
     assert owned.all()
@@ -160,11 +184,11 @@ def test_empty_structure():
 
 
 @pytest.mark.parametrize("world", [2, 3, 8])
-def test_atom_sharding_sums_to_single_rank_result(case, world):
+def test_atom_sharding_sums_to_single_rank_result(nl_case, world):
     """SURVEY 8e: every rank evaluates its owned environments + the one-cutoff halo and
     returns E/W partial sums and the forces of its owned atoms; summing the ranks (what
     the 10-double all-reduce does for E and W) must reproduce the unsharded result."""
-    g, eng = case
+    g, eng = nl_case
     args = (g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
     E0, F0, W0, own0 = eng.predict(*args)
     E, F, W = 0.0, np.zeros_like(F0), np.zeros_like(W0)
@@ -179,12 +203,13 @@ def test_atom_sharding_sums_to_single_rank_result(case, world):
     assert abs(E - E0) / N < 1e-12
     assert np.abs(F - F0).max() < 1e-11
     assert np.abs(W - W0).max() < 1e-10
+    assert_golden_efs(g, E, F, W)                   # both sides run the same neighbour kernel: check the list itself
 
 
-def test_covloss_matches_reference(case):
+def test_covloss_matches_reference(nl_case):
     """beta = get_covloss() (calculator/active.py:781-804), incl. sqrt(vscale), inf for species
     without variance scale and NaN for centres excluded via a/a_not."""
-    g, eng = case
+    g, eng = nl_case
     E, F, W, owned, beta = eng.predict(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"], want_beta=True)
     ref = g["covloss"]
     fin = np.isfinite(ref)
@@ -416,6 +441,24 @@ def test_neighbor_list_far_from_the_origin(mode, monkeypatch):
     with pytest.raises(RuntimeError, match="120 cells"):
         eng.neighbors(pos + 400.0 * cell[1], g["numbers"], cell, True)
     eng.close()
+    # opposite wraps: half the atoms 70 cells out, half -70, so neighbours are ~140 cells apart.  Prediction (int shifts)
+    # must equal the oracle's on the same atoms at home (the oracle's image search over +-140 cells would take hours);
+    # the exported list cannot hold such a shift in int8 and must refuse instead of wrapping it.
+    g = load_golden("lipso108")
+    pos = np.array(g["pos"], dtype=float)
+    out = 70.0 * g["cell"].sum(axis=0)
+    pos[0::2] += out
+    pos[1::2] -= out
+    eng = ab.SgprEngine(model_from_golden(g), species=g["meta"]["species"])
+    E, F, W, _ = eng.predict(pos, g["numbers"], g["cell"], g["meta"]["pbc"])
+    ref = o.predict(oracle_model(g), g["pos"], g["cell"], g["meta"]["pbc"], g["numbers"])
+    N = len(g["numbers"])
+    assert abs(E - ref["energy"]) / N < TOL_E_PER_ATOM
+    assert np.abs(F - ref["forces"]).max() < TOL_F
+    assert np.abs(W - ref["virial"]).max() < 1e-8
+    with pytest.raises(RuntimeError, match="int8 range"):
+        eng.neighbors(pos, g["numbers"], g["cell"], g["meta"]["pbc"])
+    eng.close()
 
 
 @pytest.mark.parametrize("name", ["lipso108", "tric_oh"])
@@ -601,7 +644,7 @@ def test_fixed_central_species_kernel():
 
 
 @pytest.mark.parametrize("world", [2, 3, 8])
-def test_peer_memory_exchange_emulated_on_one_gpu(case, world):
+def test_peer_memory_exchange_emulated_on_one_gpu(nl_case, world):
     """The force exchange bench.py --gpus N uses (sgpr_predict_p2p + sgpr_p2p_collect): every emulated rank evaluates
     only the environments it owns and adds neighbour forces into the OWNER's accumulation buffer.  Here the peer table
     points at ``world`` local buffers of one GPU (one handle per emulated rank); the assembled result must equal the
@@ -610,7 +653,7 @@ def test_peer_memory_exchange_emulated_on_one_gpu(case, world):
 
     import autoforce_b200 as ab
 
-    g, eng0 = case
+    g, eng0 = nl_case
     N = len(g["numbers"])
     E0, F0, W0, _ = eng0.predict(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
     dev = torch.device("cuda", 0)
@@ -638,6 +681,7 @@ def test_peer_memory_exchange_emulated_on_one_gpu(case, world):
         assert abs(ew[0] - E0) / N < 1e-12
         assert np.abs(F.cpu().numpy() - F0).max() < 1e-10
         assert np.abs(ew[1:].reshape(3, 3) - W0).max() < 1e-9
+        assert_golden_efs(g, ew[0], F.cpu().numpy(), ew[1:].reshape(3, 3))
     finally:
         for e in engines:
             e.close()
@@ -716,22 +760,28 @@ def test_sync_free_steps_and_overflow_recovery():
     ref_eng.close()
 
 
-@pytest.mark.parametrize("world", [2, 4])
-def test_fused_exchange_step_emulated_on_one_gpu(world):
+@pytest.mark.parametrize("world,mode", [(2, None), (4, None), (2, "bins"), (4, "bins")], ids=["2", "4", "2-bins", "4-bins"])
+def test_fused_exchange_step_emulated_on_one_gpu(world, mode, monkeypatch):
     """sgpr_p2p_step (no NCCL: mailboxes + stamped flags) with ``world`` ranks emulated on ONE GPU: one handle and one
     stream per rank, the ranks' symmetric blocks are plain device buffers.  Several steps (sizing, warm, CUDA-graph
-    replay, both buffer parities, moving atoms) must reproduce the unsharded result on every rank."""
+    replay, both buffer parities, moving atoms) must reproduce the unsharded result on every rank, and the oracle's.
+    The cell has 27 bins, so the ranks run the warp-per-atom neighbour kernel unless "bins" forces the block-per-bin one
+    (the unsharded reference then keeps the warp kernel)."""
     import torch
 
     import autoforce_b200 as ab
     from autoforce_b200 import synth
+    from oracle_engine import to_oracle
 
     Zs = [3, 8]
     model = synth.synth_model(Zs, 40, 5, lmax=3, nmax=3, rc=6.0)
+    om = to_oracle(model)
     pos0, cell, numbers = synth.fcc(6, Zs, 0.1, 1)
     N = len(numbers)
     dev = torch.device("cuda", 0)
     ref = ab.SgprEngine(model, species=Zs)
+    if mode:
+        monkeypatch.setenv("SGPR_NL", mode)
     engines = [ab.SgprEngine(model, species=Zs) for _ in range(world)]
     streams = [torch.cuda.Stream(device=dev) for _ in range(world)]
     stride = 3 * N + 8
@@ -768,6 +818,10 @@ def test_fused_exchange_step_emulated_on_one_gpu(world):
                 covered += owns[r].to(torch.int32)
             assert bool((covered == 1).all())
             assert np.abs(F.cpu().numpy() - F0).max() < 1e-10, step
+            out = o.predict(om, pos, cell, True, numbers)
+            assert abs(ew[0] - out["energy"]) / N < TOL_E_PER_ATOM, step
+            assert np.abs(F.cpu().numpy() - out["forces"]).max() < TOL_F, step
+            assert np.abs(ew[1:].reshape(3, 3) - out["virial"]).max() < 1e-8, step
     finally:
         for e in engines + [ref]:
             e.close()
