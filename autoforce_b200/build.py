@@ -12,7 +12,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIBPATH = os.path.join(LIBDIR, "libsgpr_b200.so")
 SOURCES = ["api.cu", "nl.cu", "descriptor.cu", "gemm.cu", "i8gemm.cu", "md.cu", "relax.cu"]
-HEADERS = ["sgpr_internal.cuh", "sgpr_math.cuh", "gemm_kernel.cuh", "i8gemm_kernel.cuh", "i8gemm2_kernel.cuh", os.path.join("..", "..", "include", "sgpr_b200.h")]
+HEADERS = ["sgpr_internal.cuh", "sgpr_math.cuh", "gemm_kernel.cuh", "i8gemm_kernel.cuh", os.path.join("..", "..", "include", "sgpr_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

@@ -795,14 +795,8 @@ extern "C" __attribute__((visibility("default"))) int sgpr_create(const sgpr_mod
         const char* trs = getenv("SGPR_I8_TR");
         h->use_i8 = dp.normalize && !(eng && strcmp(eng, "dmma") == 0);
         h->i8_tr = (trs && atoi(trs) == 8) ? 8 : 7;
-        const char* tr2 = getenv("SGPR_I8_TR2");   // back projection (forces only): like the kernel matrix, or 6 / 7 / 8
-        h->i8_tr2 = tr2 ? (atoi(tr2) == 8 ? 8 : atoi(tr2) == 6 ? 6 : 7) : h->i8_tr;
-        const char* c2 = getenv("SGPR_I8_CTA2");
-        h->i8_cta2 = c2 && atoi(c2) == 1;
-        const char* epw = getenv("SGPR_I8_EPW");
-        h->i8_epw = epw ? atoi(epw) : 0;
-        const char* nss = getenv("SGPR_I8_NS");
-        h->i8_ns = (nss && atoi(nss) == 5) ? 5 : 6;
+        const char* tr2 = getenv("SGPR_I8_TR2");   // back projection (forces only): like the kernel matrix, or 7 / 8
+        h->i8_tr2 = tr2 ? (atoi(tr2) == 8 ? 8 : 7) : h->i8_tr;
         if (h->use_i8) {
             st = i8_prepare_model(h, false);
             if (st == SGPR_OK) st = i8_prepare_covloss(h);
@@ -830,7 +824,7 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->nl_first, &h->nl_pairs, &h->scan_tmp, &h->phat, &h->cbuf, &h->pnorm, &h->sflag, &h->gmat,
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
-                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_rows, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local, &h->i8_probs2,
+                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_rows, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local,
                       &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr,
                       &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part,
                       &h->rx_pos, &h->rx_vel, &h->rx_F, &h->rx_beta, &h->rx_ew, &h->rx_part};
@@ -838,7 +832,6 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
     if (h->pinned) cudaFreeHost(h->pinned);
     if (h->i8_probs_pinned) cudaFreeHost(h->i8_probs_pinned);
     if (h->status_pinned) cudaFreeHost(h->status_pinned);
-    if (h->i8_probs2_pinned) cudaFreeHost(h->i8_probs2_pinned);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     for (int i = 0; i < 6; ++i)
         if (h->ev[i]) cudaEventDestroy(h->ev[i]);

@@ -12,7 +12,6 @@
 // descriptors are normalised (|k| <= 1 by Cauchy-Schwarz); un-normalised models use the DMMA path.
 #include <math.h>
 
-#include "i8gemm2_kernel.cuh"
 #include "i8gemm_kernel.cuh"
 #include "sgpr_internal.cuh"
 
@@ -252,11 +251,11 @@ struct Epi2 {   // back projection: g = mumax * C
     }
 };
 
-template <int NS, int TR, class Epi, int EPW = 2>
-int launch_ns(sgpr_context* h, const Common* cm_d, const Problem* probs_d, const Epi& epi, cudaStream_t st) {
+template <int TR, int EPW = 2, class Epi>
+int launch(sgpr_context* h, const Common* cm_d, const Problem* probs_d, const Epi& epi, cudaStream_t st) {
     constexpr int STAGES = 3;
-    auto kern = i8gemm_kernel<NS, TR, STAGES, Epi, 0, EPW>;
-    const size_t smem = smem_bytes<NS, STAGES>();
+    auto kern = i8gemm_kernel<kNS, TR, STAGES, Epi, 0, EPW>;
+    const size_t smem = smem_bytes<kNS, STAGES>();
     static bool done = false;   // per instantiation
     if (!done) {
         SGPR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -264,28 +263,6 @@ int launch_ns(sgpr_context* h, const Common* cm_d, const Problem* probs_d, const
     }
     // persistent: one CTA per SM; the tile count lives on the device (CTAs beyond it exit at once)
     kern<<<h->sm_count, 64 + 128 * EPW, smem, st>>>(cm_d, probs_d, epi);
-    SGPR_CUDA(cudaGetLastError());
-    h->stats.kernel_launches += 1;
-    return SGPR_OK;
-}
-
-template <int TR, class Epi>
-int launch(sgpr_context* h, const Common* cm_d, const Problem* probs_d, const Epi& epi, cudaStream_t st) {
-    return launch_ns<kNS, TR, Epi>(h, cm_d, probs_d, epi, st);
-}
-
-// CTA-pair variant (i8gemm2_kernel.cuh): static cluster dims (2,1,1), one pair per TPC
-template <int NS, int TR, class Epi>
-int launch2(sgpr_context* h, const Common* cm_d, const Problem2* probs_d, const Epi& epi, cudaStream_t st) {
-    constexpr int STAGES = 3;
-    auto kern = i8gemm2_kernel<NS, TR, STAGES, Epi>;
-    const size_t smem = smem_bytes2<NS, STAGES>();
-    static bool done = false;
-    if (!done) {
-        SGPR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        done = true;
-    }
-    kern<<<h->sm_count & ~1, NTHREADS, smem, st>>>(cm_d, probs_d, epi);
     SGPR_CUDA(cudaGetLastError());
     h->stats.kernel_launches += 1;
     return SGPR_OK;
@@ -442,16 +419,13 @@ static int build_problems(sgpr_context* h, int which, std::vector<Problem>& prob
             P.aux = h->mu.as<double>() + m0;
             P.N = m1 - m0;
             P.Kpad = h->i8_kp1;
-            const int ns1 = (h->i8_ns == 5 && h->i8_tr == 7) ? 5 : kNS;
-            SGPR_TRY(make_map(&P.mapA, h->p8.as<signed char>(), ns1, cap, P.Kpad, cap, BM));
-            SGPR_TRY(make_map(&P.mapB, h->z8.as<signed char>() + (size_t)m0 * 64, ns1, P.N, P.Kpad, (long long)h->M, BN));
+            SGPR_TRY(make_map(&P.mapA, h->p8.as<signed char>(), kNS, cap, P.Kpad, cap, BM));
+            SGPR_TRY(make_map(&P.mapB, h->z8.as<signed char>() + (size_t)m0 * 64, kNS, P.N, P.Kpad, (long long)h->M, BN));
         } else if (which == 2) {
             P.N = dp.D;
             P.Kpad = ((m1 - m0) + 63) / 64 * 64;
-            // t + u <= 6 uses the 5 most significant digit slices of both operands (same buffers, same slice stride)
-            const int ns2 = (h->i8_tr2 == 6 || (h->i8_ns == 5 && h->i8_tr2 == 7)) ? 5 : kNS;
-            SGPR_TRY(make_map(&P.mapA, h->g8.as<signed char>(), ns2, cap, h->i8_mp, cap, BM));
-            SGPR_TRY(make_map(&P.mapB, h->zt8.as<signed char>() + (size_t)s * kNS * dp.D * h->i8_mp, ns2, dp.D, h->i8_mp, (long long)dp.D, BN));
+            SGPR_TRY(make_map(&P.mapA, h->g8.as<signed char>(), kNS, cap, h->i8_mp, cap, BM));
+            SGPR_TRY(make_map(&P.mapB, h->zt8.as<signed char>() + (size_t)s * kNS * dp.D * h->i8_mp, kNS, dp.D, h->i8_mp, (long long)dp.D, BN));
         } else {
             P.aux = h->crs.as<double>() + (size_t)s * h->M;
             P.N = h->M;
@@ -485,7 +459,7 @@ static void count_work(sgpr_context* h, int which) {
             h->stats.covloss_flops += 2.0 * M * (double)h->M * (m1 - m0);
         } else {
             const int tr = which == 2 ? h->i8_tr2 : h->i8_tr;
-            const int npairs = tr == 8 ? 26 : tr == 6 ? 15 : (h->i8_ns == 5 ? 19 : 21);
+            const int npairs = tr == 8 ? 26 : 21;
             const double N = which == 1 ? (m1 - m0) : dp.D;
             const double Kpad = which == 1 ? h->i8_kp1 : ((m1 - m0) + 63) / 64 * 64;
             h->stats.gemm_flops += 2.0 * M * N * (which == 1 ? dp.D : (m1 - m0));
@@ -506,7 +480,7 @@ static int device_problems(sgpr_context* h, int which, cudaStream_t st, const Pr
     mix((unsigned long long)(uintptr_t)h->z8.p); mix((unsigned long long)(uintptr_t)h->zt8.p); mix((unsigned long long)(uintptr_t)h->c8.p);
     mix((unsigned long long)(uintptr_t)h->cov_nk.p); mix((unsigned long long)(uintptr_t)h->i8_probs.p);
     mix((unsigned long long)(uintptr_t)h->mu.p); mix((unsigned long long)(uintptr_t)h->crs.p);
-    mix(h->i8_cap_rows); mix(h->M); mix(h->i8_kp1); mix(h->i8_mp); mix(h->i8_tr2); mix(h->i8_ns); mix(h->i8_model_version);
+    mix(h->i8_cap_rows); mix(h->M); mix(h->i8_kp1); mix(h->i8_mp); mix(h->i8_model_version);
     for (int s = 0; s <= h->S; ++s) mix(h->m_first[s]);
     Problem* dev = h->i8_probs.as<Problem>() + slot * kMaxSpecies;
     if (h->i8_prob_sig[slot] != sig) {
@@ -523,47 +497,6 @@ static int device_problems(sgpr_context* h, int which, cudaStream_t st, const Pr
     }
     *out = dev;
     *sd_out = h->i8_setup[slot];
-    return SGPR_OK;
-}
-
-// Problem2 descriptors (CTA-pair kernel) of GEMM 1 / 2, same caching rule as device_problems
-static int device_problems2(sgpr_context* h, int which, cudaStream_t st, const Problem2** out) {
-    const DescParams& dp = h->dp;
-    SGPR_TRY(h->i8_probs2.ensure(sizeof(Problem2) * 2 * kMaxSpecies));
-    if (!h->i8_probs2_pinned) SGPR_CUDA(cudaMallocHost(&h->i8_probs2_pinned, sizeof(Problem2) * 2 * kMaxSpecies));
-    const int slot = which - 1;
-    Problem2* dev = h->i8_probs2.as<Problem2>() + slot * kMaxSpecies;
-    const unsigned long long sig = h->i8_prob_sig[slot] ^ (unsigned long long)(uintptr_t)h->i8_probs2.p;
-    if (h->i8_prob2_sig[slot] != sig || sig == 0) {
-        const long long cap = (long long)h->i8_cap_rows;
-        std::vector<Problem2> probs;
-        for (int s = 0; s < h->S; ++s) {
-            const int m0 = h->m_first[s], m1 = h->m_first[s + 1];
-            if (m1 == m0 || !dp.central_enabled[s]) continue;
-            Problem2 P;
-            P.aux = which == 1 ? h->mu.as<double>() + m0 : nullptr;
-            if (which == 1) {
-                const int ns1 = (h->i8_ns == 5 && h->i8_tr == 7) ? 5 : kNS;
-                P.N = m1 - m0;
-                P.Kpad = h->i8_kp1;
-                SGPR_TRY(make_map(&P.mapA, h->p8.as<signed char>(), ns1, cap, P.Kpad, cap, BM));
-                SGPR_TRY(make_map(&P.mapBh, h->z8.as<signed char>() + (size_t)m0 * 64, ns1, P.N, P.Kpad, (long long)h->M, BNH));
-            } else {
-                const int ns2 = (h->i8_tr2 == 6 || (h->i8_ns == 5 && h->i8_tr2 == 7)) ? 5 : kNS;
-                P.N = dp.D;
-                P.Kpad = ((m1 - m0) + 63) / 64 * 64;
-                SGPR_TRY(make_map(&P.mapA, h->g8.as<signed char>(), ns2, cap, h->i8_mp, cap, BM));
-                SGPR_TRY(make_map(&P.mapBh, h->zt8.as<signed char>() + (size_t)s * kNS * dp.D * h->i8_mp, ns2, dp.D, h->i8_mp, (long long)dp.D, BNH));
-            }
-            probs.push_back(P);
-        }
-        Problem2* pin = (Problem2*)h->i8_probs2_pinned + slot * kMaxSpecies;
-        SGPR_CUDA(cudaStreamSynchronize(st));
-        for (size_t i = 0; i < probs.size(); ++i) pin[i] = probs[i];
-        if (!probs.empty()) SGPR_CUDA(cudaMemcpyAsync(dev, pin, sizeof(Problem2) * probs.size(), cudaMemcpyHostToDevice, st));
-        h->i8_prob2_sig[slot] = sig;
-    }
-    *out = dev;
     return SGPR_OK;
 }
 
@@ -599,15 +532,9 @@ static int kernel_matrix_impl(sgpr_context* h, cudaStream_t st, bool store_k8, c
     e.cap_rows = (long long)h->i8_cap_rows;
     e.xi = h->xi;
     e.xi_int = h->xi_int;
-    if (h->i8_cta2 && h->i8_tr == 7) {
-        const Problem2* p2 = nullptr;
-        SGPR_TRY(device_problems2(h, 1, st, &p2));
-        return h->i8_ns == 5 ? launch2<5, 7>(h, common_d(h, 1), p2, e, st) : launch2<6, 7>(h, common_d(h, 1), p2, e, st);
-    }
-    if (h->i8_tr == 7 && h->i8_ns == 5) return launch_ns<5, 7>(h, common_d(h, 1), probs_d, e, st);
     // descriptors of one K chunk (a single species with the default lmax/nmax): the main loop is one stage per tile and
     // the fused epilogue is the kernel -- twice the epilogue warps
-    if (h->i8_tr == 7 && h->i8_kp1 <= 64 && h->i8_epw != 2) return launch_ns<kNS, 7, Epi1, 4>(h, common_d(h, 1), probs_d, e, st);
+    if (h->i8_tr == 7 && h->i8_kp1 <= 64) return launch<7, 4>(h, common_d(h, 1), probs_d, e, st);
     return h->i8_tr == 8 ? launch<8>(h, common_d(h, 1), probs_d, e, st) : launch<7>(h, common_d(h, 1), probs_d, e, st);
 }
 
@@ -631,13 +558,6 @@ int i8_back_projection(sgpr_context* h, cudaStream_t st) {
     e.gvec = h->gvec.as<double>();
     e.ldp = h->dp.ldp;
     e.mumax = h->i8_mumax;
-    if (h->i8_cta2 && h->i8_tr2 == 7) {
-        const Problem2* p2 = nullptr;
-        SGPR_TRY(device_problems2(h, 2, st, &p2));
-        return h->i8_ns == 5 ? launch2<5, 7>(h, common_d(h, 2), p2, e, st) : launch2<6, 7>(h, common_d(h, 2), p2, e, st);
-    }
-    if (h->i8_tr2 == 6) return launch_ns<5, 6>(h, common_d(h, 2), probs_d, e, st);
-    if (h->i8_tr2 == 7 && h->i8_ns == 5) return launch_ns<5, 7>(h, common_d(h, 2), probs_d, e, st);
     return h->i8_tr2 == 8 ? launch<8>(h, common_d(h, 2), probs_d, e, st) : launch<7>(h, common_d(h, 2), probs_d, e, st);
 }
 

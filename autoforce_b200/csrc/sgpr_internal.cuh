@@ -172,9 +172,7 @@ struct sgpr_context {
     bool use_i8 = false;        // GEMMs on tcgen05 (int8 digit slices) instead of FP64 DMMA
     bool use_i8_now = false;    // ... for the current call (compat / K-matrix calls use the DMMA path)
     int i8_tr = 7;              // kernel matrix: truncation t + u <= i8_tr (7: 21 slice products, 8: 26)
-    int i8_tr2 = 7;             // back projection: 7 / 8, or 6 (SGPR_I8_TR2=6: 15 products of 5 slices, ~4e-11 mumax on dE/dq_hat)
-    int i8_ns = 6;              // digit slices read by the GEMMs with t + u <= 7 (SGPR_I8_NS=5: the 5 most significant of the
-                                // 6 stored: 19 products, 38-bit operands)
+    int i8_tr2 = 7;             // back projection: the same choice, 7 or 8 (SGPR_I8_TR2; unset: as i8_tr)
     int i8_kp1 = 0, i8_mp = 0;  // K paddings (multiples of 64) of GEMM 1 (D) and GEMM 2 (max M_s)
     size_t i8_cap_rows = 0;     // row capacity of p8 / g8 (slice stride)
     double i8_mumax = 1.0;      // power of two >= max xi |mu|
@@ -187,11 +185,6 @@ struct sgpr_context {
     unsigned long long i8_prob_sig[3] = {0, 0, 0};   // what the uploaded descriptors were built from (addresses, shapes)
     sgpr::I8Setup i8_setup[3];
     int i8_nprob = 0;
-    int i8_epw = 0;              // SGPR_I8_EPW=2: never use the 4-epilogue-warps-per-quarter kernel (A/B switch)
-    bool i8_cta2 = false;        // SGPR_I8_CTA2=1: CTA-pair (cta_group::2) variant of the two hot GEMMs
-    sgpr::DevBuf i8_probs2;      // its problem descriptors
-    void* i8_probs2_pinned = nullptr;
-    unsigned long long i8_prob2_sig[2] = {0, 0};
     unsigned long long i8_model_version = 0;
     // ---- species row ranges / pair count stay on the device (sync-free steps, DESIGN.md section 4.2)
     sgpr::DevBuf row_first_d;   // [S+1] first descriptor row of each central species (device copy of row_first)

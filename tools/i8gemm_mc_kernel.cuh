@@ -17,10 +17,20 @@
 // armed the barrier just drive the transaction count negative until it does.  TMEM, the MMA schedule and the
 // epilogue are those of the single-CTA kernel (cta_group::1).
 #pragma once
-#include "i8gemm2_kernel.cuh"   // cluster helpers
+#include "i8gemm_kernel.cuh"
 
 namespace sgpr {
 namespace i8g {
+
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+__device__ __forceinline__ void cluster_sync_all() {
+    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
 
 struct ProblemMC {
     CUtensorMap mapAs;    // A operand (as Problem::mapA) with a box of {64 B, BM / CS rows, 1 chunk, 1 slice}
