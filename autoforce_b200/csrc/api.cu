@@ -1528,9 +1528,9 @@ static int batch_front(sgpr_context* h, int B, const int64_t* first_h, int64_t N
     const Geom unused{};
     // cell sort -> neighbour list (the call's one sizing synchronisation) -> descriptors
     if (h->timing) cudaEventRecord(h->ev[0], st);
-    SGPR_TRY(batch_cell_sort(h, N, pos_d, Z_d, *bg, st));
+    SGPR_TRY(cell_sort(h, N, pos_d, Z_d, unused, st, bg));
     int64_t n_pairs = 0;
-    SGPR_TRY(batch_neighbor_build(h, N, *bg, st, &n_pairs));
+    SGPR_TRY(neighbor_build(h, N, unused, st, &n_pairs, false, bg));
     h->stats.n_active = h->n_active;
     h->stats.n_pairs = n_pairs;
     if (h->timing) cudaEventRecord(h->ev[1], st);

@@ -295,22 +295,63 @@ __device__ __forceinline__ void frac_bin(const Geom& g, double x, double y, doub
     }
 }
 
+// the geometry an environment's search uses: the call's, or (batch) that of the centre's structure
+template <bool BATCH>
+__device__ __forceinline__ const Geom& env_geom(const Geom& g, const BatchGeom& bg, int b) {
+    if constexpr (BATCH)
+        return bg.geoms[b];
+    else
+        return g;
+}
+
+// structure of atom i (first: atom offsets) or of bin i (first: bin_base): the last b with first[b] <= i (empty
+// structures are skipped; every structure has at least one bin)
+template <class T>
+__device__ __forceinline__ int batch_of(const T* __restrict__ first, int B, long long i) {
+    int lo = 0, hi = B;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (first[mid] <= i) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// BATCH: keys (bin_base[b] + bin) * S + species -- structure-major, so every structure is one contiguous range of the
+// cell order and of each species' rows; errors go to bg.err and name the first failing structure (atomicMin)
+template <bool BATCH>
 __global__ void bin_count_kernel(int64_t N, const double* __restrict__ pos, const int32_t* __restrict__ Z,
-                                 const int* __restrict__ ztab, Geom g, int S, int* __restrict__ cnt,
-                                 int* __restrict__ key_out, int* __restrict__ rank_out, int* __restrict__ err) {
+                                 const int* __restrict__ ztab, Geom g_call, int S, int* __restrict__ cnt,
+                                 int* __restrict__ key_out, int* __restrict__ rank_out, int* __restrict__ err,
+                                 BatchGeom bg = BatchGeom{}) {
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= N) return;
+    int sb = 0, bbase = 0;
+    if constexpr (BATCH) {
+        sb = batch_of(bg.first, bg.B, i);
+        bbase = bg.bin_base[sb];
+    }
+    const Geom& g = env_geom<BATCH>(g_call, bg, sb);
     int z = Z[i];
     int s = (z >= 0 && z < 128) ? ztab[z] : -1;
     if (s < 0) {
-        atomicExch(&err[0], 1);
-        atomicExch(&err[1], z);
+        if constexpr (BATCH) {
+            atomicMin(&bg.err[0], ((unsigned long long)sb << 32) | (unsigned)z);
+        } else {
+            atomicExch(&err[0], 1);
+            atomicExch(&err[1], z);
+        }
         s = 0;
     }
     int b[3], w[3];
     frac_bin(g, pos[3 * i], pos[3 * i + 1], pos[3 * i + 2], b, w);
-    if (abs(w[0]) > 120 || abs(w[1]) > 120 || abs(w[2]) > 120) atomicExch(&err[0], 2);
-    int bin = (b[0] * g.nb[1] + b[1]) * g.nb[2] + b[2];
+    if (abs(w[0]) > 120 || abs(w[1]) > 120 || abs(w[2]) > 120) {
+        if constexpr (BATCH)
+            atomicMin(&bg.err[1], (unsigned long long)sb);
+        else
+            atomicExch(&err[0], 2);
+    }
+    int bin = bbase + (b[0] * g.nb[1] + b[1]) * g.nb[2] + b[2];
     int key = bin * S + s;
     key_out[i] = key;
     rank_out[i] = atomicAdd(&cnt[key], 1);
@@ -328,46 +369,6 @@ __global__ void scatter_order_kernel(int64_t N, const int* __restrict__ key, con
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= N) return;
     order[cstart[key[i]] + rank[i]] = (int)i;
-}
-
-// one thread per key: sort the (short) run by original index -> deterministic cell order
-__global__ void sort_runs_kernel(int nkeys, const int* __restrict__ cstart, int* __restrict__ order) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= nkeys) return;
-    int b = cstart[k], e = cstart[k + 1];
-    for (int i = b + 1; i < e; ++i) {
-        int v = order[i];
-        int j = i - 1;
-        while (j >= b && order[j] > v) {
-            order[j + 1] = order[j];
-            --j;
-        }
-        order[j + 1] = v;
-    }
-}
-
-__global__ void gather_atoms_kernel(int64_t N, const double* __restrict__ pos, const int* __restrict__ key,
-                                    const int* __restrict__ order, const int* __restrict__ cstart,
-                                    const int* __restrict__ rstartT, Geom g, int S, AtomRec* __restrict__ atoms,
-                                    int* __restrict__ abin, int* __restrict__ rowof) {
-    int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c >= N) return;
-    int i = order[c];
-    int k = key[i];
-    int bin = k / S, s = k - bin * S;
-    double x = pos[3 * (int64_t)i], y = pos[3 * (int64_t)i + 1], z = pos[3 * (int64_t)i + 2];
-    int b[3], w[3];
-    frac_bin(g, x, y, z, b, w);
-    AtomRec r;
-    r.x = x;
-    r.y = y;
-    r.z = z;
-    r.meta = (unsigned long long)(unsigned int)i | ((unsigned long long)s << 32) |
-             ((unsigned long long)(w[0] + 128) << 40) | ((unsigned long long)(w[1] + 128) << 48) |
-             ((unsigned long long)(w[2] + 128) << 56);
-    atoms[c] = r;
-    abin[c] = bin;
-    rowof[c] = rstartT[s * g.ncell + bin] + (int)(c - cstart[k]);
 }
 
 // Exclusive prefix sum of n items by ONE block of 1024 threads, in tiles of 8192 with a running carry.  Lanes read
@@ -443,13 +444,19 @@ __global__ void __launch_bounds__(kScanThreads) key_scan_kernel(int nkeys, int n
 }
 
 // One warp per bin: order every (bin, species) run by original index (the atomics of bin_count_kernel hand out arbitrary
-// ranks; the cell order must not depend on them) and write the cell-ordered atom records of the bin.
+// ranks; the cell order must not depend on them) and write the cell-ordered atom records of the bin.  BATCH: the bin's
+// structure gives the Geom and goes to bg.astr.
+template <bool BATCH>
 __global__ void sort_gather_kernel(int ncell, int64_t N, const double* __restrict__ pos, const int* __restrict__ cstart,
-                                   const int* __restrict__ rstartT, Geom g, int S, int* __restrict__ order,
-                                   AtomRec* __restrict__ atoms, int* __restrict__ abin, int* __restrict__ rowof) {
+                                   const int* __restrict__ rstartT, Geom g_call, int S, int* __restrict__ order,
+                                   AtomRec* __restrict__ atoms, int* __restrict__ abin, int* __restrict__ rowof,
+                                   BatchGeom bg = BatchGeom{}) {
     const int lane = threadIdx.x & 31;
     const int bin = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (bin >= ncell) return;
+    int sb = 0;
+    if constexpr (BATCH) sb = batch_of(bg.bin_base, bg.B, bin);
+    const Geom& g = env_geom<BATCH>(g_call, bg, sb);
     for (int s = 0; s < S; ++s) {
         const int k = bin * S + s;
         const int b = cstart[k], e = cstart[k + 1];
@@ -481,16 +488,10 @@ __global__ void sort_gather_kernel(int ncell, int64_t N, const double* __restric
             const double x = pos[3 * (int64_t)i], y = pos[3 * (int64_t)i + 1], z = pos[3 * (int64_t)i + 2];
             int b3[3], w[3];
             frac_bin(g, x, y, z, b3, w);
-            AtomRec r;
-            r.x = x;
-            r.y = y;
-            r.z = z;
-            r.meta = (unsigned long long)(unsigned int)i | ((unsigned long long)s << 32) |
-                     ((unsigned long long)(w[0] + 128) << 40) | ((unsigned long long)(w[1] + 128) << 48) |
-                     ((unsigned long long)(w[2] + 128) << 56);
-            atoms[c] = r;
+            atoms[c] = atom_rec(x, y, z, i, s, w);
             abin[c] = bin;
             rowof[c] = row0 + (c - b);
+            if constexpr (BATCH) bg.astr[c] = sb;
         }
     }
 }
@@ -514,14 +515,18 @@ int scan_exclusive_ll(sgpr_context* h, const long long* in, long long* out, int 
 // Workspace layout after cell_sort (all int32 unless noted):
 //   cnt     [nkeys+1]   atoms per key (last entry 0 so the exclusive scan yields the total)
 //   cstart  [nkeys+1]   first cell-order index of each key
-//   rstart  [2*(nkeys+1)]  transposed counts, then their scan: first row of (species, bin)
+//   rstart  [2*(nkeys+1)]  transposed counts (cub path), then the species-major scan: first row of (species, bin)
 //   keyrank [2N]        key per original atom, arbitrary rank within key
 //   order   [N]         original index of cell-order atom c
 //   atoms   [N] AtomRec ; rowof [2N]: abin[c], rowof[c]
-//   misc    [16] ints   err flag(2) ...
-int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const Geom& g, cudaStream_t st) {
+//   errflag             error flags (single structure) and the pair cursor; bg->err (batch), bg->astr [N] (batch)
+// bg: a batch (sgpr_predict_batch) -- bins of all its structures, keys structure-major (bin_count_kernel<true>); its
+// errors are reported by neighbor_build's sizing step.
+int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const Geom& g, cudaStream_t st,
+              const BatchGeom* bg) {
     const int S = h->S;
-    const int nkeys = g.ncell * S;
+    const int ncell = bg ? bg->ncell : g.ncell;
+    const int nkeys = ncell * S;
     SGPR_TRY(h->cnt.ensure(sizeof(int) * (nkeys + 1)));
     SGPR_TRY(h->cstart.ensure(sizeof(int) * (nkeys + 1)));
     SGPR_TRY(h->rstart.ensure(sizeof(int) * 2 * (nkeys + 1)));
@@ -536,146 +541,34 @@ int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_
     int* key = h->keyrank.as<int>();
     int* rank = key + (N + 1);
     int* err = h->errflag.as<int>();
+    const BatchGeom bgv = bg ? *bg : BatchGeom{};
     SGPR_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (nkeys + 1), st));
     SGPR_CUDA(cudaMemsetAsync(err, 0, kErrflagBytes, st));   // error flags and the pair cursor
+    if (bg) SGPR_CUDA(cudaMemsetAsync(bg->err, 0x7f, sizeof(unsigned long long) * 2, st));
     const int T = 256;
     const int nblkN = (int)((N + T - 1) / T);
     const int nblkK = (nkeys + T - 1) / T;
     if (N > 0)
-        bin_count_kernel<<<nblkN, T, 0, st>>>(N, pos_d, Z_d, h->ztab.as<int>(), g, S, cnt, key, rank, err);
+        (bg ? bin_count_kernel<true> : bin_count_kernel<false>)<<<nblkN, T, 0, st>>>(N, pos_d, Z_d, h->ztab.as<int>(), g, S,
+                                                                                     cnt, key, rank, err, bgv);
+    int launches = 4;
     if (h->nl_lean && nkeys + 1 <= kScanMaxKeys) {
-        // lean path (< 2^18 bin x species keys): 4 kernels instead of 9
-        key_scan_kernel<<<2, kScanThreads, 0, st>>>(nkeys, g.ncell, S, cnt, cstart, rstartT);
-        if (N > 0) {
-            scatter_order_kernel<<<nblkN, T, 0, st>>>(N, key, rank, cstart, h->order.as<int>());
-            sort_gather_kernel<<<(g.ncell + 7) / 8, 256, 0, st>>>(g.ncell, N, pos_d, cstart, rstartT, g, S, h->order.as<int>(),
-                                                               h->atoms.as<AtomRec>(), h->rowof.as<int>(),
-                                                               h->rowof.as<int>() + (N + 1));
-        }
-        h->stats.kernel_launches += 4;
-        SGPR_CUDA(cudaGetLastError());
-        return SGPR_OK;
-    }
-    SGPR_CUDA(cudaMemsetAsync(cntT, 0, sizeof(int) * (nkeys + 1), st));
-    transpose_cnt_kernel<<<nblkK, T, 0, st>>>(g.ncell, S, cnt, cntT);
-    SGPR_TRY(scan_exclusive_int(h, cnt, cstart, nkeys + 1, st));
-    SGPR_TRY(scan_exclusive_int(h, cntT, rstartT, nkeys + 1, st));
-    if (N > 0) {
-        scatter_order_kernel<<<nblkN, T, 0, st>>>(N, key, rank, cstart, h->order.as<int>());
-        sort_runs_kernel<<<nblkK, T, 0, st>>>(nkeys, cstart, h->order.as<int>());
-        gather_atoms_kernel<<<nblkN, T, 0, st>>>(N, pos_d, key, h->order.as<int>(), cstart, rstartT, g, S,
-                                                 h->atoms.as<AtomRec>(), h->rowof.as<int>(),
-                                                 h->rowof.as<int>() + (N + 1));
-    }
-    h->stats.kernel_launches += 9;  // 5 own kernels + 2 cub scans (2 kernels each)
-    SGPR_CUDA(cudaGetLastError());
-    return SGPR_OK;
-}
-
-// ---------------------------------------------------------------------------------
-// cell sort of a batch: keys (bin_base[b] + bin) * S + species -- structure-major, so every structure is one contiguous
-// range of the cell order and of each species' rows, and the second (species-major) scan still gives one row block per
-// central species for the whole batch
-// ---------------------------------------------------------------------------------
-// structure of atom i: the last b with first[b] <= i (empty structures are skipped)
-__device__ __forceinline__ int batch_of(const long long* __restrict__ first, int B, long long i) {
-    int lo = 0, hi = B;
-    while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (first[mid] <= i) lo = mid;
-        else hi = mid;
-    }
-    return lo;
-}
-
-__global__ void batch_bin_count_kernel(int64_t N, const double* __restrict__ pos, const int32_t* __restrict__ Z,
-                                       const int* __restrict__ ztab, BatchGeom bg, int S, int* __restrict__ cnt,
-                                       int* __restrict__ key_out, int* __restrict__ rank_out) {
-    int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= N) return;
-    const int b = batch_of(bg.first, bg.B, i);
-    int z = Z[i];
-    int s = (z >= 0 && z < 128) ? ztab[z] : -1;
-    if (s < 0) {
-        atomicMin(&bg.err[0], ((unsigned long long)b << 32) | (unsigned)z);
-        s = 0;
-    }
-    int bn[3], w[3];
-    frac_bin(bg.geoms[b], pos[3 * i], pos[3 * i + 1], pos[3 * i + 2], bn, w);
-    if (abs(w[0]) > 120 || abs(w[1]) > 120 || abs(w[2]) > 120) atomicMin(&bg.err[1], (unsigned long long)b);
-    const Geom& g = bg.geoms[b];
-    int bin = bg.bin_base[b] + (bn[0] * g.nb[1] + bn[1]) * g.nb[2] + bn[2];
-    int key = bin * S + s;
-    key_out[i] = key;
-    rank_out[i] = atomicAdd(&cnt[key], 1);
-}
-
-// cell-ordered atom records (runs already sorted by original index), global bin, row, structure
-__global__ void batch_gather_kernel(int64_t N, const double* __restrict__ pos, const int* __restrict__ key,
-                                    const int* __restrict__ order, const int* __restrict__ cstart,
-                                    const int* __restrict__ rstartT, BatchGeom bg, int S, AtomRec* __restrict__ atoms,
-                                    int* __restrict__ abin, int* __restrict__ rowof) {
-    int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c >= N) return;
-    int i = order[c];
-    int k = key[i];
-    int bin = k / S, s = k - bin * S;
-    const int b = batch_of(bg.first, bg.B, i);
-    double x = pos[3 * (int64_t)i], y = pos[3 * (int64_t)i + 1], z = pos[3 * (int64_t)i + 2];
-    int b3[3], w[3];
-    frac_bin(bg.geoms[b], x, y, z, b3, w);
-    AtomRec r;
-    r.x = x;
-    r.y = y;
-    r.z = z;
-    r.meta = (unsigned long long)(unsigned int)i | ((unsigned long long)s << 32) |
-             ((unsigned long long)(w[0] + 128) << 40) | ((unsigned long long)(w[1] + 128) << 48) |
-             ((unsigned long long)(w[2] + 128) << 56);
-    atoms[c] = r;
-    abin[c] = bin;
-    rowof[c] = rstartT[s * bg.ncell + bin] + (int)(c - cstart[k]);
-    bg.astr[c] = b;
-}
-
-// Same workspace layout as cell_sort, plus h->astr.  Errors are reported by batch_neighbor_build's sizing step.
-int batch_cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const BatchGeom& bg, cudaStream_t st) {
-    const int S = h->S;
-    const int nkeys = bg.ncell * S;
-    SGPR_TRY(h->cnt.ensure(sizeof(int) * (nkeys + 1)));
-    SGPR_TRY(h->cstart.ensure(sizeof(int) * (nkeys + 1)));
-    SGPR_TRY(h->rstart.ensure(sizeof(int) * 2 * (nkeys + 1)));
-    SGPR_TRY(h->keyrank.ensure(sizeof(int) * 2 * (N + 1)));
-    SGPR_TRY(h->order.ensure(sizeof(int) * (N + 1)));
-    SGPR_TRY(h->atoms.ensure(sizeof(AtomRec) * (N + 1)));
-    SGPR_TRY(h->rowof.ensure(sizeof(int) * 2 * (N + 1)));
-    int* cnt = h->cnt.as<int>();
-    int* cstart = h->cstart.as<int>();
-    int* cntT = h->rstart.as<int>();
-    int* rstartT = cntT + (nkeys + 1);
-    int* key = h->keyrank.as<int>();
-    int* rank = key + (N + 1);
-    SGPR_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int) * (nkeys + 1), st));
-    SGPR_CUDA(cudaMemsetAsync(h->errflag.p, 0, kErrflagBytes, st));   // error flags and the pair cursor
-    SGPR_CUDA(cudaMemsetAsync(bg.err, 0x7f, sizeof(unsigned long long) * 2, st));
-    const int T = 256;
-    const int nblkN = (int)((N + T - 1) / T);
-    const int nblkK = (nkeys + T - 1) / T;
-    if (N > 0) batch_bin_count_kernel<<<nblkN, T, 0, st>>>(N, pos_d, Z_d, h->ztab.as<int>(), bg, S, cnt, key, rank);
-    if (nkeys + 1 <= kScanMaxKeys) {
-        key_scan_kernel<<<2, kScanThreads, 0, st>>>(nkeys, bg.ncell, S, cnt, cstart, rstartT);
+        // both scans in one launch (< 2^18 bin x species keys)
+        key_scan_kernel<<<2, kScanThreads, 0, st>>>(nkeys, ncell, S, cnt, cstart, rstartT);
     } else {
         SGPR_CUDA(cudaMemsetAsync(cntT, 0, sizeof(int) * (nkeys + 1), st));
-        transpose_cnt_kernel<<<nblkK, T, 0, st>>>(bg.ncell, S, cnt, cntT);
+        transpose_cnt_kernel<<<nblkK, T, 0, st>>>(ncell, S, cnt, cntT);
         SGPR_TRY(scan_exclusive_int(h, cnt, cstart, nkeys + 1, st));
         SGPR_TRY(scan_exclusive_int(h, cntT, rstartT, nkeys + 1, st));
+        launches = 8;   // transpose + 2 cub scans (2 kernels each) instead of key_scan
     }
     if (N > 0) {
         scatter_order_kernel<<<nblkN, T, 0, st>>>(N, key, rank, cstart, h->order.as<int>());
-        sort_runs_kernel<<<nblkK, T, 0, st>>>(nkeys, cstart, h->order.as<int>());
-        batch_gather_kernel<<<nblkN, T, 0, st>>>(N, pos_d, key, h->order.as<int>(), cstart, rstartT, bg, S,
-                                                 h->atoms.as<AtomRec>(), h->rowof.as<int>(), h->rowof.as<int>() + (N + 1));
+        (bg ? sort_gather_kernel<true> : sort_gather_kernel<false>)<<<(ncell + 7) / 8, 256, 0, st>>>(
+            ncell, N, pos_d, cstart, rstartT, g, S, h->order.as<int>(), h->atoms.as<AtomRec>(), h->rowof.as<int>(),
+            h->rowof.as<int>() + (N + 1), bgv);
     }
-    h->stats.kernel_launches += 5;
+    h->stats.kernel_launches += launches;
     SGPR_CUDA(cudaGetLastError());
     return SGPR_OK;
 }
@@ -740,15 +633,6 @@ constexpr int kMaskSlots = 64;
 // per-lane counters, one warp reduction at the end), accept masks per candidate batch and halo
 // marks.  FILL pass: replays the traversal, takes the accept bits from the masks and writes the
 // pairs species-sorted (per-species ballots give each accepted candidate its rank).
-// the geometry an environment's search uses: the call's, or (batch) that of the centre's structure
-template <bool BATCH>
-__device__ __forceinline__ const Geom& env_geom(const Geom& g, const BatchGeom& bg, int b) {
-    if constexpr (BATCH)
-        return bg.geoms[b];
-    else
-        return g;
-}
-
 // BATCH: a batch of structures (sgpr_predict_batch) -- each environment reads its structure's Geom, and its stencil
 // stays inside that structure's bins (bg.bin_base); same traversal, pair_test and pair order as a call on the structure
 template <bool FILL, int NS, bool BATCH = false>
@@ -1290,7 +1174,7 @@ static int check_err_flags(const int* err) {
     return SGPR_OK;
 }
 
-// batch errors name the first structure that failed (batch_bin_count_kernel)
+// batch errors name the first structure that failed (bin_count_kernel<true>)
 static int check_batch_err(const unsigned long long* berr) {
     const unsigned long long none = 0x7f7f7f7f7f7f7f7full;
     if (berr[0] != none) {
@@ -1439,32 +1323,19 @@ static int nl_finish(sgpr_context* h, const Geom& g, cudaStream_t st, const int*
 
 // Neighbour list of ALL atoms (single-GPU path): rows in cell order, descriptor rows from the species-major scan of
 // cell_sort.  Output: nl_rows [N] (begin, end) into nl_pairs, each row ordered by neighbour species, then bin traversal
-// order, then cell order; h->row_first.
-int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, int64_t* n_pairs, bool warm) {
+// order, then cell order; h->row_first.  bg: all atoms of a batch, one warp per environment (batched neighbor_kernel);
+// always a sizing step.
+int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, int64_t* n_pairs, bool warm,
+                   const BatchGeom* bg) {
     h->active_all = true;
     h->n_active = N;
     SGPR_TRY(h->nl_cnt.ensure(sizeof(int) * ((size_t)N * h->S + 1)));
     SGPR_TRY(h->nl_masks.ensure(sizeof(unsigned) * kMaskSlots * ((size_t)N + 1)));
     SGPR_TRY(h->nl_rows.ensure(sizeof(longlong2) * ((size_t)N + 1)));
-    launch_count(h, 0, (int)N, g, nullptr, st, 0);
-    const int nkeys = g.ncell * h->S;
-    const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
-    return nl_finish(h, g, st, rstartT, (int)sizeof(int) * g.ncell, n_pairs, 0, (int)N, warm);
-}
-
-// Neighbour list of all atoms of a batch: one warp per environment (batched neighbor_kernel), rows in the batch's cell
-// order, species row ranges from batch_cell_sort's species-major scan.  Always a sizing step.
-int batch_neighbor_build(sgpr_context* h, int64_t N, const BatchGeom& bg, cudaStream_t st, int64_t* n_pairs) {
-    h->active_all = true;
-    h->n_active = N;
-    SGPR_TRY(h->nl_cnt.ensure(sizeof(int) * ((size_t)N * h->S + 1)));
-    SGPR_TRY(h->nl_masks.ensure(sizeof(unsigned) * kMaskSlots * ((size_t)N + 1)));
-    SGPR_TRY(h->nl_rows.ensure(sizeof(longlong2) * ((size_t)N + 1)));
-    const Geom unused{};
-    launch_count(h, 0, (int)N, unused, nullptr, st, -1, &bg);
-    const int nkeys = bg.ncell * h->S;
-    const int* rstartT = h->rstart.as<int>() + (nkeys + 1);
-    return nl_finish(h, unused, st, rstartT, (int)sizeof(int) * bg.ncell, n_pairs, 0, 0, false, &bg);
+    launch_count(h, 0, (int)N, g, nullptr, st, 0, bg);
+    const int ncell = bg ? bg->ncell : g.ncell;
+    const int* rstartT = h->rstart.as<int>() + (ncell * h->S + 1);
+    return nl_finish(h, g, st, rstartT, (int)sizeof(int) * ncell, n_pairs, 0, (int)N, warm, bg);
 }
 
 // ---------------------------------------------------------------------------------

@@ -46,6 +46,17 @@ struct __align__(32) AtomRec {
 __host__ __device__ inline int meta_orig(unsigned long long m) { return (int)(m & 0xffffffffull); }
 __host__ __device__ inline int meta_species(unsigned long long m) { return (int)((m >> 32) & 0xff); }
 __host__ __device__ inline int meta_w(unsigned long long m, int c) { return (int)((m >> (40 + 8 * c)) & 0xff) - 128; }
+// record of original atom i, species s, wrap shift w[3] (|w| <= 120: the cell sort flags larger shifts)
+__device__ __forceinline__ AtomRec atom_rec(double x, double y, double z, int i, int s, const int* w) {
+    AtomRec r;
+    r.x = x;
+    r.y = y;
+    r.z = z;
+    r.meta = (unsigned long long)(unsigned int)i | ((unsigned long long)s << 32) |
+             ((unsigned long long)(w[0] + 128) << 40) | ((unsigned long long)(w[1] + 128) << 48) |
+             ((unsigned long long)(w[2] + 128) << 56);
+    return r;
+}
 
 // Neighbour pair record (8 bytes): cell-order index of j, bin-level image shift
 // (relative to WRAPPED positions) and species of j.
@@ -167,7 +178,8 @@ struct sgpr_context {
     sgpr::DevBuf erow_part, erow, prow;  // per-row energy partials / local energies / descriptor norms
     sgpr::DevBuf ttab;          // [D] kappa*nnl*(1 + [a==b]) per packed entry
     // ---- tcgen05 int8-sliced GEMM path (i8gemm.cu)
-    bool nl_lean = true;        // SGPR_NL_LEAN=0: force the many-kernel cell sort / row scan that very large systems use -- test hook
+    bool nl_lean = true;        // SGPR_NL_LEAN=0: force the cub scans of the cell sort and the many-kernel row scan that
+                                // very large systems use, on single structures and batches -- test hook
     int nl_mode = 0;            // SGPR_NL: 0 auto, 1 "warp" (one warp per environment), 2 "bins" (one block per bin) -- test hook
     bool use_i8 = false;        // GEMMs on tcgen05 (int8 digit slices) instead of FP64 DMMA
     bool use_i8_now = false;    // ... for the current call (compat / K-matrix calls use the DMMA path)
@@ -292,13 +304,13 @@ int build_geometry(sgpr_context* h, int64_t N, const double* pos_d, const double
 // structure is not periodic on all axes)
 int build_geometry_batch(sgpr_context* h, int B, const int64_t* first_h, const double* pos_d, const double* cell_h,
                          const int32_t* pbc_h, cudaStream_t st, std::vector<Geom>* gs);
-// structure-major cell sort + neighbour list of all atoms of a batch (sizing: synchronises the stream)
-int batch_cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const BatchGeom& bg, cudaStream_t st);
-int batch_neighbor_build(sgpr_context* h, int64_t N, const BatchGeom& bg, cudaStream_t st, int64_t* n_pairs);
-int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const Geom& g, cudaStream_t st);
+// bg: a batch -- structure-major cell sort and neighbour list of all its atoms (g unused; sizing: warm = false)
+int cell_sort(sgpr_context* h, int64_t N, const double* pos_d, const int32_t* Z_d, const Geom& g, cudaStream_t st,
+              const BatchGeom* bg = nullptr);
 // warm = true: no device-to-host copy, no synchronisation -- pair count, error flags and species row ranges stay on
 // the device (status_d, row_first_d); needs h->pairs_cap from an earlier sizing step; *n_pairs is then not set
-int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, int64_t* n_pairs, bool warm = false);
+int neighbor_build(sgpr_context* h, int64_t N, const Geom& g, cudaStream_t st, int64_t* n_pairs, bool warm = false,
+                   const BatchGeom* bg = nullptr);
 int neighbor_build_sharded(sgpr_context* h, int64_t N, const Geom& g, int rank, int world, cudaStream_t st,
                            int64_t* n_pairs, bool with_halo = true, bool warm = false);
 int scan_exclusive_ll(sgpr_context* h, const long long* in, long long* out, int n, cudaStream_t st);

@@ -465,11 +465,18 @@ def test_neighbor_list_far_from_the_origin(mode, monkeypatch):
 def test_many_kernel_front_end_of_very_large_systems(name, monkeypatch):
     """Above 2^18 bin x species keys / 2^16 rows the cell sort and the row scan use cub scans and separate kernels instead
     of the one-block versions; SGPR_NL_LEAN=0 forces that path on a small case.  Same lists, same results, also on
-    sync-free (warm) steps."""
+    sync-free (warm) steps, and for a batch (structure-major keys of many structures): the same E and W, bit for bit,
+    as the one-block path."""
     import autoforce_b200 as ab
+    from test_gpu_batch import golden_batch, run_batch
 
-    monkeypatch.setenv("SGPR_NL_LEAN", "0")
     g = load_golden(name)
+    structs = golden_batch(g)
+    monkeypatch.delenv("SGPR_NL_LEAN", raising=False)
+    lean = ab.SgprEngine(model_from_golden(g), species=g["meta"]["species"])   # reads SGPR_NL_LEAN when created
+    E0, F0, W0 = run_batch(lean, structs)
+    lean.close()
+    monkeypatch.setenv("SGPR_NL_LEAN", "0")
     eng = ab.SgprEngine(model_from_golden(g), species=g["meta"]["species"])
     first, J, S = eng.neighbors(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
     f0, J0, S0 = o.neighbor_list(g["pos"], g["cell"], g["meta"]["pbc"], g["meta"]["kernel"]["rc"])
@@ -479,6 +486,9 @@ def test_many_kernel_front_end_of_very_large_systems(name, monkeypatch):
         E, F, W, _ = eng.predict(g["pos"], g["numbers"], g["cell"], g["meta"]["pbc"])
         assert abs(E - float(g["energy"])) / len(g["numbers"]) < TOL_E_PER_ATOM
         assert np.abs(F - g["forces"]).max() < TOL_F
+    E, F, W = run_batch(eng, structs)
+    assert np.array_equal(E, E0) and np.array_equal(W, W0)
+    assert np.abs(F - F0).max() < 1e-12
     eng.close()
 
 
