@@ -96,13 +96,22 @@ __global__ void atom_terms_kernel(int64_t N, int n_active, const int* __restrict
     if (threadIdx.x == 0) part[blockIdx.x] = red[0];
 }
 
-// covloss (calculator/active.py:781-804): beta_i = sqrt(clamp(1 - c_i, 0)) * sqrt(vscale[Z_i])
+constexpr double kEpsF64 = 2.220446049250313e-16;   // the eps of q = p / (|p| + eps) (descriptor.cu: kEps)
+// Normalised rows with |p| below this are finished in float64.  q = p / (|p| + eps) makes the self kernel
+// alpha = (q.q)^xi = (|p| / (|p| + eps))^(2 xi), far below 1 when |p| ~ eps (every neighbour close to rc), and c / alpha
+// needs K relative to |q|^xi, while the int8 digits of q and K are absolute steps of 2^-46.  Above it |q| > 1 - 2^-12,
+// so the int8 covloss is as accurate as for |q| = 1, and |p| = prow - eps is exact to 2^-53 relative.
+constexpr double kCovFp64Norm = 0x1p-40;
+
+// covloss (calculator/active.py:781-804): beta_i = sqrt(clamp(1 - c_i / alpha_i, 0)) * sqrt(vscale[Z_i]).  Normalised rows
+// with |p| < kCovFp64Norm are listed in fix[] (fix[0] = count) for beta_fp64_rows_kernel instead.
 __global__ void beta_finish_kernel(int n_active, const int* __restrict__ active, const AtomRec* __restrict__ atoms,
                                    const int* __restrict__ rowof, const longlong2* __restrict__ nl_rows,
                                    const unsigned char* __restrict__ owned, const unsigned char* __restrict__ sp_on,
                                    const int* __restrict__ sp_enabled, const double* __restrict__ cpart, int n_part,
                                    int part_ld, const double* __restrict__ clone, const double* __restrict__ vscale,
-                                   const double* __restrict__ prow, int normalized, double xi, double* __restrict__ beta) {
+                                   const double* __restrict__ prow, int normalized, double xi, int* __restrict__ fix,
+                                   double* __restrict__ beta) {
     for (int env = blockIdx.x * blockDim.x + threadIdx.x; env < n_active; env += gridDim.x * blockDim.x) {
         const int c = active ? active[env] : env;
         if (owned && !owned[c]) continue;
@@ -114,14 +123,86 @@ __global__ void beta_finish_kernel(int n_active, const int* __restrict__ active,
             cc = clone[sp];
         } else if (sp_on[sp]) {
             const int row = rowof[c];
+            // the self kernel alpha = k(x,x) = (q.q)^xi (active.py:784-791).  Un-normalised: q = p, prow = |p|.
+            // Normalised: q = p / (|p| + eps), prow = |p| + eps.
+            const double P = prow[row];
+            if (normalized && P - kEpsF64 < kCovFp64Norm) {
+                fix[1 + atomicAdd(fix, 1)] = env;
+                continue;
+            }
             for (int p = 0; p < n_part; ++p) cc += cpart[(size_t)p * part_ld + row];
-            // un-normalised descriptors: c / alpha with the self kernel alpha = k(x,x) = (p.p)^xi (active.py:784-791)
-            if (!normalized) cc /= pow(prow[row] * prow[row], xi);
+            const double q = normalized ? (P - kEpsF64) / P : P;
+            cc /= pow(q * q, xi);
         }
         double b = sqrt(fmax(1.0 - cc, 0.0));
         // the reference divides c by the self kernel k(x,x) = 0 for an excluded centre -> NaN (active.py:784-791)
         if (!lone && !sp_enabled[sp]) b = nan("");
         beta[meta_orig(meta)] = b * sqrt(vscale[sp]);
+    }
+}
+
+// sum over the block, valid in thread 0; red[] is free again on return
+__device__ double block_sum(double v, double* red) {
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double t = 0.0;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += red[w];
+    __syncthreads();
+    return t;
+}
+
+struct SpeciesBlocks {
+    int first[SGPR_MAX_SPECIES + 1];   // inducing LCEs of species s: sorted rows first[s] .. first[s+1]
+};
+
+// covloss of the rows beta_finish_kernel listed in fix[], in float64 from the descriptor rows (one block per row):
+// alpha = (q.q)^xi, K_p = (q . z_p)^xi over the species' inducing LCEs, b = choli_t K, c = b.b -- what the oracle does.
+__global__ void beta_fp64_rows_kernel(const int* __restrict__ fix, const int* __restrict__ active,
+                                      const AtomRec* __restrict__ atoms, const int* __restrict__ rowof,
+                                      const double* __restrict__ phat, int ldp, int D, const double* __restrict__ zhat,
+                                      SpeciesBlocks mb, const double* __restrict__ choli_t, int M, int ld_zt,
+                                      const double* __restrict__ vscale, double xi, int xi_int, double* __restrict__ beta) {
+    extern __shared__ double ksm[];   // K of the row, [M_s]
+    __shared__ double red[32];
+    const int n = fix[0];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    for (int i = blockIdx.x; i < n; i += gridDim.x) {
+        const int env = fix[1 + i];
+        const int c = active ? active[env] : env;
+        const unsigned long long meta = atoms[c].meta;
+        const int sp = meta_species(meta);
+        const double* q = phat + (size_t)rowof[c] * ldp;
+        double s = 0.0;
+        for (int e = threadIdx.x; e < D; e += blockDim.x) s = fma(q[e], q[e], s);
+        const double qq = block_sum(s, red);
+        const int m0 = mb.first[sp], Ms = mb.first[sp + 1] - m0;
+        for (int p = warp; p < Ms; p += nw) {
+            const double* z = zhat + (size_t)(m0 + p) * ldp;
+            double d = 0.0;
+            for (int e = lane; e < D; e += 32) d = fma(q[e], z[e], d);
+            for (int o = 16; o; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
+            if (lane == 0) {
+                double k = d;
+                if (xi_int >= 1)
+                    for (int t = 1; t < xi_int; ++t) k *= d;
+                else
+                    k = pow(d, xi);
+                ksm[p] = k;
+            }
+        }
+        __syncthreads();
+        const double* L = choli_t + (size_t)sp * M * ld_zt;
+        double cc = 0.0;
+        for (int k = threadIdx.x; k < M; k += blockDim.x) {
+            const double* Lk = L + (size_t)k * ld_zt;
+            double b = 0.0;
+            for (int p = 0; p < Ms; ++p) b = fma(Lk[p], ksm[p], b);
+            cc = fma(b, b, cc);
+        }
+        cc = block_sum(cc, red);   // also orders this row's reads of ksm before the next row's writes
+        if (threadIdx.x == 0) beta[meta_orig(meta)] = sqrt(fmax(1.0 - cc / pow(qq, xi), 0.0)) * sqrt(vscale[sp]);
     }
 }
 
@@ -824,7 +905,7 @@ extern "C" __attribute__((visibility("default"))) void sgpr_destroy(sgpr_handle 
                       &h->nl_first, &h->nl_pairs, &h->scan_tmp, &h->phat, &h->cbuf, &h->pnorm, &h->sflag, &h->gmat,
                       &h->gvec, &h->epart, &h->wpart, &h->fcell, &h->misc, &h->stage_pos, &h->stage_z, &h->stage_out,
                       &h->rowmap, &h->owned, &h->shard_tmp, &h->row_owned, &h->choli_t, &h->vscale_d, &h->clone_d,
-                      &h->kcmat, &h->cpart, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_rows, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local,
+                      &h->kcmat, &h->cpart, &h->cov_fp64, &h->nl_masks, &h->erow_part, &h->erow, &h->prow, &h->ttab, &h->z8, &h->zt8, &h->p8, &h->g8, &h->i8_probs, &h->k8, &h->c8, &h->crs, &h->nl_rows, &h->cov_nk, &h->row_first_d, &h->status_d, &h->p2p_local,
                       &h->b_geom, &h->b_first, &h->b_bins, &h->b_cell, &h->b_err, &h->astr, &h->wenv, &h->jsel, &h->kscr,
                       &h->md_pos, &h->md_mom, &h->md_F, &h->md_beta, &h->md_ew, &h->md_part,
                       &h->rx_pos, &h->rx_vel, &h->rx_F, &h->rx_beta, &h->rx_ew, &h->rx_part};
@@ -1019,11 +1100,37 @@ static int covloss_stage(sgpr_context* h, cudaStream_t st, int64_t N, const int*
         SGPR_TRY(h->misc.ensure(sizeof(int) * SGPR_MAX_SPECIES));
         SGPR_CUDA(cudaMemcpyAsync(h->misc.p, h->dp.central_enabled, sizeof(int) * SGPR_MAX_SPECIES,
                                   cudaMemcpyHostToDevice, st));
+        SGPR_TRY(h->cov_fp64.ensure(sizeof(int) * (nrows + 1)));
+        SGPR_CUDA(cudaMemsetAsync(h->cov_fp64.p, 0, sizeof(int), st));
+        const int* rowof = h->rowof.as<int>() + (N + 1);
         beta_finish_kernel<<<h->sm_count * 2, 256, 0, st>>>(
-            (int)h->n_active, active, h->atoms.as<AtomRec>(), h->rowof.as<int>() + (N + 1), h->nl_rows.as<longlong2>(),
+            (int)h->n_active, active, h->atoms.as<AtomRec>(), rowof, h->nl_rows.as<longlong2>(),
             owned, h->sp_on.as<unsigned char>(), h->misc.as<int>(), h->cpart.as<double>(), n_part, (int)nrows,
-            h->clone_d.as<double>(), h->vscale_d.as<double>(), h->prow.as<double>(), h->dp.normalize, h->xi, beta_d);
+            h->clone_d.as<double>(), h->vscale_d.as<double>(), h->prow.as<double>(), h->dp.normalize, h->xi,
+            h->cov_fp64.as<int>(), beta_d);
         h->stats.kernel_launches += 1;
+        if (h->dp.normalize) {
+            SpeciesBlocks mb{};
+            int maxMs = 1;
+            for (int s = 0; s <= h->S; ++s) mb.first[s] = h->m_first[s];
+            for (int s = 0; s < h->S; ++s) maxMs = std::max(maxMs, h->m_first[s + 1] - h->m_first[s]);
+            const size_t smem = sizeof(double) * (size_t)maxMs;
+            static size_t smem_set = 48 * 1024;   // the default limit of dynamic shared memory
+            if (smem > smem_set) {
+                if (cudaFuncSetAttribute(beta_fp64_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
+                    cudaSuccess) {
+                    cudaGetLastError();
+                    set_error("covloss: %d inducing LCEs of one species exceed the shared memory of a block", maxMs);
+                    return SGPR_ERR_INVALID;
+                }
+                smem_set = smem;
+            }
+            beta_fp64_rows_kernel<<<h->sm_count, 256, smem, st>>>(
+                h->cov_fp64.as<int>(), active, h->atoms.as<AtomRec>(), rowof, h->phat.as<double>(), h->dp.ldp, h->dp.D,
+                h->zhat.as<double>(), mb, h->choli_t.as<double>(), h->M, h->ld_zt, h->vscale_d.as<double>(), h->xi,
+                h->xi_int, beta_d);
+            h->stats.kernel_launches += 1;
+        }
     }
     SGPR_CUDA(cudaGetLastError());
     return SGPR_OK;

@@ -175,6 +175,7 @@ struct sgpr_context {
     sgpr::DevBuf vscale_d;    // [S] model._vscale (inf where unseen)
     sgpr::DevBuf clone_d;     // [S] c of a neighbour-less atom of species s
     sgpr::DevBuf kcmat, cpart;  // covloss: K^xi [rows, ldg], per-row partial sums of squares
+    sgpr::DevBuf cov_fp64;      // covloss: [0] count, [1..] environments finished in float64 (beta_fp64_rows_kernel)
     sgpr::DevBuf erow_part, erow, prow;  // per-row energy partials / local energies / descriptor norms
     sgpr::DevBuf ttab;          // [D] kappa*nnl*(1 + [a==b]) per packed entry
     // ---- tcgen05 int8-sliced GEMM path (i8gemm.cu)

@@ -182,7 +182,6 @@ class Case:
     rc: float
     make: object       # (Zs, seed) -> pos, cell, numbers, pbc
     expect: tuple      # (bin_plan key, value) pairs the geometry must have
-    tol_beta2: float = TOL_BETA2
 
 
 T, F = True, False
@@ -208,10 +207,7 @@ CASES = [
          (("ncell", 125), ("reach", (1, 1, 1)), ("wrapped", T), ("kernel", "bins"), ("NS", 8))),
     Case("sparse_gas", "500 atoms in a 150 A box: bins merged by the max(4096, 4N) rule, empty bins, lone atoms", EIGHT,
          6.0, sparse_gas,
-         (("nb", (12, 12, 24)), ("merges", 2), ("reach", (1, 1, 1)), ("kernel", "bins"), ("NS", 8)),
-         # open finding (DESIGN section 7): beta^2 of environments with a single neighbour is 1.6e-8 off the oracle,
-         # identically through both neighbour kernels and the batch path, while E, F and W agree at the usual bars
-         tol_beta2=1e-7),
+         (("nb", (12, 12, 24)), ("merges", 2), ("reach", (1, 1, 1)), ("kernel", "bins"), ("NS", 8))),
     Case("faces", "atoms exactly on cell faces: wrap at fractional 1, -0.0, 1 - 2^-53, clamp at -2^-60", (3, 8, 15, 29),
          4.5, faces,
          (("nb", (3, 3, 3)), ("reach", (1, 1, 1)), ("wrapped", T), ("clamped", T), ("kernel", "warp"), ("NS", 4))),
@@ -304,12 +300,12 @@ def engine(model, Zs):
     return ab.SgprEngine(model, species=sorted(Zs))
 
 
-def assert_matches(out, E, Fo, W, cell, N, beta=None, tag="", tol_beta2=TOL_BETA2):
+def assert_matches(out, E, Fo, W, cell, N, beta=None, tag=""):
     assert abs(E - out["energy"]) / N < TOL_E, tag
     assert np.abs(Fo - out["forces"]).max() < TOL_F, tag
     assert np.abs(W - out["virial"]).max() / vol(cell) < TOL_SIGMA, tag
     if beta is not None:
-        assert np.abs(beta ** 2 - out["beta"] ** 2).max() < tol_beta2, tag
+        assert np.abs(beta ** 2 - out["beta"] ** 2).max() < TOL_BETA2, tag
 
 
 @pytest.mark.gpu
@@ -333,7 +329,7 @@ def test_neighbor_case(name, mode, monkeypatch):
         for _ in range(2):                                         # sizing step, then a warm one
             E, Fo, W, owned, beta = eng.predict(pos, Z, cell, pbc, want_beta=True)
             assert owned.all()
-            assert_matches(out, E, Fo, W, cell, len(Z), beta, name, c.tol_beta2)
+            assert_matches(out, E, Fo, W, cell, len(Z), beta, name)
     finally:
         eng.close()
 
@@ -350,7 +346,7 @@ def test_whole_table_in_one_batch():
     a0 = 0
     for b, ((pos, cell, Z, pbc), out) in enumerate(zip(structs, refs)):
         N = len(Z)
-        assert_matches(out, Eb[b], Fb[a0:a0 + N], Wb[b], cell, N, bb[a0:a0 + N], CASES[b].name, CASES[b].tol_beta2)
+        assert_matches(out, Eb[b], Fb[a0:a0 + N], Wb[b], cell, N, bb[a0:a0 + N], CASES[b].name)
         a0 += N
 
 
